@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- images/sec of the lines->VPs hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config C] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config C] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the path (segments -> lines -> sphere votes -> CNN ->
 EM -> VPs) over one synthetic batch of BASELINE.json config C.
@@ -26,6 +26,8 @@ e2e      : same metric through the public API from pinned HOST buffers, H2D and 
 roofline : dominant kernel of the step vs the measured peak in MEASURED_PEAKS.json.
 cpu_baseline / --impl reference : the CPU oracle (numpy/torch restatement of the
            reference path, oracle/) on a bounded sample of the same batch.
+--dump-outputs DIR : the EM result of the last end-to-end step (after the gather, with several ranks) as
+           DIR/<name>.npy; the inputs depend on the arguments only, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -155,6 +157,36 @@ def make_workload(cfg, rank, n_images=None):
     off = np.zeros(B + 1, dtype=np.int32)
     off[1:] = np.cumsum(n)
     return name, np.concatenate(segs, axis=0), off
+
+
+DUMP_LIMIT_BYTES = 60_000_000          # array data; with the .npy headers the files stay below 64 MB
+
+
+def dump_outputs(dirname, res, off):
+    """The flat EM result arrays of one step (Pipeline(..., raw=True), or pipeline.gather_raw's with several ranks) as
+    DIR/<name>.npy in float64.  Entries the library leaves undefined (VP rows beyond n_vp; every field but `status`
+    of an image without VPs) are stored as 0, so that two runs compare byte for byte; `vp_assoc` is in image order.
+    Above DUMP_LIMIT_BYTES in all, a fixed seeded sample of the images is stored; `image_index` lists the images stored."""
+    B, M = len(off) - 1, res["vp"].shape[1]
+    n = np.diff(off).astype(np.int64)
+    start = np.asarray(res.get("assoc_start", off[:-1]), dtype=np.int64)
+    keep = np.arange(B)
+    per_image = 8 * (4 + 6 * M + n)
+    if per_image.sum() > DUMP_LIMIT_BYTES:
+        order = np.random.RandomState(0).permutation(B)
+        keep = np.sort(order[:np.searchsorted(np.cumsum(per_image[order]), DUMP_LIMIT_BYTES, side="right")])
+    ok = res["status"][keep] == 0
+    n_vp = np.where(ok, res["n_vp"][keep], 0)
+    rows = np.arange(M)[None, :] < n_vp[:, None]
+    out = {"image_index": keep, "status": res["status"][keep], "n_vp": n_vp,
+           "iterations": np.where(ok, res["iterations"][keep], 0), "vp": np.where(rows[:, :, None], res["vp"][keep], 0.0)}
+    for k in ("sigma", "counts", "counts_weighted"):
+        out[k] = np.where(rows, res[k][keep], 0)
+    out["vp_assoc"] = np.concatenate([np.zeros(0)] + [res["vp_assoc"][start[i]:start[i] + n[i]] if good else np.zeros(n[i])
+                                                      for i, good in zip(keep, ok)])
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(dirname, k + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 # ------------------------------------------------------------------ CPU oracle arm
@@ -612,6 +644,8 @@ def run_ours(args, rank, world, local_rank):
                             "stream; the pair pass then does not overlap stages 1-2 as it does in the timed legs)",
             "images_with_vps": n_ok,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, *((full, off_all) if full is not None else (out, off)))
         emit(line)
     if world > 1:
         dist.barrier()
@@ -651,7 +685,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--settle", type=int, default=30, help="upper bound of the extra untimed settling steps after the warm-up")
     ap.add_argument("--clock-period", type=float, default=0.005, help="seconds between NVML clock samples in the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the EM result of the last timed end-to-end step as DIR/<name>.npy (float64, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's result (--impl ours)")
     # stdout carries the ONE JSON line and nothing else: libraries that write to file descriptor 1 (NCCL prints its
     # version banner there) are sent to stderr; emit() writes the line to the real stdout
     sys.stdout.flush()
