@@ -206,6 +206,36 @@ VPK_API int vpk_segments_from_lsd(vpk_ctx* ctx, const double* lsd, int32_t ncols
 VPK_API int vpk_pipeline_upload_lsd(vpk_ctx* ctx, const double* lsd, int32_t ncols, const int32_t* offsets,
                                     const int32_t* widths, const int32_t* heights, int32_t n_images);
 
+/* ---- N4: the LSD line segment detector ----------------------------------------- */
+/* lsd.detect_line_segments (lsdpython/lsd.pyx:17-18, LSD 1.6's LineSegmentDetection) as evaluation.detect_lsd_lines
+ * calls it (reference evaluation.py:227-251), on the device for a ragged batch of grayscale images. */
+typedef struct vpk_lsd_config {
+    double scale;        /* 0.8  */
+    double sigma_scale;  /* 0.6  */
+    double quant;        /* 2.0  */
+    double ang_th;       /* 22.5 */
+    double log_eps;      /* 0.0  */
+    double density_th;   /* 0.7  */
+    int32_t n_bins;      /* 1024 */
+} vpk_lsd_config;
+VPK_API void vpk_lsd_default_config(vpk_lsd_config* cfg);
+/* pixel types of vpk_lsd's images */
+enum { VPK_PIX_U8 = 0, VPK_PIX_F64 = 1 };
+/* images: host array of gray values of type `dtype`; image b is the row-major heights[b] x widths[b] block that
+ * starts at element pixel_offsets[b] (pixel_offsets has B+1 entries, pixel_offsets[b+1] - pixel_offsets[b] =
+ * widths[b] * heights[b]).  Runs the detector, keeps the rows on the device and writes the number of segments
+ * of every image to counts_out (B).  A sampled side (ceil(side * scale)) must be below 65536. */
+VPK_API int vpk_lsd(vpk_ctx* ctx, const void* images, int32_t dtype, const int64_t* pixel_offsets, const int32_t* widths,
+                    const int32_t* heights, int32_t n_images, const vpk_lsd_config* cfg, int32_t* counts_out);
+/* rows of the last vpk_lsd call: (sum counts, 7) float64 x1, y1, x2, y2, width, p, -log10(NFA) in pixels of the
+ * input images, image after image, each image's rows in LSD's own output order. */
+VPK_API int vpk_lsd_fetch(vpk_ctx* ctx, double* rows_out);
+/* vpk_lsd followed by vpk_pipeline_upload_lsd's normalisation, on the device: the rows never leave it; only the
+ * per-image counts come back (counts_out (B), may be NULL). */
+VPK_API int vpk_pipeline_upload_images(vpk_ctx* ctx, const void* images, int32_t dtype, const int64_t* pixel_offsets,
+                                       const int32_t* widths, const int32_t* heights, int32_t n_images,
+                                       const vpk_lsd_config* cfg, int32_t* counts_out);
+
 /* ---- N1: horizon line and orthogonal VP triplet --------------------------- */
 /* calc_horizon.calculate_horizon_and_ortho_vp(em_result, maxbest=10, theta_vmin=pi/10, theta_z=pi/4)
  * (reference calc_horizon.py:19-225; callers example.py:65, benchmark.py:233) for a batch of EM

@@ -22,7 +22,9 @@ SYMBOLS = [
     "vpk_cnn_load", "vpk_cnn_forward", "vpk_debug_gemm", "vpk_em_default_config", "vpk_em", "vpk_em_distribution", "vpk_em_stats", "vpk_em_phase_cycles", "vpk_pipeline_upload", "vpk_pipeline_run",
     "vpk_pipeline_fetch", "vpk_pipeline_host", "vpk_pipeline_stage_ms", "vpk_horizon", "vpk_pipeline_horizon",
     "vpk_segments_from_lsd", "vpk_pipeline_upload_lsd",
+    "vpk_lsd_default_config", "vpk_lsd", "vpk_lsd_fetch", "vpk_pipeline_upload_images",
 ]
+PIX_U8, PIX_F64 = 0, 1
 
 
 class VpkError(RuntimeError):
@@ -37,6 +39,12 @@ class EmConfig(C.Structure):
                 ("do_iterations", C.c_int32), ("use_weights", C.c_int32), ("wbias", C.c_double),
                 ("merge_thresh", C.c_double), ("outlier_thresh", C.c_double), ("final_convergence", C.c_double),
                 ("s_thresh", C.c_double)]
+
+
+class LsdConfig(C.Structure):
+    """vpk_lsd_config: the parameters of lsd.detect_line_segments (lsdpython/lsd.pyx:17-18)."""
+    _fields_ = [("scale", C.c_double), ("sigma_scale", C.c_double), ("quant", C.c_double), ("ang_th", C.c_double),
+                ("log_eps", C.c_double), ("density_th", C.c_double), ("n_bins", C.c_int32)]
 
 
 class EmResult(C.Structure):
@@ -99,6 +107,13 @@ def load():
         lib.vpk_pipeline_upload_lsd.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]
         lib.vpk_pipeline_horizon.argtypes = [C.c_void_p, C.c_int32, C.c_double, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.vpk_lsd_default_config.argtypes = [C.POINTER(LsdConfig)]
+        lib.vpk_lsd_default_config.restype = None
+        lib.vpk_lsd.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                C.POINTER(LsdConfig), C.c_void_p]
+        lib.vpk_lsd_fetch.argtypes = [C.c_void_p, C.c_void_p]
+        lib.vpk_pipeline_upload_images.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                   C.c_int32, C.POINTER(LsdConfig), C.c_void_p]
         lib.vpk_abi_version.argtypes = []
         lib.vpk_last_error.argtypes = []
         _lib = lib
@@ -199,6 +214,16 @@ def em_config(**kw):
     for k, v in kw.items():
         if not hasattr(cfg, k):
             raise TypeError("unknown EM option %r" % k)
+        setattr(cfg, k, v)
+    return cfg
+
+
+def lsd_config(**kw):
+    cfg = LsdConfig()
+    load().vpk_lsd_default_config(C.byref(cfg))
+    for k, v in kw.items():
+        if not hasattr(cfg, k):
+            raise TypeError("unknown LSD option %r" % k)
         setattr(cfg, k, v)
     return cfg
 

@@ -96,6 +96,37 @@ int vpk_pipeline_upload_lsd(vpk_ctx* ctx, const double* lsd, int32_t ncols, cons
     return VPK_OK;
 }
 
+int vpk_pipeline_upload_images(vpk_ctx* ctx, const void* images, int32_t dtype, const int64_t* pixel_offsets, const int32_t* widths,
+                               const int32_t* heights, int32_t B, const vpk_lsd_config* cfg, int32_t* counts_out) {
+    if (!ctx || !widths || !heights || B <= 0) { set_error("vpk_pipeline_upload_images: bad argument"); return VPK_ERR_ARG; }
+    std::vector<int32_t> counts(B), row_off;
+    const double* d_rows = nullptr;
+    VPK_TRY(lsd_dev(ctx, images, dtype, pixel_offsets, widths, heights, B, cfg, counts.data(), &d_rows, row_off));
+    if (!ctx->pipe) {
+        ctx->pipe = new PipeState();
+        for (auto& e : ctx->pipe->ev) VPK_CUDA(cudaEventCreate(&e));
+    }
+    PipeState* p = ctx->pipe;
+    const int64_t sumN = row_off[B];
+    p->B = B; p->sumN = sumN; p->have_result = false;
+    p->h_offsets = row_off;
+    VPK_TRY(p->seg.ensure((sumN + 1) * 4 * sizeof(double)));
+    VPK_TRY(p->lines.ensure((sumN + 1) * 3 * sizeof(double)));
+    VPK_TRY(p->offsets.ensure((size_t)(3 * (B + 1)) * sizeof(int32_t)));
+    int32_t* d_off = p->offsets.as<int32_t>();
+    int32_t* d_w = d_off + (B + 1);
+    int32_t* d_h = d_w + (B + 1);
+    cudaStream_t st = ctx->stream;
+    VPK_CUDA(cudaMemcpyAsync(d_off, row_off.data(), (B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    VPK_CUDA(cudaMemcpyAsync(d_w, widths, B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    VPK_CUDA(cudaMemcpyAsync(d_h, heights, B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    // the detector's rows are normalised where they are: they never leave the device
+    VPK_TRY(segments_from_lsd_dev(ctx, d_rows, 7, d_off, d_w, d_h, B, sumN, p->seg.as<double>(), nullptr));
+    VPK_CUDA(cudaStreamSynchronize(st));
+    if (counts_out) memcpy(counts_out, counts.data(), (size_t)B * sizeof(int32_t));
+    return VPK_OK;
+}
+
 int vpk_pipeline_run(vpk_ctx* ctx, int32_t S, int32_t sphere_mode, double alpha, const vpk_em_config* cfg_in) {
     if (!ctx || !ctx->pipe || ctx->pipe->B <= 0) { set_error("vpk_pipeline_run: no batch uploaded"); return VPK_ERR_STATE; }
     if (S != VPK_CNN_SIZE) { set_error("vpk_pipeline_run: the CNN input is %dx%d (cnn/deploy.prototxt:7); size=%d", VPK_CNN_SIZE, VPK_CNN_SIZE, S); return VPK_ERR_ARG; }

@@ -86,6 +86,7 @@ struct PendingEvent {
 struct CnnState;   // cnn.cu
 struct EmState;    // em.cu
 struct PipeState;  // pipeline.cu
+struct LsdState;   // lsd.cu
 
 }  // namespace vpk
 
@@ -113,6 +114,7 @@ struct vpk_ctx {
     vpk::CnnState* cnn = nullptr;
     vpk::EmState* em = nullptr;
     vpk::PipeState* pipe = nullptr;
+    vpk::LsdState* lsd = nullptr;
 };
 
 namespace vpk {
@@ -197,8 +199,15 @@ size_t horizon_out_bytes(int32_t B);
 int horizon_upload_truth(vpk_ctx* ctx, DBuf& buf, const double* true_horizons, const double* scales, const double* heights, int32_t B);
 void horizon_unpack(const void* h_rec, int32_t B, double* points, int32_t* best_combo, double* errors);
 
+// lsd.cu: the LSD detector on a ragged batch of images; leaves the (sum N, 7) rows on the device (*d_rows,
+// image b's rows start at row_offsets[b], which the host also gets) and writes the B counts to counts_out
+int lsd_dev(vpk_ctx* ctx, const void* images, int32_t dtype, const int64_t* pixel_offsets, const int32_t* widths,
+            const int32_t* heights, int32_t B, const vpk_lsd_config* cfg, int32_t* counts_out, const double** d_rows,
+            std::vector<int32_t>& row_offsets);
+
 void cnn_free(vpk_ctx* ctx);
 void em_free(vpk_ctx* ctx);
 void pipe_free(vpk_ctx* ctx);
+void lsd_free(vpk_ctx* ctx);
 
 }  // namespace vpk

@@ -1,8 +1,8 @@
 """Host mirror of the parts of the reference's evaluation.py that sit between the LSD detector and the
 hot path (SURVEY.md section 8(f), row N2): the normalisation of the raw LSD rows
 (`detect_lsd_lines`, evaluation.py:227-251, everything after the `lsd.detect_line_segments` call) and the
-line construction (evaluation.py:158-168), on the device through the C ABI (`vpk_segments_from_lsd`).
-The LSD detector itself stays upstream (row N4).  No CPU fallback."""
+line construction (evaluation.py:158-168), on the device through the C ABI (`vpk_segments_from_lsd`), and
+`detect_lsd_lines` itself with the detector on the device too (row N4, `vpk_lsd`).  No CPU fallback."""
 import numpy as np
 
 from . import _lib
@@ -35,6 +35,19 @@ def segments_from_lsd(lsd_lines, image_shape):
     """What detect_lsd_lines returns for one image (evaluation.py:251): {'segments': (N,4), 'nfa': (N,)}."""
     out = segments_from_lsd_batch([lsd_lines], [image_shape], want_lines=False)
     return {"segments": out["segments"], "nfa": out["nfa"]}
+
+
+def detect_lsd_lines(image):
+    """evaluation.detect_lsd_lines (reference evaluation.py:227-251) for a 2-D grayscale image: gray values as
+    float64, scaled by 255 when the image's maximum is at most 1, LSD with lsd.pyx's defaults, then the
+    normalisation above.  Returns {'segments': (N,4), 'nfa': (N,)}.  (RGB -> gray stays with the caller.)"""
+    from . import lsd
+    gray = np.array(image, dtype=np.float64)
+    if gray.ndim != 2:
+        raise ValueError("detect_lsd_lines takes a 2-D grayscale image, got shape %r" % (gray.shape,))
+    if gray.max() <= 1:
+        gray *= 255
+    return segments_from_lsd(lsd.detect_line_segments(gray), gray.shape)
 
 
 # ---------------------------------------------------------------------------------------------------

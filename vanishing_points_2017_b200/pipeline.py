@@ -68,6 +68,23 @@ class Pipeline:
         _lib.check(self.ctx.lib.vpk_pipeline_upload_lsd(self.ctx.h, _lib.ptr(lsd), lsd.shape[1], _lib.ptr(off), _lib.ptr(w),
                                                         _lib.ptr(h), self._B), "vpk_pipeline_upload_lsd")
 
+    def upload_images(self, images, **lsd_kwargs):
+        """upload() from grayscale images (a list of 2-D arrays of any sizes, uint8 or float64 gray values): the
+        LSD detector (lsd.detect_line_segments with `lsd_kwargs`, lsd.pyx's defaults otherwise) and the
+        normalisation of evaluation.py:240-249 run on the device into the resident batch; only the per-image
+        segment counts come back.  Returns them."""
+        from .lsd import pack_images
+        if len(images) == 0:
+            raise ValueError("upload_images needs at least one image")
+        flat, dt, off, w, h = pack_images(images)
+        cfg = _lib.lsd_config(**lsd_kwargs)
+        counts = np.empty(len(images), np.int32)
+        _lib.check(self.ctx.lib.vpk_pipeline_upload_images(self.ctx.h, _lib.ptr(flat), dt, _lib.ptr(off), _lib.ptr(w), _lib.ptr(h),
+                                                           len(images), C.byref(cfg), _lib.ptr(counts)), "vpk_pipeline_upload_images")
+        self._B = len(images)
+        self._off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
+        return counts
+
     def run(self):
         _lib.check(self.ctx.lib.vpk_pipeline_run(self.ctx.h, self.size, self.mode, self.alpha, C.byref(self.cfg)),
                    "vpk_pipeline_run")
