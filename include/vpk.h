@@ -236,6 +236,29 @@ VPK_API int vpk_pipeline_upload_images(vpk_ctx* ctx, const void* images, int32_t
                                        const int32_t* widths, const int32_t* heights, int32_t n_images,
                                        const vpk_lsd_config* cfg, int32_t* counts_out);
 
+/* ---- N5: photo preparation in front of LSD ------------------------------------ */
+/* The head of evaluation.create_data_pickles (reference evaluation.py:139-154): `convert ... -resize TxT` (here
+ * OpenCV 4.13's INTER_AREA rule in float64), the 8-bit RGB read back, skimage.color.rgb2gray; DESIGN.md section 4.7.
+ * Photos: host array of uint8 RGB, photo b the row-major heights[b] x widths[b] x 3 block starting at byte
+ * byte_offsets[b] (B+1 entries, byte_offsets[b+1] - byte_offsets[b] = 3 * widths[b] * heights[b]).  target_size <= 0:
+ * no resize; otherwise s = target_size / max(w, h) and, if s < 1, W' = max(1, rint(w s)), H' = max(1, rint(h s)).
+ * Photos are never enlarged. */
+/* the prepared size (W', H') of one w x h photo; host only, needs no device or context */
+VPK_API int vpk_prepared_size(int32_t w, int32_t h, int32_t target_size, int32_t* out_w, int32_t* out_h);
+/* gray_out: the reference's datum['image'], rgb2gray's float64 output in [0, 1], photo after photo, each a row-major
+ * out_heights[b] x out_widths[b] plane (sum W' H' doubles, see vpk_prepared_size); out_widths / out_heights (B). */
+VPK_API int vpk_prepare_images(vpk_ctx* ctx, const uint8_t* rgb, const int64_t* byte_offsets, const int32_t* widths,
+                               const int32_t* heights, int32_t n_images, int32_t target_size, int32_t* out_widths,
+                               int32_t* out_heights, double* gray_out);
+/* vpk_prepare_images followed by vpk_pipeline_upload_images on the prepared planes times 255 (detect_lsd_lines' scaling,
+ * evaluation.py:229-231), on the device: the planes are written where the detector reads them, and the detector's
+ * frames are the prepared sizes.  Only the per-image counts and prepared sizes come back (each may be NULL);
+ * vpk_lsd_fetch returns the rows.  A sampled prepared side (ceil(side * scale)) must be below 65536. */
+VPK_API int vpk_pipeline_upload_photos(vpk_ctx* ctx, const uint8_t* rgb, const int64_t* byte_offsets, const int32_t* widths,
+                                       const int32_t* heights, int32_t n_images, int32_t target_size,
+                                       const vpk_lsd_config* cfg, int32_t* counts_out, int32_t* out_widths,
+                                       int32_t* out_heights);
+
 /* ---- N1: horizon line and orthogonal VP triplet --------------------------- */
 /* calc_horizon.calculate_horizon_and_ortho_vp(em_result, maxbest=10, theta_vmin=pi/10, theta_z=pi/4)
  * (reference calc_horizon.py:19-225; callers example.py:65, benchmark.py:233) for a batch of EM

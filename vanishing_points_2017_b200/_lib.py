@@ -23,6 +23,7 @@ SYMBOLS = [
     "vpk_pipeline_fetch", "vpk_pipeline_host", "vpk_pipeline_stage_ms", "vpk_horizon", "vpk_pipeline_horizon",
     "vpk_segments_from_lsd", "vpk_pipeline_upload_lsd",
     "vpk_lsd_default_config", "vpk_lsd", "vpk_lsd_fetch", "vpk_pipeline_upload_images",
+    "vpk_prepared_size", "vpk_prepare_images", "vpk_pipeline_upload_photos",
 ]
 PIX_U8, PIX_F64 = 0, 1
 
@@ -114,6 +115,11 @@ def load():
         lib.vpk_lsd_fetch.argtypes = [C.c_void_p, C.c_void_p]
         lib.vpk_pipeline_upload_images.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                                    C.c_int32, C.POINTER(LsdConfig), C.c_void_p]
+        lib.vpk_prepared_size.argtypes = [C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
+        lib.vpk_prepare_images.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
+                                           C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.vpk_pipeline_upload_photos.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                                   C.c_int32, C.POINTER(LsdConfig), C.c_void_p, C.c_void_p, C.c_void_p]
         lib.vpk_abi_version.argtypes = []
         lib.vpk_last_error.argtypes = []
         _lib = lib

@@ -186,12 +186,20 @@ __global__ void lsd_gather(const double* __restrict__ slab, const int32_t* __res
 
 static unsigned blocks(int64_t n) { return (unsigned)((n + kThreads - 1) / kThreads); }
 
-int lsd_dev(vpk_ctx* ctx, const void* images, int32_t dtype, const int64_t* pixel_offsets, const int32_t* widths,
-            const int32_t* heights, int32_t B, const vpk_lsd_config* cfg_in, int32_t* counts_out, const double** d_rows,
-            std::vector<int32_t>& row_offsets) {
-    vpk_lsd_config cfg;
+static Meta meta_view(const char* mp, int B) {
+    Meta m;
+    m.in_off = reinterpret_cast<const int64_t*>(mp);
+    m.aux_off = m.in_off + (B + 1); m.pix_off = m.aux_off + (B + 1); m.item_off = m.pix_off + (B + 1);
+    m.W = reinterpret_cast<const int32_t*>(m.item_off + (B + 1));
+    m.H = m.W + B; m.X = m.H + B; m.Y = m.X + B;
+    return m;
+}
+
+int lsd_plan(const int64_t* pixel_offsets, const int32_t* widths, const int32_t* heights, int32_t B, int32_t dtype,
+             const vpk_lsd_config* cfg_in, int32_t* counts_out, LsdPlan& p) {
+    vpk_lsd_config& cfg = p.cfg;
     if (cfg_in) cfg = *cfg_in; else vpk_lsd_default_config(&cfg);
-    if (!ctx || !pixel_offsets || !widths || !heights || B <= 0 || !counts_out) { set_error("vpk_lsd: bad argument"); return VPK_ERR_ARG; }
+    if (!pixel_offsets || !widths || !heights || B <= 0 || !counts_out) { set_error("vpk_lsd: bad argument"); return VPK_ERR_ARG; }
     if (dtype != VPK_PIX_U8 && dtype != VPK_PIX_F64) { set_error("vpk_lsd: dtype must be VPK_PIX_U8 or VPK_PIX_F64"); return VPK_ERR_ARG; }
     if (!(cfg.scale > 0.0) || !(cfg.sigma_scale > 0.0) || !(cfg.quant >= 0.0) || !(cfg.ang_th > 0.0 && cfg.ang_th < 180.0) ||
         !(cfg.density_th >= 0.0 && cfg.density_th <= 1.0) || cfg.n_bins <= 0 || cfg.n_bins > (1 << 24)) {
@@ -199,12 +207,13 @@ int lsd_dev(vpk_ctx* ctx, const void* images, int32_t dtype, const int64_t* pixe
         return VPK_ERR_ARG;
     }
     if (pixel_offsets[0] != 0) { set_error("vpk_lsd: pixel_offsets[0] must be 0"); return VPK_ERR_ARG; }
+    p.B = B; p.dtype = dtype;
     // geometry: int64 offsets for in / aux / pix / item, then W, H, X, Y
-    std::vector<int64_t> off64(4 * (size_t)(B + 1), 0);
-    std::vector<int32_t> dims(4 * (size_t)B);
-    int64_t *in_off = off64.data(), *aux_off = in_off + (B + 1), *pix_off = aux_off + (B + 1), *item_off = pix_off + (B + 1);
-    int maxX = 0, maxY = 0;
-    int64_t max_pix = 0;
+    p.off64.assign(4 * (size_t)(B + 1), 0);
+    p.dims.assign(4 * (size_t)B, 0);
+    int64_t *in_off = p.off64.data(), *aux_off = in_off + (B + 1), *pix_off = aux_off + (B + 1), *item_off = pix_off + (B + 1);
+    int32_t* dims = p.dims.data();
+    p.maxX = 0; p.maxY = 0; p.max_pix = 0;
     for (int b = 0; b < B; ++b) {
         const int W = widths[b], H = heights[b];
         if (W <= 0 || H <= 0 || pixel_offsets[b + 1] - pixel_offsets[b] != (int64_t)W * H) {
@@ -222,20 +231,26 @@ int lsd_dev(vpk_ctx* ctx, const void* images, int32_t dtype, const int64_t* pixe
         aux_off[b + 1] = aux_off[b] + (int64_t)X * H;
         pix_off[b + 1] = pix_off[b] + (int64_t)X * Y;
         item_off[b + 1] = item_off[b] + (X > 1 && Y > 1 ? (int64_t)(X - 1) * (Y - 1) : 0);
-        maxX = std::max(maxX, X); maxY = std::max(maxY, Y);
-        max_pix = std::max(max_pix, (int64_t)X * Y);
+        p.maxX = std::max(p.maxX, X); p.maxY = std::max(p.maxY, Y);
+        p.max_pix = std::max(p.max_pix, (int64_t)X * Y);
     }
+    if (item_off[B] > INT32_MAX) { set_error("vpk_lsd: %lld pixels in one call; split the batch below 2^31", (long long)item_off[B]); return VPK_ERR_ARG; }
+    return VPK_OK;
+}
+
+int lsd_input(vpk_ctx* ctx, const LsdPlan& p, void** d_in) {
+    const int B = p.B;
+    const int64_t* in_off = p.off64.data();
+    const int64_t *aux_off = in_off + (B + 1), *pix_off = aux_off + (B + 1), *item_off = pix_off + (B + 1);
     const int64_t n_in = in_off[B], n_pix = pix_off[B], n_items = item_off[B];
-    if (n_items > INT32_MAX) { set_error("vpk_lsd: %lld pixels in one call; split the batch below 2^31", (long long)n_items); return VPK_ERR_ARG; }
-    if (!images) { set_error("vpk_lsd: images is NULL"); return VPK_ERR_ARG; }
     VPK_CUDA(cudaSetDevice(ctx->device));
     if (!ctx->lsd) ctx->lsd = new LsdState();
     LsdState* s = ctx->lsd;
     s->B = 0; s->sumN = 0;
     cudaStream_t st = ctx->stream;
-    const size_t esz = dtype == VPK_PIX_U8 ? 1 : sizeof(double);
-    const bool sampled = cfg.scale != 1.0;
-    VPK_TRY(s->meta.ensure(off64.size() * sizeof(int64_t) + dims.size() * sizeof(int32_t)));
+    const size_t esz = p.dtype == VPK_PIX_U8 ? 1 : sizeof(double);
+    const bool sampled = p.cfg.scale != 1.0;
+    VPK_TRY(s->meta.ensure(p.off64.size() * sizeof(int64_t) + p.dims.size() * sizeof(int32_t)));
     VPK_TRY(s->in.ensure((size_t)n_in * esz));
     if (sampled) { VPK_TRY(s->aux.ensure((size_t)aux_off[B] * sizeof(double))); VPK_TRY(s->smp.ensure((size_t)n_pix * sizeof(double))); }
     VPK_TRY(s->ang.ensure((size_t)n_pix * sizeof(double)));
@@ -246,14 +261,25 @@ int lsd_dev(vpk_ctx* ctx, const void* images, int32_t dtype, const int64_t* pixe
     VPK_TRY(s->counts.ensure((size_t)B * sizeof(int32_t)));
     VPK_TRY(s->next.ensure(sizeof(int)));
     char* mp = s->meta.as<char>();
-    Meta m;
-    m.in_off = reinterpret_cast<const int64_t*>(mp);
-    m.aux_off = m.in_off + (B + 1); m.pix_off = m.aux_off + (B + 1); m.item_off = m.pix_off + (B + 1);
-    m.W = reinterpret_cast<const int32_t*>(m.item_off + (B + 1));
-    m.H = m.W + B; m.X = m.H + B; m.Y = m.X + B;
-    VPK_CUDA(cudaMemcpyAsync(mp, off64.data(), off64.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-    VPK_CUDA(cudaMemcpyAsync(mp + off64.size() * sizeof(int64_t), dims.data(), dims.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    if (n_in) VPK_CUDA(cudaMemcpyAsync(s->in.p, images, (size_t)n_in * esz, cudaMemcpyHostToDevice, st));
+    VPK_CUDA(cudaMemcpyAsync(mp, p.off64.data(), p.off64.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    VPK_CUDA(cudaMemcpyAsync(mp + p.off64.size() * sizeof(int64_t), p.dims.data(), p.dims.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    *d_in = s->in.p;
+    return VPK_OK;
+}
+
+int lsd_detect(vpk_ctx* ctx, const LsdPlan& p, int32_t* counts_out, const double** d_rows, std::vector<int32_t>& row_offsets) {
+    const int B = p.B;
+    const vpk_lsd_config& cfg = p.cfg;
+    const int32_t dtype = p.dtype;
+    const int64_t* in_off = p.off64.data();
+    const int64_t *aux_off = in_off + (B + 1), *pix_off = aux_off + (B + 1), *item_off = pix_off + (B + 1);
+    const int64_t n_pix = pix_off[B], n_items = item_off[B];
+    const int maxX = p.maxX, maxY = p.maxY;
+    const int64_t max_pix = p.max_pix;
+    LsdState* s = ctx->lsd;
+    cudaStream_t st = ctx->stream;
+    const bool sampled = cfg.scale != 1.0;
+    const Meta m = meta_view(s->meta.as<char>(), B);
     VPK_CUDA(cudaMemsetAsync(s->maxg.p, 0, (size_t)B * sizeof(unsigned long long), st));
 
     const double prec = lsd::dv(lsd::mul(lsd::kPi, cfg.ang_th), 180.0);
@@ -363,6 +389,21 @@ int lsd_dev(vpk_ctx* ctx, const void* images, int32_t dtype, const int64_t* pixe
     s->sumN = sumN;
     *d_rows = s->rows.as<double>();
     return VPK_OK;
+}
+
+int lsd_dev(vpk_ctx* ctx, const void* images, int32_t dtype, const int64_t* pixel_offsets, const int32_t* widths,
+            const int32_t* heights, int32_t B, const vpk_lsd_config* cfg_in, int32_t* counts_out, const double** d_rows,
+            std::vector<int32_t>& row_offsets) {
+    if (!ctx) { set_error("vpk_lsd: bad argument"); return VPK_ERR_ARG; }
+    LsdPlan p;
+    VPK_TRY(lsd_plan(pixel_offsets, widths, heights, B, dtype, cfg_in, counts_out, p));
+    if (!images) { set_error("vpk_lsd: images is NULL"); return VPK_ERR_ARG; }
+    void* d_in = nullptr;
+    VPK_TRY(lsd_input(ctx, p, &d_in));
+    const int64_t n_in = p.off64[B];
+    const size_t esz = dtype == VPK_PIX_U8 ? 1 : sizeof(double);
+    if (n_in) VPK_CUDA(cudaMemcpyAsync(d_in, images, (size_t)n_in * esz, cudaMemcpyHostToDevice, ctx->stream));
+    return lsd_detect(ctx, p, counts_out, d_rows, row_offsets);
 }
 
 }  // namespace vpk

@@ -35,6 +35,33 @@ void pipe_free(vpk_ctx* ctx) {
     ctx->pipe = nullptr;
 }
 
+// The detector's rows (d_rows, image b's from row_off[b]) into the resident batch: normalised where they are
+// (widths / heights: the frames the detector saw), they never leave the device
+static int upload_detected(vpk_ctx* ctx, const double* d_rows, const std::vector<int32_t>& row_off, const int32_t* widths,
+                           const int32_t* heights, int32_t B) {
+    if (!ctx->pipe) {
+        ctx->pipe = new PipeState();
+        for (auto& e : ctx->pipe->ev) VPK_CUDA(cudaEventCreate(&e));
+    }
+    PipeState* p = ctx->pipe;
+    const int64_t sumN = row_off[B];
+    p->B = B; p->sumN = sumN; p->have_result = false;
+    p->h_offsets = row_off;
+    VPK_TRY(p->seg.ensure((sumN + 1) * 4 * sizeof(double)));
+    VPK_TRY(p->lines.ensure((sumN + 1) * 3 * sizeof(double)));
+    VPK_TRY(p->offsets.ensure((size_t)(3 * (B + 1)) * sizeof(int32_t)));
+    int32_t* d_off = p->offsets.as<int32_t>();
+    int32_t* d_w = d_off + (B + 1);
+    int32_t* d_h = d_w + (B + 1);
+    cudaStream_t st = ctx->stream;
+    VPK_CUDA(cudaMemcpyAsync(d_off, row_off.data(), (B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    VPK_CUDA(cudaMemcpyAsync(d_w, widths, B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    VPK_CUDA(cudaMemcpyAsync(d_h, heights, B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    VPK_TRY(segments_from_lsd_dev(ctx, d_rows, 7, d_off, d_w, d_h, B, sumN, p->seg.as<double>(), nullptr));
+    VPK_CUDA(cudaStreamSynchronize(st));
+    return VPK_OK;
+}
+
 }  // namespace vpk
 
 using namespace vpk;
@@ -102,28 +129,30 @@ int vpk_pipeline_upload_images(vpk_ctx* ctx, const void* images, int32_t dtype, 
     std::vector<int32_t> counts(B), row_off;
     const double* d_rows = nullptr;
     VPK_TRY(lsd_dev(ctx, images, dtype, pixel_offsets, widths, heights, B, cfg, counts.data(), &d_rows, row_off));
-    if (!ctx->pipe) {
-        ctx->pipe = new PipeState();
-        for (auto& e : ctx->pipe->ev) VPK_CUDA(cudaEventCreate(&e));
-    }
-    PipeState* p = ctx->pipe;
-    const int64_t sumN = row_off[B];
-    p->B = B; p->sumN = sumN; p->have_result = false;
-    p->h_offsets = row_off;
-    VPK_TRY(p->seg.ensure((sumN + 1) * 4 * sizeof(double)));
-    VPK_TRY(p->lines.ensure((sumN + 1) * 3 * sizeof(double)));
-    VPK_TRY(p->offsets.ensure((size_t)(3 * (B + 1)) * sizeof(int32_t)));
-    int32_t* d_off = p->offsets.as<int32_t>();
-    int32_t* d_w = d_off + (B + 1);
-    int32_t* d_h = d_w + (B + 1);
-    cudaStream_t st = ctx->stream;
-    VPK_CUDA(cudaMemcpyAsync(d_off, row_off.data(), (B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    VPK_CUDA(cudaMemcpyAsync(d_w, widths, B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    VPK_CUDA(cudaMemcpyAsync(d_h, heights, B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    // the detector's rows are normalised where they are: they never leave the device
-    VPK_TRY(segments_from_lsd_dev(ctx, d_rows, 7, d_off, d_w, d_h, B, sumN, p->seg.as<double>(), nullptr));
-    VPK_CUDA(cudaStreamSynchronize(st));
+    VPK_TRY(upload_detected(ctx, d_rows, row_off, widths, heights, B));
     if (counts_out) memcpy(counts_out, counts.data(), (size_t)B * sizeof(int32_t));
+    return VPK_OK;
+}
+
+int vpk_pipeline_upload_photos(vpk_ctx* ctx, const uint8_t* rgb, const int64_t* byte_offsets, const int32_t* widths,
+                               const int32_t* heights, int32_t B, int32_t target_size, const vpk_lsd_config* cfg,
+                               int32_t* counts_out, int32_t* out_widths, int32_t* out_heights) {
+    if (!ctx) { set_error("vpk_pipeline_upload_photos: bad argument"); return VPK_ERR_ARG; }
+    PrepPlan pp;
+    VPK_TRY(prep_plan(rgb, byte_offsets, widths, heights, B, target_size, "vpk_pipeline_upload_photos", pp));
+    // the detector reads the prepared planes (float64, x 255) where the preparation kernel writes them
+    std::vector<int32_t> counts(B), row_off;
+    LsdPlan lp;
+    VPK_TRY(lsd_plan(pp.pix_off.data(), pp.W.data(), pp.H.data(), B, VPK_PIX_F64, cfg, counts.data(), lp));
+    void* d_in = nullptr;
+    VPK_TRY(lsd_input(ctx, lp, &d_in));
+    VPK_TRY(prep_run(ctx, pp, rgb, 255.0, static_cast<double*>(d_in)));
+    const double* d_rows = nullptr;
+    VPK_TRY(lsd_detect(ctx, lp, counts.data(), &d_rows, row_off));
+    VPK_TRY(upload_detected(ctx, d_rows, row_off, pp.W.data(), pp.H.data(), B));
+    if (counts_out) memcpy(counts_out, counts.data(), (size_t)B * sizeof(int32_t));
+    if (out_widths) memcpy(out_widths, pp.W.data(), (size_t)B * sizeof(int32_t));
+    if (out_heights) memcpy(out_heights, pp.H.data(), (size_t)B * sizeof(int32_t));
     return VPK_OK;
 }
 

@@ -87,6 +87,7 @@ struct CnnState;   // cnn.cu
 struct EmState;    // em.cu
 struct PipeState;  // pipeline.cu
 struct LsdState;   // lsd.cu
+struct PrepState;  // image_prep.cu
 
 }  // namespace vpk
 
@@ -115,6 +116,7 @@ struct vpk_ctx {
     vpk::EmState* em = nullptr;
     vpk::PipeState* pipe = nullptr;
     vpk::LsdState* lsd = nullptr;
+    vpk::PrepState* prep = nullptr;
 };
 
 namespace vpk {
@@ -204,10 +206,39 @@ void horizon_unpack(const void* h_rec, int32_t B, double* points, int32_t* best_
 int lsd_dev(vpk_ctx* ctx, const void* images, int32_t dtype, const int64_t* pixel_offsets, const int32_t* widths,
             const int32_t* heights, int32_t B, const vpk_lsd_config* cfg, int32_t* counts_out, const double** d_rows,
             std::vector<int32_t>& row_offsets);
+// The same in three steps, for input that is produced on the device: lsd_plan validates the call and lays out
+// its geometry (host only), lsd_input sizes the workspaces and returns the device buffer the detector reads
+// (row-major pixels of type `dtype` at pixel_offsets), lsd_detect runs the detector on what was written there.
+struct LsdPlan {
+    vpk_lsd_config cfg;
+    int32_t B = 0, dtype = 0;
+    std::vector<int64_t> off64;     // offsets (B+1 each) of the input, x-pass, sampled-pixel and seed-item arrays
+    std::vector<int32_t> dims;      // W, H, X, Y (B each)
+    int maxX = 0, maxY = 0;
+    int64_t max_pix = 0;
+};
+int lsd_plan(const int64_t* pixel_offsets, const int32_t* widths, const int32_t* heights, int32_t B, int32_t dtype,
+             const vpk_lsd_config* cfg, int32_t* counts_out, LsdPlan& plan);
+int lsd_input(vpk_ctx* ctx, const LsdPlan& plan, void** d_in);
+int lsd_detect(vpk_ctx* ctx, const LsdPlan& plan, int32_t* counts_out, const double** d_rows, std::vector<int32_t>& row_offsets);
+
+// image_prep.cu: resize (INTER_AREA) + rgb2gray of a ragged batch of uint8 RGB photos.  prep_plan validates the
+// call and computes the prepared sizes (host only); prep_run copies the photos to the device and writes the float64
+// gray planes, multiplied by out_scale, to d_out (image b's W'*H' plane at plan.pix_off[b]).
+struct PrepPlan {
+    int32_t B = 0;
+    std::vector<int32_t> w, h, W, H;
+    std::vector<int64_t> src_off;   // B+1 byte offsets of the photos
+    std::vector<int64_t> pix_off;   // B+1 pixel offsets of the prepared planes
+};
+int prep_plan(const uint8_t* rgb, const int64_t* byte_offsets, const int32_t* widths, const int32_t* heights, int32_t B,
+              int32_t target_size, const char* who, PrepPlan& plan);
+int prep_run(vpk_ctx* ctx, const PrepPlan& plan, const uint8_t* rgb, double out_scale, double* d_out);
 
 void cnn_free(vpk_ctx* ctx);
 void em_free(vpk_ctx* ctx);
 void pipe_free(vpk_ctx* ctx);
 void lsd_free(vpk_ctx* ctx);
+void prep_free(vpk_ctx* ctx);
 
 }  // namespace vpk

@@ -85,6 +85,28 @@ class Pipeline:
         self._off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
         return counts
 
+    def upload_photos(self, photos, target_size=None, **lsd_kwargs):
+        """upload_images() from RGB photos (a list of (H, W, 3) uint8 arrays of any sizes): the preparation of
+        evaluation.py:139-154 (images.prepare_images: resize to `target_size`, rgb2gray), LSD on the gray planes
+        times 255 and the normalisation run on the device; the photos cross PCIe as uint8 RGB and nothing but the
+        per-image counts and sizes comes back.  Returns (counts, shapes): shapes are the prepared (H', W') pairs,
+        the frames the segments are normalised in (horizons(image_heights=...), evaluation.reference_data)."""
+        from .images import pack_photos, _target
+        flat, off, w, h = pack_photos(photos)
+        if len(w) == 0:
+            raise ValueError("upload_photos needs at least one photo")
+        cfg = _lib.lsd_config(**lsd_kwargs)
+        B = len(w)
+        counts = np.empty(B, np.int32)
+        ow = np.empty(B, np.int32)
+        oh = np.empty(B, np.int32)
+        _lib.check(self.ctx.lib.vpk_pipeline_upload_photos(self.ctx.h, _lib.ptr(flat), _lib.ptr(off), _lib.ptr(w), _lib.ptr(h), B,
+                                                           _target(target_size), C.byref(cfg), _lib.ptr(counts), _lib.ptr(ow),
+                                                           _lib.ptr(oh)), "vpk_pipeline_upload_photos")
+        self._B = B
+        self._off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
+        return counts, [(int(a), int(b)) for a, b in zip(oh, ow)]
+
     def run(self):
         _lib.check(self.ctx.lib.vpk_pipeline_run(self.ctx.h, self.size, self.mode, self.alpha, C.byref(self.cfg)),
                    "vpk_pipeline_run")

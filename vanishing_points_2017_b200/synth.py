@@ -86,22 +86,20 @@ def lines_from_segments(seg):
     return np.stack([y1 - y2, x2 - x1, x1 * y2 - y1 * x2], axis=1)
 
 
-def render_scene(seed, n_segments, width=640, height=480, noise_sigma=2.0, line_width=2.5):
-    """A grayscale (height, width) float64 image of make_scene(seed, n_segments, width, height)'s segments: each is
-    an anti-aliased bar `line_width` px wide (coverage falls off linearly over one pixel at its border) darker or
-    brighter than a uniform background by a random contrast, plus Gaussian noise of `noise_sigma`, clipped to
-    0..255.  Integer-valued (rounded), so the uint8 and float64 copies of it are the same image.  The LSD tests and
-    tools/lsd_bench.py render their inputs here."""
-    sc = make_scene(seed, n_segments, width, height)
-    rs = np.random.RandomState(seed + 7919)
+def _pixel_segments(sc, width, height):
+    """make_scene's segments in pixels (inverse of evaluation.py:240-249)."""
     s = float(max(width, height))
     seg = sc["segments"].copy()
-    seg[:, [0, 2]] = seg[:, [0, 2]] * (s / 2.0) + width / 2.0        # inverse of evaluation.py:240-249
+    seg[:, [0, 2]] = seg[:, [0, 2]] * (s / 2.0) + width / 2.0
     seg[:, [1, 3]] = -seg[:, [1, 3]] * (s / 2.0) + height / 2.0
-    img = np.full((height, width), rs.uniform(70.0, 180.0))
-    contrast = rs.uniform(25.0, 70.0, seg.shape[0]) * rs.choice([-1.0, 1.0], seg.shape[0])
+    return seg
+
+
+def _bars(seg, width, height, line_width):
+    """(rows, cols, coverage) of every anti-aliased bar `line_width` px wide along seg (pixels); coverage falls off
+    linearly over one pixel at the border.  Segments outside the image yield nothing."""
     hw = 0.5 * line_width
-    for (x1, y1, x2, y2), c in zip(seg, contrast):
+    for k, (x1, y1, x2, y2) in enumerate(seg):
         x0, x9 = int(max(np.floor(min(x1, x2) - hw - 1), 0)), int(min(np.ceil(max(x1, x2) + hw + 1), width - 1))
         y0, y9 = int(max(np.floor(min(y1, y2) - hw - 1), 0)), int(min(np.ceil(max(y1, y2) + hw + 1), height - 1))
         if x9 < x0 or y9 < y0:
@@ -111,10 +109,44 @@ def render_scene(seed, n_segments, width=640, height=480, noise_sigma=2.0, line_
         L2 = dx * dx + dy * dy
         t = np.clip(((xx - x1) * dx + (yy - y1) * dy) / max(L2, 1e-12), 0.0, 1.0)
         d = np.hypot(xx - (x1 + t * dx), yy - (y1 + t * dy))
-        cov = np.clip(hw + 0.5 - d, 0.0, 1.0)
-        img[y0:y9 + 1, x0:x9 + 1] += c * cov
+        yield k, slice(y0, y9 + 1), slice(x0, x9 + 1), np.clip(hw + 0.5 - d, 0.0, 1.0)
+
+
+def render_scene(seed, n_segments, width=640, height=480, noise_sigma=2.0, line_width=2.5):
+    """A grayscale (height, width) float64 image of make_scene(seed, n_segments, width, height)'s segments: each is
+    an anti-aliased bar `line_width` px wide (coverage falls off linearly over one pixel at its border) darker or
+    brighter than a uniform background by a random contrast, plus Gaussian noise of `noise_sigma`, clipped to
+    0..255.  Integer-valued (rounded), so the uint8 and float64 copies of it are the same image.  The LSD tests and
+    tools/lsd_bench.py render their inputs here."""
+    sc = make_scene(seed, n_segments, width, height)
+    rs = np.random.RandomState(seed + 7919)
+    seg = _pixel_segments(sc, width, height)
+    img = np.full((height, width), rs.uniform(70.0, 180.0))
+    contrast = rs.uniform(25.0, 70.0, seg.shape[0]) * rs.choice([-1.0, 1.0], seg.shape[0])
+    for k, ys, xs, cov in _bars(seg, width, height, line_width):
+        img[ys, xs] += contrast[k] * cov
     img += rs.normal(0.0, noise_sigma, img.shape)
     return np.clip(np.round(img), 0.0, 255.0)
+
+
+def render_photo(seed, n_segments, width=2000, height=1333, noise_sigma=2.0, line_width=None):
+    """An RGB (height, width, 3) uint8 photo of make_scene(seed, n_segments, width, height)'s segments:
+    render_scene's bars (`line_width` defaults to 2.5 px per 640 px of the longer side, so the scene looks the same
+    after resizing to 640) on a uniform background of a random colour, each bar with its own contrast per channel,
+    plus independent Gaussian noise of `noise_sigma` per channel, rounded and clipped to 0..255.  The photo
+    preparation tests and tools/image_prep_bench.py render their inputs here."""
+    sc = make_scene(seed, n_segments, width, height)
+    rs = np.random.RandomState(seed + 7927)
+    if line_width is None:
+        line_width = 2.5 * max(width, height) / 640.0
+    seg = _pixel_segments(sc, width, height)
+    img = np.empty((height, width, 3))
+    img[:] = rs.uniform(70.0, 180.0, 3)
+    contrast = rs.uniform(25.0, 70.0, (seg.shape[0], 3)) * rs.choice([-1.0, 1.0], (seg.shape[0], 1))
+    for k, ys, xs, cov in _bars(seg, width, height, line_width):
+        img[ys, xs, :] += cov[:, :, None] * contrast[k]
+    img += rs.normal(0.0, noise_sigma, img.shape)
+    return np.clip(np.round(img), 0.0, 255.0).astype(np.uint8)
 
 
 def ideal_response(vps, grid=20, seed=0, peak=0.9, noise=0.05):
