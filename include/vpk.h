@@ -102,6 +102,28 @@ VPK_API int vpk_cnn_load(vpk_ctx* ctx, const float* const* weights, const float*
  * (fc8 before the sigmoid) may be NULL. */
 VPK_API int vpk_cnn_forward(vpk_ctx* ctx, const uint8_t* images, int32_t n_images, float* sigout, float* logits_out);
 
+/* Diagnostics: raw copy of activation buffer `which` (VPK_CNN_BUF_*) of the last chunk (up to 1024 images) the last
+ * vpk_cnn_forward ran, for its first n_images images (<= that chunk's size), in the device layout: padding rings and
+ * group padding included.  Per image, row-major, NHWC:
+ *   A1     bf16 (125, 125, 64)  conv1 operand: [Y, X, kwb*16 + dy*4 + dx] = image[4Y+dy, 4(X+kwb)+dx] - mean,
+ *                               0 where X + kwb > 124
+ *   C1     bf16 (123, 123, 96)  conv1 + ReLU + norm1
+ *   A2     bf16 (65, 65, 128)   pool1, zero ring of 2; channel c of group c / 48 at (c / 48) * 64 + c % 48
+ *   C2     bf16 (61, 61, 256)   conv2 + ReLU + norm2
+ *   A3     bf16 (32, 32, 256)   pool2, zero ring of 1
+ *   A4     bf16 (32, 32, 384)   conv3 + ReLU, zero ring of 1
+ *   A5     bf16 (32, 32, 384)   conv4 + ReLU, zero ring of 1
+ *   C5     bf16 (30, 30, 256)   conv5 + ReLU
+ *   A6     bf16 (15, 15, 256)   pool5 = fc6 input (fc6's K runs over (y, x, c), Caffe's over (c, y, x))
+ *   F6, F7 bf16 (4096)          fc6 / fc7 + ReLU
+ *   LOGITS float32 (400)        fc8
+ *   SIG    float32 (400)        sigmoid of fc8
+ * Fails with VPK_ERR_STATE if no vpk_cnn_forward ran since the context's CNN was created or a pipeline run reused
+ * the buffers, and with VPK_ERR_ARG for a bad `which` or too many images. */
+enum { VPK_CNN_BUF_A1 = 0, VPK_CNN_BUF_C1, VPK_CNN_BUF_A2, VPK_CNN_BUF_C2, VPK_CNN_BUF_A3, VPK_CNN_BUF_A4, VPK_CNN_BUF_A5,
+       VPK_CNN_BUF_C5, VPK_CNN_BUF_A6, VPK_CNN_BUF_F6, VPK_CNN_BUF_F7, VPK_CNN_BUF_LOGITS, VPK_CNN_BUF_SIG, VPK_CNN_NBUF };
+VPK_API int vpk_cnn_debug_fetch(vpk_ctx* ctx, int32_t which, int32_t n_images, void* out);
+
 /* Diagnostics: one plain GEMM out = act(a * b^T + bias) through the tcgen05 kernel every
  * CNN layer uses.  a (m,k) and b (n,k) are bf16 bit patterns, out (m,n) float32;
  * k % 64 == 0, bn % 16 == 0, 16 <= bn <= 256, n % bn == 0.  ksplit > 1: the K range is dealt to

@@ -56,11 +56,13 @@ def forward(images, weights, biases, mean=None, return_layers=False):
         x = F.relu(F.conv2d(x, w[0], b[0], stride=4))                              # deploy.prototxt:9-33
         layers["conv1"] = x
         x = F.local_response_norm(x, 5, alpha=1e-4, beta=0.75, k=1.0)              # :34-44
+        layers["norm1"] = x
         x = F.max_pool2d(x, 3, 2, ceil_mode=True)                                  # :45-55
         layers["pool1"] = x
         x = F.relu(F.conv2d(x, w[1], b[1], padding=2, groups=2))                   # :56-81
         layers["conv2"] = x
         x = F.local_response_norm(x, 5, alpha=1e-4, beta=0.75, k=1.0)              # :82-92
+        layers["norm2"] = x
         x = F.max_pool2d(x, 3, 2, ceil_mode=True)                                  # :93-103
         layers["pool2"] = x
         x = F.relu(F.conv2d(x, w[2], b[2], padding=1))                             # :104-128

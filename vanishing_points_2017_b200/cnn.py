@@ -40,6 +40,7 @@ class Net:
     def __init__(self, ctx, weights, biases):
         self.ctx = ctx
         self._mean_loaded = None
+        self._last_chunk = 0
         self._w = [np.ascontiguousarray(w, dtype=np.float32) for w in weights]
         self._b = [np.ascontiguousarray(b, dtype=np.float32) for b in biases]
         for w, shape in zip(self._w, LAYER_SHAPES):
@@ -68,7 +69,35 @@ class Net:
         logits = np.empty((n, 400), dtype=np.float32) if want_logits else None
         _lib.check(self.ctx.lib.vpk_cnn_forward(self.ctx.h, _lib.ptr(images), n, _lib.ptr(sig), _lib.ptr(logits)),
                    "vpk_cnn_forward")
+        if n:
+            self._last_chunk = (n - 1) % 1024 + 1          # vpk_cnn_forward runs the batch in chunks of 1024
         return (sig, logits) if want_logits else sig
+
+    def debug_activations(self, which, n=None, raw=False):
+        """Activation buffer `which` (a name of ACTIVATIONS) of the last chunk forward_batch ran (its last 1024 or
+        fewer images), copied as the device holds it: padding rings and group padding included (layouts in
+        include/vpk.h).  Returns an (n, H, W, C) array for the convolution buffers, (n, K) for f6 / f7 / logits / sig;
+        bf16 buffers as float32, or as their uint16 bit patterns with raw=True.  n defaults to the whole chunk."""
+        index, shape, is_bf16 = ACTIVATIONS[which]
+        if n is None:
+            n = self._last_chunk
+        out = np.empty((n,) + shape, dtype=np.uint16 if is_bf16 else np.float32)
+        _lib.check(self.ctx.lib.vpk_cnn_debug_fetch(self.ctx.h, index, int(n), _lib.ptr(out)), "vpk_cnn_debug_fetch")
+        return out if raw or not is_bf16 else bf16_bits_to_float(out)
+
+
+# name -> (vpk_cnn_debug_fetch index, per-image shape, bf16?)   (include/vpk.h, VPK_CNN_BUF_*)
+ACTIVATIONS = {
+    "a1": (0, (125, 125, 64), True), "c1": (1, (123, 123, 96), True), "a2": (2, (65, 65, 128), True),
+    "c2": (3, (61, 61, 256), True), "a3": (4, (32, 32, 256), True), "a4": (5, (32, 32, 384), True),
+    "a5": (6, (32, 32, 384), True), "c5": (7, (30, 30, 256), True), "a6": (8, (15, 15, 256), True),
+    "f6": (9, (4096,), True), "f7": (10, (4096,), True), "logits": (11, (400,), False), "sig": (12, (400,), False),
+}
+
+
+def bf16_bits_to_float(bits):
+    """uint16 bf16 bit patterns -> float32 (exact)."""
+    return (np.asarray(bits, dtype=np.uint16).astype(np.uint32) << 16).view(np.float32)
 
 
 def init_caffe(model_def=None, model_weights=None, gpu_id=0):

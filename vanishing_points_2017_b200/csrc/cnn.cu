@@ -33,6 +33,7 @@ struct CnnState {
     // activations (sized for `cap` images)
     int cap = 0;
     DBuf a1, c1, a2, c2, a3, a4, a5, c5, a6, f6, f7, logits, sig, img, splitk;
+    int last_n = 0;                                          // images of the last chunk vpk_cnn_forward ran (0: none, see vpk_cnn_debug_fetch)
 };
 
 void cnn_free(vpk_ctx* ctx) {
@@ -389,6 +390,7 @@ int cnn_forward_dev(vpk_ctx* ctx, const uint8_t* d_images, int32_t n, float* d_s
     CnnState* s = ctx->cnn;
     if (!s || !s->loaded) { set_error("vpk_cnn_forward: call vpk_cnn_load first"); return VPK_ERR_STATE; }
     if (n <= 0) return VPK_OK;
+    s->last_n = 0;                                         // the buffers no longer hold what vpk_cnn_forward left (sigout may go elsewhere)
     VPK_TRY(ensure_activations(ctx, n));
     s->persistent = !(getenv("VPK_GEMM_PERSIST") && atoi(getenv("VPK_GEMM_PERSIST")) == 0);      // A/B switch, default on
     typedef __nv_bfloat16 bf;
@@ -558,7 +560,29 @@ int vpk_cnn_forward(vpk_ctx* ctx, const uint8_t* images, int32_t n, float* sigou
         if (logits_out)
             VPK_CUDA(cudaMemcpyAsync(logits_out + (size_t)i0 * 400, s->logits.p, (size_t)nb * 400 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
         VPK_CUDA(cudaStreamSynchronize(ctx->stream));
+        s->last_n = nb;
     }
+    return VPK_OK;
+}
+
+// Diagnostics: raw copy of one activation buffer of the last chunk vpk_cnn_forward ran (layouts in vpk.h).
+int vpk_cnn_debug_fetch(vpk_ctx* ctx, int32_t which, int32_t n_images, void* out) {
+    if (!ctx || !out || which < 0 || which >= VPK_CNN_NBUF || n_images < 0) { set_error("vpk_cnn_debug_fetch: bad argument"); return VPK_ERR_ARG; }
+    CnnState* s = ctx->cnn;
+    if (!s || s->last_n <= 0) { set_error("vpk_cnn_debug_fetch: no vpk_cnn_forward since the last load or pipeline run"); return VPK_ERR_STATE; }
+    if (n_images > s->last_n) {
+        set_error("vpk_cnn_debug_fetch: %d images asked for, the last chunk had %d", n_images, s->last_n);
+        return VPK_ERR_ARG;
+    }
+    // per-image bytes, in the order of the VPK_CNN_BUF_* enum
+    static const size_t per_image[VPK_CNN_NBUF] = {15625 * 64 * 2, 123 * 123 * 96 * 2, 65 * 65 * 128 * 2, 61 * 61 * 256 * 2,
+                                                   32 * 32 * 256 * 2, 32 * 32 * 384 * 2, 32 * 32 * 384 * 2, 30 * 30 * 256 * 2,
+                                                   57600 * 2, 4096 * 2, 4096 * 2, 400 * 4, 400 * 4};
+    const DBuf* bufs[VPK_CNN_NBUF] = {&s->a1, &s->c1, &s->a2, &s->c2, &s->a3, &s->a4, &s->a5, &s->c5, &s->a6, &s->f6, &s->f7, &s->logits, &s->sig};
+    if (n_images == 0) return VPK_OK;
+    VPK_CUDA(cudaSetDevice(ctx->device));
+    VPK_CUDA(cudaMemcpyAsync(out, bufs[which]->p, per_image[which] * n_images, cudaMemcpyDeviceToHost, ctx->stream));
+    VPK_CUDA(cudaStreamSynchronize(ctx->stream));
     return VPK_OK;
 }
 
