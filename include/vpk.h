@@ -281,6 +281,50 @@ VPK_API int vpk_pipeline_upload_photos(vpk_ctx* ctx, const uint8_t* rgb, const i
                                        const vpk_lsd_config* cfg, int32_t* counts_out, int32_t* out_widths,
                                        int32_t* out_heights);
 
+/* ---- N6: JPEG decoding in front of photo preparation ---------------------------- */
+/* The read of the dataset's JPEG files by `convert` (reference evaluation.py:142-143), on the device and bit for bit
+ * with libjpeg-turbo 3.1's default decode (islow IDCT, fancy upsampling, jdcolor.c's YCbCr -> RGB); DESIGN.md
+ * section 4.8.  Decoded: baseline and extended sequential Huffman JPEG (SOF0 / SOF1), 8-bit, one interleaved scan,
+ * 3 components in YCbCr or 1 component (gray), sampling factors up to 4 with integer ratios, restart intervals.
+ * EXIF orientation is ignored (the stored orientation, as `convert` without -auto-orient sees it).
+ * Files: host array `data`, file b the byte_offsets[b] .. byte_offsets[b+1] bytes (B+1 non-decreasing entries). */
+enum {
+    VPK_JPEG_OK = 0,
+    VPK_JPEG_PROGRESSIVE = 1,   /* SOF2 */
+    VPK_JPEG_ARITHMETIC = 2,    /* SOF9..SOF15, DAC */
+    VPK_JPEG_PRECISION = 3,     /* not 8-bit samples */
+    VPK_JPEG_COLOR = 4,         /* CMYK / YCCK (4 components), or RGB (Adobe transform 0, or component IDs 'R','G','B') */
+    VPK_JPEG_LAYOUT = 5,        /* 2 components, a scan without every component (multi-scan), fractional sampling, DNL */
+    VPK_JPEG_MALFORMED = 6,     /* markers the parser cannot follow: truncated or overrunning segments, missing tables */
+    VPK_JPEG_LOSSLESS = 7,      /* lossless or hierarchical process (SOF3, SOF5..SOF7, DHP, EXP) */
+    VPK_JPEG_CORRUPT = 8        /* status after decoding: the entropy-coded data is inconsistent (ends before the last
+                                 * block, a code not in its table, a run past coefficient 63, data left over, RSTn out
+                                 * of sequence); the photo's pixels are unspecified but deterministic */
+};
+/* Reads the markers of every file up to its SOS segment, never the entropy-coded data; host only, needs no device or
+ * context.  widths / heights / components (B, each may be NULL) receive the frame's size and component count (0
+ * unless the parser read a SOF0 / SOF1 frame header); support (B, may be NULL) VPK_JPEG_OK or the reason a file is refused. */
+VPK_API int vpk_jpeg_info(const uint8_t* data, const int64_t* byte_offsets, int32_t n, int32_t* widths, int32_t* heights,
+                          int32_t* components, int32_t* support);
+/* Decodes every file on the device.  pixels_out: photo after photo, row-major height x width x components bytes (RGB,
+ * or gray for 1 component); status_out (B): VPK_JPEG_OK or VPK_JPEG_CORRUPT.  Fails with VPK_ERR_ARG before any
+ * device work, naming the first refused file and its reason. */
+VPK_API int vpk_decode_jpegs(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t n, uint8_t* pixels_out,
+                             int32_t* status_out);
+/* vpk_decode_jpegs followed by vpk_pipeline_upload_photos on the decoded photos, on the device: only the files cross
+ * PCIe, the decoder writes the RGB photos where the preparation kernel reads them.  counts_out / out_widths /
+ * out_heights as vpk_pipeline_upload_photos, status_out (B) as vpk_decode_jpegs (each may be NULL; a CORRUPT photo's
+ * rows come from its unspecified pixels).  A refused file or a 1-component file (gray photos cannot be prepared)
+ * fails the call with VPK_ERR_ARG, naming its index and reason. */
+VPK_API int vpk_pipeline_upload_jpegs(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t n,
+                                      int32_t target_size, const vpk_lsd_config* cfg, int32_t* counts_out,
+                                      int32_t* out_widths, int32_t* out_heights, int32_t* status_out);
+/* Decoder statistics of the last decode on this context: out[0] subsequences, out[1] subsequences re-decoded after
+ * their first decode (the synchronisation work), out[2] the most synchronisation rounds inside one CTA, out[3] extra
+ * launches across CTAs.  out[1] and out[2] are counted only while profiling is enabled (vpk_profile_enable), 0
+ * otherwise.  Fails with VPK_ERR_STATE before any decode. */
+VPK_API int vpk_jpeg_stats(vpk_ctx* ctx, int64_t* out);
+
 /* ---- N1: horizon line and orthogonal VP triplet --------------------------- */
 /* calc_horizon.calculate_horizon_and_ortho_vp(em_result, maxbest=10, theta_vmin=pi/10, theta_z=pi/4)
  * (reference calc_horizon.py:19-225; callers example.py:65, benchmark.py:233) for a batch of EM

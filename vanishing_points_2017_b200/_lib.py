@@ -24,8 +24,12 @@ SYMBOLS = [
     "vpk_segments_from_lsd", "vpk_pipeline_upload_lsd",
     "vpk_lsd_default_config", "vpk_lsd", "vpk_lsd_fetch", "vpk_pipeline_upload_images",
     "vpk_prepared_size", "vpk_prepare_images", "vpk_pipeline_upload_photos",
+    "vpk_jpeg_info", "vpk_decode_jpegs", "vpk_pipeline_upload_jpegs", "vpk_jpeg_stats",
 ]
 PIX_U8, PIX_F64 = 0, 1
+# vpk.h VPK_JPEG_*: support codes of vpk_jpeg_info and the decode status
+JPEG_REASONS = ["ok", "progressive", "arithmetic", "precision", "color", "layout", "malformed", "lossless", "corrupt"]
+JPEG_OK, JPEG_CORRUPT = 0, 8
 
 
 class VpkError(RuntimeError):
@@ -121,6 +125,11 @@ def load():
                                            C.c_void_p, C.c_void_p, C.c_void_p]
         lib.vpk_pipeline_upload_photos.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                                    C.c_int32, C.POINTER(LsdConfig), C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.vpk_jpeg_info.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.vpk_decode_jpegs.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
+        lib.vpk_pipeline_upload_jpegs.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(LsdConfig),
+                                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.vpk_jpeg_stats.argtypes = [C.c_void_p, C.c_void_p]
         lib.vpk_abi_version.argtypes = []
         lib.vpk_last_error.argtypes = []
         _lib = lib

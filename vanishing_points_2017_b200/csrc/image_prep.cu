@@ -200,7 +200,7 @@ static void prepared_size(int w, int h, int target, int* W, int* H) {
     *H = std::max(1, (int)nearbyint(h * s));
 }
 
-int prep_plan(const uint8_t* rgb, const int64_t* byte_offsets, const int32_t* widths, const int32_t* heights, int32_t B,
+int prep_plan(const int64_t* byte_offsets, const int32_t* widths, const int32_t* heights, int32_t B,
               int32_t target_size, const char* who, PrepPlan& p) {
     if (!byte_offsets || !widths || !heights || B <= 0) { set_error("%s: bad argument", who); return VPK_ERR_ARG; }
     if (byte_offsets[0] != 0) { set_error("%s: byte_offsets[0] must be 0", who); return VPK_ERR_ARG; }
@@ -218,7 +218,14 @@ int prep_plan(const uint8_t* rgb, const int64_t* byte_offsets, const int32_t* wi
         prepared_size(w, h, target_size, &p.W[b], &p.H[b]);
         p.pix_off[b + 1] = p.pix_off[b] + (int64_t)p.W[b] * p.H[b];
     }
-    if (!rgb) { set_error("%s: rgb is NULL", who); return VPK_ERR_ARG; }
+    return VPK_OK;
+}
+
+int prep_input(vpk_ctx* ctx, const PrepPlan& p, uint8_t** d_rgb) {
+    VPK_CUDA(cudaSetDevice(ctx->device));
+    if (!ctx->prep) ctx->prep = new PrepState();
+    VPK_TRY(ctx->prep->rgb.ensure((size_t)std::max<int64_t>(p.src_off[p.B], 1)));
+    *d_rgb = ctx->prep->rgb.as<uint8_t>();
     return VPK_OK;
 }
 
@@ -229,7 +236,7 @@ static size_t tile_smem(int TW, int TH, double fx, double fy, int* nx, int* ny) 
     return (size_t)(TW + TH) * sizeof(Taps) + (size_t)*ny * TW * 3 * sizeof(double) + (((size_t)*nx * *ny * 3 + 15) & ~(size_t)15);
 }
 
-int prep_run(vpk_ctx* ctx, const PrepPlan& p, const uint8_t* rgb, double out_scale, double* d_out) {
+int prep_run(vpk_ctx* ctx, const PrepPlan& p, double out_scale, double* d_out) {
     const int B = p.B;
     VPK_CUDA(cudaSetDevice(ctx->device));
     if (!ctx->prep) ctx->prep = new PrepState();
@@ -271,10 +278,8 @@ int prep_run(vpk_ctx* ctx, const PrepPlan& p, const uint8_t* rgb, double out_sca
     const int64_t n_src = p.src_off[B], n_out = p.pix_off[B];
     const size_t im_bytes = (size_t)B * sizeof(PrepImage);
     VPK_TRY(s->meta.ensure(im_bytes + (size_t)(B + 1) * sizeof(int32_t)));
-    VPK_TRY(s->rgb.ensure((size_t)n_src));
     VPK_CUDA(cudaMemcpyAsync(s->meta.p, im.data(), im_bytes, cudaMemcpyHostToDevice, st));
     VPK_CUDA(cudaMemcpyAsync(s->meta.as<char>() + im_bytes, tile_off.data(), (size_t)(B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    VPK_CUDA(cudaMemcpyAsync(s->rgb.p, rgb, (size_t)n_src, cudaMemcpyHostToDevice, st));
     if (smem > 48 * 1024) VPK_CUDA(cudaFuncSetAttribute(image_prep, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     KernelScope ks(ctx, "image_prep");
     image_prep<<<tile_off[B], kPrepThreads, smem, st>>>(s->rgb.as<uint8_t>(), s->meta.as<PrepImage>(),
@@ -301,13 +306,17 @@ int vpk_prepare_images(vpk_ctx* ctx, const uint8_t* rgb, const int64_t* byte_off
                        int32_t n_images, int32_t target_size, int32_t* out_widths, int32_t* out_heights, double* gray_out) {
     if (!ctx || !out_widths || !out_heights) { set_error("vpk_prepare_images: bad argument"); return VPK_ERR_ARG; }
     PrepPlan p;
-    VPK_TRY(prep_plan(rgb, byte_offsets, widths, heights, n_images, target_size, "vpk_prepare_images", p));
+    VPK_TRY(prep_plan(byte_offsets, widths, heights, n_images, target_size, "vpk_prepare_images", p));
+    if (!rgb) { set_error("vpk_prepare_images: rgb is NULL"); return VPK_ERR_ARG; }
     if (!gray_out) { set_error("vpk_prepare_images: gray_out is NULL"); return VPK_ERR_ARG; }
     VPK_CUDA(cudaSetDevice(ctx->device));
     if (!ctx->prep) ctx->prep = new PrepState();
     const int64_t n_out = p.pix_off[n_images];
     VPK_TRY(ctx->prep->out.ensure((size_t)n_out * sizeof(double)));
-    VPK_TRY(prep_run(ctx, p, rgb, 1.0, ctx->prep->out.as<double>()));
+    uint8_t* d_rgb = nullptr;
+    VPK_TRY(prep_input(ctx, p, &d_rgb));
+    VPK_CUDA(cudaMemcpyAsync(d_rgb, rgb, (size_t)p.src_off[n_images], cudaMemcpyHostToDevice, ctx->stream));
+    VPK_TRY(prep_run(ctx, p, 1.0, ctx->prep->out.as<double>()));
     VPK_CUDA(cudaMemcpyAsync(gray_out, ctx->prep->out.p, (size_t)n_out * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     VPK_CUDA(cudaStreamSynchronize(ctx->stream));
     memcpy(out_widths, p.W.data(), (size_t)n_images * sizeof(int32_t));

@@ -139,20 +139,54 @@ int vpk_pipeline_upload_photos(vpk_ctx* ctx, const uint8_t* rgb, const int64_t* 
                                int32_t* counts_out, int32_t* out_widths, int32_t* out_heights) {
     if (!ctx) { set_error("vpk_pipeline_upload_photos: bad argument"); return VPK_ERR_ARG; }
     PrepPlan pp;
-    VPK_TRY(prep_plan(rgb, byte_offsets, widths, heights, B, target_size, "vpk_pipeline_upload_photos", pp));
+    VPK_TRY(prep_plan(byte_offsets, widths, heights, B, target_size, "vpk_pipeline_upload_photos", pp));
+    if (!rgb) { set_error("vpk_pipeline_upload_photos: rgb is NULL"); return VPK_ERR_ARG; }
     // the detector reads the prepared planes (float64, x 255) where the preparation kernel writes them
     std::vector<int32_t> counts(B), row_off;
     LsdPlan lp;
     VPK_TRY(lsd_plan(pp.pix_off.data(), pp.W.data(), pp.H.data(), B, VPK_PIX_F64, cfg, counts.data(), lp));
     void* d_in = nullptr;
     VPK_TRY(lsd_input(ctx, lp, &d_in));
-    VPK_TRY(prep_run(ctx, pp, rgb, 255.0, static_cast<double*>(d_in)));
+    uint8_t* d_rgb = nullptr;
+    VPK_TRY(prep_input(ctx, pp, &d_rgb));
+    VPK_CUDA(cudaMemcpyAsync(d_rgb, rgb, (size_t)pp.src_off[B], cudaMemcpyHostToDevice, ctx->stream));
+    VPK_TRY(prep_run(ctx, pp, 255.0, static_cast<double*>(d_in)));
     const double* d_rows = nullptr;
     VPK_TRY(lsd_detect(ctx, lp, counts.data(), &d_rows, row_off));
     VPK_TRY(upload_detected(ctx, d_rows, row_off, pp.W.data(), pp.H.data(), B));
     if (counts_out) memcpy(counts_out, counts.data(), (size_t)B * sizeof(int32_t));
     if (out_widths) memcpy(out_widths, pp.W.data(), (size_t)B * sizeof(int32_t));
     if (out_heights) memcpy(out_heights, pp.H.data(), (size_t)B * sizeof(int32_t));
+    return VPK_OK;
+}
+
+int vpk_pipeline_upload_jpegs(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t B, int32_t target_size,
+                              const vpk_lsd_config* cfg, int32_t* counts_out, int32_t* out_widths, int32_t* out_heights,
+                              int32_t* status_out) {
+    if (!ctx) { set_error("vpk_pipeline_upload_jpegs: bad argument"); return VPK_ERR_ARG; }
+    std::vector<int32_t> w, h, nc;
+    VPK_TRY(jpeg_plan(ctx, data, byte_offsets, B, true, "vpk_pipeline_upload_jpegs", w, h, nc));
+    std::vector<int64_t> rgb_off(B + 1, 0);
+    for (int b = 0; b < B; ++b) rgb_off[b + 1] = rgb_off[b] + 3 * (int64_t)w[b] * h[b];
+    PrepPlan pp;
+    VPK_TRY(prep_plan(rgb_off.data(), w.data(), h.data(), B, target_size, "vpk_pipeline_upload_jpegs", pp));
+    std::vector<int32_t> counts(B), row_off, status(B);
+    LsdPlan lp;
+    VPK_TRY(lsd_plan(pp.pix_off.data(), pp.W.data(), pp.H.data(), B, VPK_PIX_F64, cfg, counts.data(), lp));
+    void* d_in = nullptr;
+    VPK_TRY(lsd_input(ctx, lp, &d_in));
+    // the decoder writes the RGB photos where the preparation kernel reads them: only the files cross PCIe
+    uint8_t* d_rgb = nullptr;
+    VPK_TRY(prep_input(ctx, pp, &d_rgb));
+    VPK_TRY(jpeg_decode(ctx, data, byte_offsets, rgb_off.data(), d_rgb, status.data()));
+    VPK_TRY(prep_run(ctx, pp, 255.0, static_cast<double*>(d_in)));
+    const double* d_rows = nullptr;
+    VPK_TRY(lsd_detect(ctx, lp, counts.data(), &d_rows, row_off));
+    VPK_TRY(upload_detected(ctx, d_rows, row_off, pp.W.data(), pp.H.data(), B));
+    if (counts_out) memcpy(counts_out, counts.data(), (size_t)B * sizeof(int32_t));
+    if (out_widths) memcpy(out_widths, pp.W.data(), (size_t)B * sizeof(int32_t));
+    if (out_heights) memcpy(out_heights, pp.H.data(), (size_t)B * sizeof(int32_t));
+    if (status_out) memcpy(status_out, status.data(), (size_t)B * sizeof(int32_t));
     return VPK_OK;
 }
 

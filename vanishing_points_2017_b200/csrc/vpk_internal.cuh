@@ -88,6 +88,7 @@ struct EmState;    // em.cu
 struct PipeState;  // pipeline.cu
 struct LsdState;   // lsd.cu
 struct PrepState;  // image_prep.cu
+struct JpegState;  // jpeg.cu
 
 }  // namespace vpk
 
@@ -117,6 +118,7 @@ struct vpk_ctx {
     vpk::PipeState* pipe = nullptr;
     vpk::LsdState* lsd = nullptr;
     vpk::PrepState* prep = nullptr;
+    vpk::JpegState* jpeg = nullptr;
 };
 
 namespace vpk {
@@ -223,22 +225,34 @@ int lsd_input(vpk_ctx* ctx, const LsdPlan& plan, void** d_in);
 int lsd_detect(vpk_ctx* ctx, const LsdPlan& plan, int32_t* counts_out, const double** d_rows, std::vector<int32_t>& row_offsets);
 
 // image_prep.cu: resize (INTER_AREA) + rgb2gray of a ragged batch of uint8 RGB photos.  prep_plan validates the
-// call and computes the prepared sizes (host only); prep_run copies the photos to the device and writes the float64
-// gray planes, multiplied by out_scale, to d_out (image b's W'*H' plane at plan.pix_off[b]).
+// call and computes the prepared sizes (host only); prep_input sizes the device buffer of the photos and returns it
+// (photo b's bytes at plan.src_off[b]); prep_run writes the float64 gray planes of what was written there, multiplied
+// by out_scale, to d_out (image b's W'*H' plane at plan.pix_off[b]).
 struct PrepPlan {
     int32_t B = 0;
     std::vector<int32_t> w, h, W, H;
     std::vector<int64_t> src_off;   // B+1 byte offsets of the photos
     std::vector<int64_t> pix_off;   // B+1 pixel offsets of the prepared planes
 };
-int prep_plan(const uint8_t* rgb, const int64_t* byte_offsets, const int32_t* widths, const int32_t* heights, int32_t B,
+int prep_plan(const int64_t* byte_offsets, const int32_t* widths, const int32_t* heights, int32_t B,
               int32_t target_size, const char* who, PrepPlan& plan);
-int prep_run(vpk_ctx* ctx, const PrepPlan& plan, const uint8_t* rgb, double out_scale, double* d_out);
+int prep_input(vpk_ctx* ctx, const PrepPlan& plan, uint8_t** d_rgb);
+int prep_run(vpk_ctx* ctx, const PrepPlan& plan, double out_scale, double* d_out);
+
+// jpeg.cu: jpeg_plan parses the files' markers (host only) and keeps the headers in the context; it fails with
+// VPK_ERR_ARG naming the first unsupported photo (or the first gray one if rgb_only) and returns each photo's size and
+// components.  jpeg_decode runs the decode of the planned files on the device: photo b's h x w x components bytes at
+// d_out + pix_off[b]; status_out (B) receives VPK_JPEG_OK or VPK_JPEG_CORRUPT.
+int jpeg_plan(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t B, bool rgb_only, const char* who,
+              std::vector<int32_t>& widths, std::vector<int32_t>& heights, std::vector<int32_t>& components);
+int jpeg_decode(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, const int64_t* pix_off, uint8_t* d_out,
+                int32_t* status_out);
 
 void cnn_free(vpk_ctx* ctx);
 void em_free(vpk_ctx* ctx);
 void pipe_free(vpk_ctx* ctx);
 void lsd_free(vpk_ctx* ctx);
 void prep_free(vpk_ctx* ctx);
+void jpeg_free(vpk_ctx* ctx);
 
 }  // namespace vpk

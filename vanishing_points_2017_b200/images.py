@@ -1,8 +1,8 @@
-"""Photo preparation in front of LSD on the device (`vpk_prepare_images`, row N5): the head of the reference's
+"""JPEG decoding (`vpk_decode_jpegs`, row N6) and photo preparation in front of LSD on the device (`vpk_prepare_images`, row N5): the head of the reference's
 evaluation.create_data_pickles (evaluation.py:139-154), i.e. `convert ... -resize TxT` (example.py:37: 640;
 benchmark.py:59-60: 800 for ECD / HLW; OpenCV 4.13's INTER_AREA rule stands in for ImageMagick), the 8-bit RGB read
 back, and skimage.color.rgb2gray.  Photos go over PCIe as uint8 RGB; the float64 gray planes are built on the device.
-DESIGN.md section 4.7.  No CPU fallback."""
+DESIGN.md sections 4.7 and 4.8.  No CPU fallback."""
 import ctypes as C
 
 import numpy as np
@@ -59,3 +59,70 @@ def prepare_images(photos, target_size=None, ctx=None):
         res.append(out[pos:pos + int(W) * int(H)].reshape(int(H), int(W)))
         pos += int(W) * int(H)
     return res
+
+
+def pack_jpegs(blobs):
+    """List of JPEG files (bytes, or 1-D uint8 arrays of the file contents) -> (flat bytes, byte offsets (B+1) int64).
+    Anything else raises ValueError."""
+    if isinstance(blobs, (bytes, bytearray, np.ndarray)) or not hasattr(blobs, "__len__"):
+        raise ValueError("blobs must be a list of JPEG files (bytes or 1-D uint8 arrays)")
+    parts = []
+    for b in blobs:
+        if isinstance(b, (bytes, bytearray, memoryview)):
+            a = np.frombuffer(bytes(b), np.uint8)
+        else:
+            a = np.asarray(b)
+            if a.ndim != 1 or a.dtype != np.uint8:
+                raise ValueError("a JPEG file must be bytes or a 1-D uint8 array, got %s %r" % (a.dtype, a.shape))
+        parts.append(a)
+    flat = np.ascontiguousarray(np.concatenate(parts) if parts else np.zeros(0, np.uint8))
+    off = np.concatenate([[0], np.cumsum([p.size for p in parts])]).astype(np.int64)
+    return flat, off
+
+
+def jpeg_info(blobs):
+    """Reads each file's markers up to the scan (never the entropy-coded data); needs no GPU.  Returns a list of
+    (width, height, components, support) with support 0 for a file the decoder takes, else the reason it is refused
+    (vpk.h VPK_JPEG_*, named in _lib.JPEG_REASONS)."""
+    flat, off = pack_jpegs(blobs)
+    B = len(off) - 1
+    if B == 0:
+        return []
+    w, h, c, s = (np.zeros(B, np.int32) for _ in range(4))
+    _lib.check(_lib.load().vpk_jpeg_info(_lib.ptr(flat), _lib.ptr(off), B, _lib.ptr(w), _lib.ptr(h), _lib.ptr(c), _lib.ptr(s)),
+               "vpk_jpeg_info")
+    return [(int(a), int(b), int(d), int(e)) for a, b, d, e in zip(w, h, c, s)]
+
+
+def decode_jpegs(blobs, ctx=None):
+    """Decodes baseline JPEG files on the device, bit for bit with libjpeg-turbo's default decode (EXIF orientation
+    ignored).  Returns (arrays, status): (H, W, 3) uint8 RGB arrays, (H, W) for 1-component files, and an int32 status
+    per file (0, or _lib.JPEG_CORRUPT for inconsistent entropy-coded data, whose pixels are unspecified).  A refused
+    file raises VpkError naming its index and reason."""
+    flat, off = pack_jpegs(blobs)
+    B = len(off) - 1
+    if B == 0:
+        return [], np.zeros(0, np.int32)
+    info = jpeg_info(blobs)
+    for k, (w, h, c, s) in enumerate(info):
+        if s != 0:
+            raise _lib.VpkError("decode_jpegs: file %d is not supported: %s" % (k, _lib.JPEG_REASONS[s]))
+    ctx = ctx or _lib.default_context()
+    out = np.empty(max(sum(w * h * c for w, h, c, _ in info), 1), np.uint8)
+    status = np.empty(B, np.int32)
+    _lib.check(ctx.lib.vpk_decode_jpegs(ctx.h, _lib.ptr(flat), _lib.ptr(off), B, _lib.ptr(out), _lib.ptr(status)), "vpk_decode_jpegs")
+    res, pos = [], 0
+    for w, h, c, _ in info:
+        n = w * h * c
+        res.append(out[pos:pos + n].reshape((h, w, 3) if c == 3 else (h, w)))
+        pos += n
+    return res, status
+
+
+def jpeg_stats(ctx=None):
+    """Decoder statistics of the context's last decode: subsequences, re-decoded subsequences and the most rounds
+    inside one CTA (both counted only while profiling is enabled), extra launches across CTAs."""
+    ctx = ctx or _lib.default_context()
+    out = np.zeros(4, np.int64)
+    _lib.check(ctx.lib.vpk_jpeg_stats(ctx.h, _lib.ptr(out)), "vpk_jpeg_stats")
+    return {"subsequences": int(out[0]), "redecoded": int(out[1]), "max_rounds": int(out[2]), "global_rounds": int(out[3])}
