@@ -187,6 +187,32 @@ VPK_API int vpk_em(vpk_ctx* ctx, const double* lines, const double* segments, co
 VPK_API int vpk_em_distribution(vpk_ctx* ctx, int32_t image, int32_t n_vp, int32_t n_lines, double* p_v, double* p_lv,
                                 double* p_vl, double* p_l, double* lvsq, double* angles);
 
+/* Diagnostics: raw copy of buffer `which` (VPK_EM_BUF_*) of image `image`'s EM workspace as the last vpk_em /
+ * vpk_pipeline_run call of this context left it, in the device layout (float64).  N = the image's lines, M = its
+ * 'vp' rows (n_vp); kMP = 32, kMPS = 36 and the layouts are those of csrc/em_core.cuh:
+ *   LSIM     ceil(N/64)*64*N   similarity matrix of em_pair: 64-column slabs of N x 64 doubles, element (j, k) at
+ *                              ((k/64)*N + j)*64 + ((k%64) ^ ((j&3)<<2))   (lsim_index)
+ *   COLSUM   N                 column sums of lsim (em_pair; 0 with use_weights = 0, set by em_init)
+ *   LWEIGHT  N                 kNN line weights (em_pair; 1 with use_weights = 0, set by em_init)
+ *   LVSQ     M*N               (M, N) row-major planes of the last superstep's em_estep: lvsq, p(v|l)
+ *   PVL      M*N
+ *   W        M*N               (M, N) weight matrix of the last superstep's em_wmat (= the decision metric)
+ *   WT       ceil(M/32)*N*36   em_wmat's operand p(v|l)*lweight: pass p (rows 32p..32p+31) at p*N*36, line n of the
+ *                              pass at n*s, s = 8*t+4, t = ceil(min(M-32p, 32)/8); rows M..8t-1 of the last pass are
+ *                              zeros, the last 4 doubles of a line are never written   (wt_index)
+ *   ESTEP    5*M               the E-step constants of those planes, rows pv | vx | vy | inv2s | coef
+ * The planes (LVSQ .. ESTEP) belong to the image's final hypotheses: an image that finished with VPK_EM_OK ends in
+ * the final-count phase (vp_localisation.py:415-437), which asks for a new E-step and weight matrix on the
+ * remaining 'vp' rows each time it drops one and finishes without another, so M is n_vp, and pv .. coef are
+ * evaluated on 'vp' and 'sigma' (vx = vp0/vp2, vy = vp1/vp2, inv2s = 1/(2 sigma), coef = 1/sqrt(2 pi sigma)).
+ * count (may be NULL) receives the buffer's size in doubles; out = NULL only asks for it.
+ * Fails with VPK_ERR_STATE before any EM call, after a batch that ran in more than one workspace wave, for LSIM
+ * of a batch run with use_weights = 0 (no pair pass), and for the planes of an image whose status is not
+ * VPK_EM_OK; with VPK_ERR_ARG for a bad `which`, an image not in the last batch or capacity < the size. */
+enum { VPK_EM_BUF_LSIM = 0, VPK_EM_BUF_COLSUM, VPK_EM_BUF_LWEIGHT, VPK_EM_BUF_LVSQ, VPK_EM_BUF_PVL, VPK_EM_BUF_W,
+       VPK_EM_BUF_WT, VPK_EM_BUF_ESTEP, VPK_EM_NBUF };
+VPK_API int vpk_em_debug_fetch(vpk_ctx* ctx, int32_t image, int32_t which, double* out, int64_t capacity, int64_t* count);
+
 /* Profiling runs only (vpk_profile_enable): accumulated algorithmic work of the weight-matrix
  * products (vp_localisation.py:515-524) since the last reset: out[0] = bytes of similarity
  * matrix consumed (8 N^2 per product), out[1] = flops (2 M N^2 per product), out[2] = number

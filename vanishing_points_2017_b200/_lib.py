@@ -19,7 +19,7 @@ EM_OK, EM_NO_INITIAL_VPS, EM_NO_VPS_LEFT, EM_CAPACITY = 0, 1, 2, 3
 SYMBOLS = [
     "vpk_create", "vpk_destroy", "vpk_abi_version", "vpk_last_error", "vpk_synchronize", "vpk_launch_count", "vpk_mark", "vpk_mark_elapsed",
     "vpk_profile_enable", "vpk_profile_reset", "vpk_profile_read", "vpk_lines_from_segments", "vpk_sphere_map",
-    "vpk_cnn_load", "vpk_cnn_forward", "vpk_cnn_debug_fetch", "vpk_debug_gemm", "vpk_em_default_config", "vpk_em", "vpk_em_distribution", "vpk_em_stats", "vpk_em_phase_cycles", "vpk_pipeline_upload", "vpk_pipeline_run",
+    "vpk_cnn_load", "vpk_cnn_forward", "vpk_cnn_debug_fetch", "vpk_debug_gemm", "vpk_em_default_config", "vpk_em", "vpk_em_distribution", "vpk_em_debug_fetch", "vpk_em_stats", "vpk_em_phase_cycles", "vpk_pipeline_upload", "vpk_pipeline_run",
     "vpk_pipeline_fetch", "vpk_pipeline_host", "vpk_pipeline_stage_ms", "vpk_horizon", "vpk_pipeline_horizon",
     "vpk_segments_from_lsd", "vpk_pipeline_upload_lsd",
     "vpk_lsd_default_config", "vpk_lsd", "vpk_lsd_fetch", "vpk_pipeline_upload_images",
@@ -98,6 +98,7 @@ def load():
         lib.vpk_em_stats.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
         lib.vpk_em_distribution.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                             C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.vpk_em_debug_fetch.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]
         lib.vpk_em_phase_cycles.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
         lib.vpk_pipeline_upload.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]
         lib.vpk_pipeline_run.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_double, C.POINTER(EmConfig)]

@@ -1590,6 +1590,65 @@ int vpk_em_distribution(vpk_ctx* ctx, int32_t image, int32_t n_vp, int32_t n_lin
     return VPK_OK;
 }
 
+int vpk_em_debug_fetch(vpk_ctx* ctx, int32_t image, int32_t which, double* out, int64_t capacity, int64_t* count) {
+    if (count) *count = 0;
+    if (!ctx || image < 0 || which < 0 || which >= VPK_EM_NBUF || capacity < 0 || (capacity > 0 && !out)) {
+        set_error("vpk_em_debug_fetch: bad argument");
+        return VPK_ERR_ARG;
+    }
+    EmState* st = ctx->em;
+    if (!st || st->wave.begun || st->wave.n <= 0 || st->wave.waves_run != 1 || st->wave.n != st->wave.key_B) {
+        set_error("vpk_em_debug_fetch: the EM workspace is kept for the last batch only, and only if it ran in one workspace wave");
+        return VPK_ERR_STATE;
+    }
+    const EmWave& W = st->wave;
+    const SlotDesc* hd = st->h_desc.as<SlotDesc>();
+    int slot = -1;
+    for (int i = 0; i < W.n; ++i) if (hd[i].img == image) { slot = i; break; }
+    if (slot < 0) { set_error("vpk_em_debug_fetch: image %d is not part of the last batch", image); return VPK_ERR_ARG; }
+    if (which == VPK_EM_BUF_LSIM && !W.key_P.cfg.use_weights) {
+        set_error("vpk_em_debug_fetch: the last batch ran with use_weights = 0, the pair pass did not compute lsim");
+        return VPK_ERR_STATE;
+    }
+    VPK_CUDA(cudaSetDevice(ctx->device));
+    const int N = hd[slot].N;
+    const Img im = make_img(N, st->ws.as<double>() + hd[slot].ws_off, nullptr);
+    const double* src = nullptr;
+    size_t n = 0;
+    EmSlot hs;
+    if (which >= VPK_EM_BUF_LVSQ) {
+        VPK_CUDA(cudaMemcpy(&hs, st->slots.as<EmSlot>() + slot, sizeof(EmSlot), cudaMemcpyDeviceToHost));
+        if (hs.status != VPK_EM_OK) {
+            set_error("vpk_em_debug_fetch: image %d finished with status %d, its last E-step planes are not kept", image, hs.status);
+            return VPK_ERR_STATE;
+        }
+    }
+    const size_t M = which >= VPK_EM_BUF_LVSQ ? (size_t)hs.M : 0;
+    switch (which) {
+    case VPK_EM_BUF_LSIM: src = im.lsim; n = lsim_doubles(N); break;
+    case VPK_EM_BUF_COLSUM: src = im.colsum; n = N; break;
+    case VPK_EM_BUF_LWEIGHT: src = im.lweight; n = N; break;
+    case VPK_EM_BUF_LVSQ: src = im.lvsq; n = M * N; break;
+    case VPK_EM_BUF_PVL: src = im.pvl; n = M * N; break;
+    case VPK_EM_BUF_W: src = im.w; n = M * N; break;
+    case VPK_EM_BUF_WT: src = im.wt; n = (M + kMP - 1) / kMP * (size_t)N * kMPS; break;
+    default: n = 5 * M; break;                                            // VPK_EM_BUF_ESTEP: from the slot state
+    }
+    if (count) *count = (int64_t)n;
+    if (!out) return VPK_OK;                                              // size query
+    if ((size_t)capacity < n) { set_error("vpk_em_debug_fetch: %zu doubles needed, room for %lld", n, (long long)capacity); return VPK_ERR_ARG; }
+    if (which == VPK_EM_BUF_ESTEP) {
+        const double* c[5] = {hs.pv, hs.vx, hs.vy, hs.inv2s, hs.coef};
+        for (int r = 0; r < 5; ++r) memcpy(out + r * M, c[r], M * sizeof(double));
+        return VPK_OK;
+    }
+    if (n) {
+        VPK_CUDA(cudaMemcpyAsync(out, src, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        VPK_CUDA(cudaStreamSynchronize(ctx->stream));
+    }
+    return VPK_OK;
+}
+
 int vpk_em_phase_cycles(vpk_ctx* ctx, uint64_t out[8], int reset) {
     if (!ctx || !out) { set_error("vpk_em_phase_cycles: bad argument"); return VPK_ERR_ARG; }
     for (int k = 0; k < 8; ++k) out[k] = ctx->em ? ctx->em->phase_cycles[k] : 0;

@@ -193,7 +193,8 @@ VPK_HD size_t slot_doubles(int N) {
            align16((size_t)(kMaxM / kMP) * kMPS * n) + 16;
 }
 
-VPK_DEV Img make_img(int N, double* ws, const double* lp) {
+// (host-callable too: vpk_em_debug_fetch finds the buffers of a slot with it)
+VPK_HD Img make_img(int N, double* ws, const double* lp) {
     Img im;
     size_t n = (size_t)N;
     im.N = N; im.lp = lp;

@@ -29,6 +29,74 @@ def em_distribution(image, n_vp, n_lines, ctx=None):
                                            _lib.ptr(a["l"]), _lib.ptr(a["lvsq"]), _lib.ptr(a["angles"])), "vpk_em_distribution")
     return PDF(**a)
 
+
+# vpk_em_debug_fetch buffer names (include/vpk.h, VPK_EM_BUF_*)
+EM_BUFFERS = ["lsim", "colsum", "lweight", "lvsq", "pvl", "w", "wt", "estep"]
+_TK, _MP, _MPS = 64, 32, 36          # csrc/em_core.cuh kTK, kMP, kMPS
+
+
+def lsim_index(N, j, k):
+    """csrc/em_core.cuh lsim_index: 64-column slabs of N x 64, the column XOR-swizzled with bits 0-1 of the row."""
+    j, k = np.asarray(j, np.int64), np.asarray(k, np.int64)
+    return ((k // _TK) * N + j) * _TK + ((k % _TK) ^ ((j & 3) << 2))
+
+
+def wpass_tiles(M, p):
+    """csrc/em_core.cuh wpass_tiles: 8-row tiles of pass p (VP rows 32p .. 32p+31) for M hypotheses."""
+    return (min(max(M - p * _MP, 1), _MP) + 7) // 8
+
+
+def wt_index(N, n, m, M):
+    """csrc/em_core.cuh wt_index: pass p = m // 32 at p*N*36, line n of the pass at stride 8 * tiles + 4."""
+    n, m = np.asarray(n, np.int64), np.asarray(m, np.int64)
+    p = m // _MP
+    stride = np.array([8 * wpass_tiles(M, q) + 4 for q in range(int(p.max(initial=0)) + 1)], np.int64)[p]
+    return p * N * _MPS + n * stride + m % _MP
+
+
+def wt_rows(M):
+    """rows of the W operand for M hypotheses: every pass but the last has 32, the last 8 * its tiles."""
+    passes = (M + _MP - 1) // _MP
+    return 0 if M == 0 else _MP * (passes - 1) + 8 * wpass_tiles(M, passes - 1)
+
+
+def unpack_lsim(raw, N):
+    """(N, N) similarity matrix from the LSIM buffer."""
+    j, k = np.meshgrid(np.arange(N), np.arange(N), indexing="ij")
+    return raw[lsim_index(N, j, k)]
+
+
+def unpack_wt(raw, N, M):
+    """(wt_rows(M), N) W operand from the WT buffer: rows M .. of the last pass are its zero padding."""
+    m, n = np.meshgrid(np.arange(wt_rows(M)), np.arange(N), indexing="ij")
+    return raw[wt_index(N, n, m, M)] if m.size else np.zeros((wt_rows(M), N))
+
+
+def _em_fetch_raw(ctx, image, which):
+    n = C.c_int64(0)
+    _lib.check(ctx.lib.vpk_em_debug_fetch(ctx.h, int(image), int(which), None, 0, C.byref(n)), "vpk_em_debug_fetch")
+    out = np.empty(n.value)
+    _lib.check(ctx.lib.vpk_em_debug_fetch(ctx.h, int(image), int(which), _lib.ptr(out), out.size, None), "vpk_em_debug_fetch")
+    return out
+
+
+def em_debug_fetch(image, name, ctx=None, raw=False):
+    """Buffer `name` (EM_BUFFERS) of image `image`'s EM workspace as the LAST EM call on `ctx` left it
+    (`vpk_em_debug_fetch`, diagnostics).  raw=True: the device layout; otherwise dense arrays: lsim (N, N),
+    colsum / lweight (N), lvsq / pvl / w (M, N), wt (wt_rows(M), N), estep a dict of pv, vx, vy, inv2s, coef (M)."""
+    ctx = ctx or _lib.default_context()
+    out = _em_fetch_raw(ctx, image, EM_BUFFERS.index(name))
+    if raw or name in ("colsum", "lweight"):
+        return out
+    if name == "estep":
+        return dict(zip(("pv", "vx", "vy", "inv2s", "coef"), out.reshape(5, -1)))
+    N = _em_fetch_raw(ctx, image, EM_BUFFERS.index("colsum")).size
+    if name == "lsim":
+        return unpack_lsim(out, N)
+    M = _em_fetch_raw(ctx, image, EM_BUFFERS.index("estep")).size // 5
+    return unpack_wt(out, N, M) if name == "wt" else out.reshape(M, N)
+
+
 _SKELETON = {"vp_assoc": None, "vp": None, "counts": None, "count_id": None, "decision_metric": None,
              "iterations": 0}
 
