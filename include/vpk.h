@@ -351,6 +351,49 @@ VPK_API int vpk_pipeline_upload_jpegs(vpk_ctx* ctx, const uint8_t* data, const i
  * otherwise.  Fails with VPK_ERR_STATE before any decode. */
 VPK_API int vpk_jpeg_stats(vpk_ctx* ctx, int64_t* out);
 
+/* ---- N7: PNG decoding in front of photo preparation ----------------------------- */
+/* The read of PNG files (reference evaluation.py:142-143: the dataset's *.png files, and the 8-bit PNG every photo
+ * is written to and read back), on the device and bit for bit with libpng's decode; DESIGN.md section 4.9.
+ * Decoded: 8-bit and lower files, non-interlaced or Adam7, any split of the zlib stream over IDAT chunks: gray (colour
+ * type 0; 1, 2, 4 or 8 bits, scaled to 0..255 as libpng's expand does) and gray + alpha (4) to gray; RGB (2), palette
+ * (3; 1 to 8 bits, an index beyond PLTE gives black) and RGBA (6) to RGB.  Alpha is dropped, not composited; tRNS,
+ * gAMA, iCCP, sRGB and eXIf are ignored (no colour management, no EXIF orientation); an APNG decodes as its default
+ * image.  Files: host array `data`, file b the byte_offsets[b] .. byte_offsets[b+1] bytes (B+1 non-decreasing entries). */
+enum {
+    VPK_PNG_OK = 0,
+    VPK_PNG_NOT_PNG = 1,        /* no PNG signature (a JPEG passed by mistake, ...) */
+    VPK_PNG_DEPTH = 2,          /* 16-bit samples */
+    VPK_PNG_MALFORMED = 3,      /* a truncated or overrunning chunk, IHDR values PNG forbids, chunks out of order or
+                                 * IDAT chunks that are not consecutive, no PLTE for colour type 3, an unknown critical
+                                 * chunk, a bad length or CRC on IHDR or on the PLTE of a palette file (elsewhere PLTE is
+                                 * ignored), no IDAT or IEND, an invalid zlib header (a method other than deflate, a
+                                 * window above 32 K, a preset dictionary, a bad check) */
+    VPK_PNG_CORRUPT = 4         /* status after decoding: an IDAT CRC mismatch, an Adler-32 mismatch, a stream that ends
+                                 * before the last row, a filter byte above 4, an invalid deflate stream (zlib's
+                                 * verdicts, up to the last row and the end of the stream right after it), running out of
+                                 * IDAT data; the file's pixels are unspecified but deterministic.  Data after the last
+                                 * row is not an error, nor are zlib's errors past it (libpng warns and decodes the
+                                 * image) */
+};
+/* Walks the chunks of every file (chunk headers, IHDR and PLTE; never the IDAT payloads); host only, needs no device
+ * or context.  widths / heights / color_types (B, each may be NULL) receive IHDR's values (0 unless IHDR was read);
+ * support (B, may be NULL) VPK_PNG_OK or the reason a file is refused. */
+VPK_API int vpk_png_info(const uint8_t* data, const int64_t* byte_offsets, int32_t n, int32_t* widths, int32_t* heights,
+                         int32_t* color_types, int32_t* support);
+/* Decodes every file on the device.  pixels_out: file after file, row-major height x width x channels bytes (RGB for
+ * colour types 2, 3 and 6, gray for 0 and 4); status_out (B): VPK_PNG_OK or VPK_PNG_CORRUPT.  Fails with VPK_ERR_ARG
+ * before any device work, naming the first refused file and its reason. */
+VPK_API int vpk_decode_pngs(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t n, uint8_t* pixels_out,
+                            int32_t* status_out);
+/* vpk_decode_pngs followed by vpk_pipeline_upload_photos on the decoded photos, on the device: only the files cross
+ * PCIe, the decoder writes the RGB photos where the preparation kernel reads them.  counts_out / out_widths /
+ * out_heights as vpk_pipeline_upload_photos, status_out (B) as vpk_decode_pngs (each may be NULL; a CORRUPT file's
+ * rows come from its unspecified pixels).  A refused file or a gray one (colour type 0 or 4: gray photos cannot be
+ * prepared) fails the call with VPK_ERR_ARG, naming its index and reason. */
+VPK_API int vpk_pipeline_upload_pngs(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t n,
+                                     int32_t target_size, const vpk_lsd_config* cfg, int32_t* counts_out,
+                                     int32_t* out_widths, int32_t* out_heights, int32_t* status_out);
+
 /* ---- N1: horizon line and orthogonal VP triplet --------------------------- */
 /* calc_horizon.calculate_horizon_and_ortho_vp(em_result, maxbest=10, theta_vmin=pi/10, theta_z=pi/4)
  * (reference calc_horizon.py:19-225; callers example.py:65, benchmark.py:233) for a batch of EM

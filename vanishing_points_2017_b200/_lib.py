@@ -25,11 +25,15 @@ SYMBOLS = [
     "vpk_lsd_default_config", "vpk_lsd", "vpk_lsd_fetch", "vpk_pipeline_upload_images",
     "vpk_prepared_size", "vpk_prepare_images", "vpk_pipeline_upload_photos",
     "vpk_jpeg_info", "vpk_decode_jpegs", "vpk_pipeline_upload_jpegs", "vpk_jpeg_stats",
+    "vpk_png_info", "vpk_decode_pngs", "vpk_pipeline_upload_pngs",
 ]
 PIX_U8, PIX_F64 = 0, 1
 # vpk.h VPK_JPEG_*: support codes of vpk_jpeg_info and the decode status
 JPEG_REASONS = ["ok", "progressive", "arithmetic", "precision", "color", "layout", "malformed", "lossless", "corrupt"]
 JPEG_OK, JPEG_CORRUPT = 0, 8
+# vpk.h VPK_PNG_*: support codes of vpk_png_info and the decode status
+PNG_REASONS = ["ok", "not png", "depth", "malformed", "corrupt"]
+PNG_OK, PNG_CORRUPT = 0, 4
 
 
 class VpkError(RuntimeError):
@@ -131,6 +135,10 @@ def load():
         lib.vpk_pipeline_upload_jpegs.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(LsdConfig),
                                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.vpk_jpeg_stats.argtypes = [C.c_void_p, C.c_void_p]
+        lib.vpk_png_info.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.vpk_decode_pngs.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
+        lib.vpk_pipeline_upload_pngs.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(LsdConfig),
+                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.vpk_abi_version.argtypes = []
         lib.vpk_last_error.argtypes = []
         _lib = lib

@@ -78,6 +78,7 @@ int vpk_destroy(vpk_ctx* ctx) {
     lsd_free(ctx);
     prep_free(ctx);
     jpeg_free(ctx);
+    png_free(ctx);
     for (auto& pe : ctx->pending) { cudaEventDestroy(pe.a); cudaEventDestroy(pe.b); }
     for (auto ev : ctx->event_pool) cudaEventDestroy(ev);
     ctx->d_lines.release(); ctx->d_segments.release(); ctx->d_offsets.release(); ctx->d_work.release();

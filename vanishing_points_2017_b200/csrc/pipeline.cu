@@ -62,6 +62,36 @@ static int upload_detected(vpk_ctx* ctx, const double* d_rows, const std::vector
     return VPK_OK;
 }
 
+// Decoded files into the resident batch: `decode(rgb_off, d_rgb, status)` writes photo b's h x w x 3 RGB bytes at
+// d_rgb + rgb_off[b], where the preparation kernel reads them; then preparation, LSD and the normalisation, as
+// vpk_pipeline_upload_photos.  Only the files cross PCIe.
+template <typename Decode>
+static int upload_decoded(vpk_ctx* ctx, const std::vector<int32_t>& w, const std::vector<int32_t>& h, int32_t B, int32_t target_size,
+                          const vpk_lsd_config* cfg, const char* who, Decode decode, int32_t* counts_out, int32_t* out_widths,
+                          int32_t* out_heights, int32_t* status_out) {
+    std::vector<int64_t> rgb_off(B + 1, 0);
+    for (int b = 0; b < B; ++b) rgb_off[b + 1] = rgb_off[b] + 3 * (int64_t)w[b] * h[b];
+    PrepPlan pp;
+    VPK_TRY(prep_plan(rgb_off.data(), w.data(), h.data(), B, target_size, who, pp));
+    std::vector<int32_t> counts(B), row_off, status(B);
+    LsdPlan lp;
+    VPK_TRY(lsd_plan(pp.pix_off.data(), pp.W.data(), pp.H.data(), B, VPK_PIX_F64, cfg, counts.data(), lp));
+    void* d_in = nullptr;
+    VPK_TRY(lsd_input(ctx, lp, &d_in));
+    uint8_t* d_rgb = nullptr;
+    VPK_TRY(prep_input(ctx, pp, &d_rgb));
+    VPK_TRY(decode(rgb_off.data(), d_rgb, status.data()));
+    VPK_TRY(prep_run(ctx, pp, 255.0, static_cast<double*>(d_in)));
+    const double* d_rows = nullptr;
+    VPK_TRY(lsd_detect(ctx, lp, counts.data(), &d_rows, row_off));
+    VPK_TRY(upload_detected(ctx, d_rows, row_off, pp.W.data(), pp.H.data(), B));
+    if (counts_out) memcpy(counts_out, counts.data(), (size_t)B * sizeof(int32_t));
+    if (out_widths) memcpy(out_widths, pp.W.data(), (size_t)B * sizeof(int32_t));
+    if (out_heights) memcpy(out_heights, pp.H.data(), (size_t)B * sizeof(int32_t));
+    if (status_out) memcpy(status_out, status.data(), (size_t)B * sizeof(int32_t));
+    return VPK_OK;
+}
+
 }  // namespace vpk
 
 using namespace vpk;
@@ -166,28 +196,24 @@ int vpk_pipeline_upload_jpegs(vpk_ctx* ctx, const uint8_t* data, const int64_t* 
     if (!ctx) { set_error("vpk_pipeline_upload_jpegs: bad argument"); return VPK_ERR_ARG; }
     std::vector<int32_t> w, h, nc;
     VPK_TRY(jpeg_plan(ctx, data, byte_offsets, B, true, "vpk_pipeline_upload_jpegs", w, h, nc));
-    std::vector<int64_t> rgb_off(B + 1, 0);
-    for (int b = 0; b < B; ++b) rgb_off[b + 1] = rgb_off[b] + 3 * (int64_t)w[b] * h[b];
-    PrepPlan pp;
-    VPK_TRY(prep_plan(rgb_off.data(), w.data(), h.data(), B, target_size, "vpk_pipeline_upload_jpegs", pp));
-    std::vector<int32_t> counts(B), row_off, status(B);
-    LsdPlan lp;
-    VPK_TRY(lsd_plan(pp.pix_off.data(), pp.W.data(), pp.H.data(), B, VPK_PIX_F64, cfg, counts.data(), lp));
-    void* d_in = nullptr;
-    VPK_TRY(lsd_input(ctx, lp, &d_in));
-    // the decoder writes the RGB photos where the preparation kernel reads them: only the files cross PCIe
-    uint8_t* d_rgb = nullptr;
-    VPK_TRY(prep_input(ctx, pp, &d_rgb));
-    VPK_TRY(jpeg_decode(ctx, data, byte_offsets, rgb_off.data(), d_rgb, status.data()));
-    VPK_TRY(prep_run(ctx, pp, 255.0, static_cast<double*>(d_in)));
-    const double* d_rows = nullptr;
-    VPK_TRY(lsd_detect(ctx, lp, counts.data(), &d_rows, row_off));
-    VPK_TRY(upload_detected(ctx, d_rows, row_off, pp.W.data(), pp.H.data(), B));
-    if (counts_out) memcpy(counts_out, counts.data(), (size_t)B * sizeof(int32_t));
-    if (out_widths) memcpy(out_widths, pp.W.data(), (size_t)B * sizeof(int32_t));
-    if (out_heights) memcpy(out_heights, pp.H.data(), (size_t)B * sizeof(int32_t));
-    if (status_out) memcpy(status_out, status.data(), (size_t)B * sizeof(int32_t));
-    return VPK_OK;
+    return upload_decoded(ctx, w, h, B, target_size, cfg, "vpk_pipeline_upload_jpegs",
+                          [&](const int64_t* rgb_off, uint8_t* d_rgb, int32_t* status) {
+                              return jpeg_decode(ctx, data, byte_offsets, rgb_off, d_rgb, status);
+                          },
+                          counts_out, out_widths, out_heights, status_out);
+}
+
+int vpk_pipeline_upload_pngs(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t B, int32_t target_size,
+                             const vpk_lsd_config* cfg, int32_t* counts_out, int32_t* out_widths, int32_t* out_heights,
+                             int32_t* status_out) {
+    if (!ctx) { set_error("vpk_pipeline_upload_pngs: bad argument"); return VPK_ERR_ARG; }
+    std::vector<int32_t> w, h, nc;
+    VPK_TRY(png_plan(ctx, data, byte_offsets, B, true, "vpk_pipeline_upload_pngs", w, h, nc));
+    return upload_decoded(ctx, w, h, B, target_size, cfg, "vpk_pipeline_upload_pngs",
+                          [&](const int64_t* rgb_off, uint8_t* d_rgb, int32_t* status) {
+                              return png_decode(ctx, data, byte_offsets, rgb_off, d_rgb, status);
+                          },
+                          counts_out, out_widths, out_heights, status_out);
 }
 
 int vpk_pipeline_run(vpk_ctx* ctx, int32_t S, int32_t sphere_mode, double alpha, const vpk_em_config* cfg_in) {

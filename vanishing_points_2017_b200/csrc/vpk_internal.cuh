@@ -89,6 +89,7 @@ struct PipeState;  // pipeline.cu
 struct LsdState;   // lsd.cu
 struct PrepState;  // image_prep.cu
 struct JpegState;  // jpeg.cu
+struct PngState;   // png.cu
 
 }  // namespace vpk
 
@@ -119,6 +120,7 @@ struct vpk_ctx {
     vpk::LsdState* lsd = nullptr;
     vpk::PrepState* prep = nullptr;
     vpk::JpegState* jpeg = nullptr;
+    vpk::PngState* png = nullptr;
 };
 
 namespace vpk {
@@ -248,11 +250,21 @@ int jpeg_plan(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, in
 int jpeg_decode(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, const int64_t* pix_off, uint8_t* d_out,
                 int32_t* status_out);
 
+// png.cu: the same for PNG files.  png_plan walks the files' chunks (host only) and keeps the headers in the context;
+// it fails with VPK_ERR_ARG naming the first unsupported file (or the first gray one if rgb_only) and returns each
+// file's size and output channels (1 for the gray colour types 0 and 4, else 3).  png_decode writes file b's
+// h x w x channels bytes at d_out + pix_off[b]; status_out (B) receives VPK_PNG_OK or VPK_PNG_CORRUPT.
+int png_plan(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t B, bool rgb_only, const char* who,
+             std::vector<int32_t>& widths, std::vector<int32_t>& heights, std::vector<int32_t>& components);
+int png_decode(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, const int64_t* pix_off, uint8_t* d_out,
+               int32_t* status_out);
+
 void cnn_free(vpk_ctx* ctx);
 void em_free(vpk_ctx* ctx);
 void pipe_free(vpk_ctx* ctx);
 void lsd_free(vpk_ctx* ctx);
 void prep_free(vpk_ctx* ctx);
 void jpeg_free(vpk_ctx* ctx);
+void png_free(vpk_ctx* ctx);
 
 }  // namespace vpk

@@ -1,8 +1,8 @@
-"""JPEG decoding (`vpk_decode_jpegs`, row N6) and photo preparation in front of LSD on the device (`vpk_prepare_images`, row N5): the head of the reference's
+"""PNG decoding (`vpk_decode_pngs`, row N7), JPEG decoding (`vpk_decode_jpegs`, row N6) and photo preparation in front of LSD on the device (`vpk_prepare_images`, row N5): the head of the reference's
 evaluation.create_data_pickles (evaluation.py:139-154), i.e. `convert ... -resize TxT` (example.py:37: 640;
 benchmark.py:59-60: 800 for ECD / HLW; OpenCV 4.13's INTER_AREA rule stands in for ImageMagick), the 8-bit RGB read
 back, and skimage.color.rgb2gray.  Photos go over PCIe as uint8 RGB; the float64 gray planes are built on the device.
-DESIGN.md sections 4.7 and 4.8.  No CPU fallback."""
+DESIGN.md sections 4.7, 4.8 and 4.9.  No CPU fallback."""
 import ctypes as C
 
 import numpy as np
@@ -61,11 +61,11 @@ def prepare_images(photos, target_size=None, ctx=None):
     return res
 
 
-def pack_jpegs(blobs):
-    """List of JPEG files (bytes, or 1-D uint8 arrays of the file contents) -> (flat bytes, byte offsets (B+1) int64).
-    Anything else raises ValueError."""
+def pack_jpegs(blobs, kind="JPEG"):
+    """List of JPEG (or `kind`) files (bytes, or 1-D uint8 arrays of the file contents) -> (flat bytes, byte offsets
+    (B+1) int64).  Anything else raises ValueError."""
     if isinstance(blobs, (bytes, bytearray, np.ndarray)) or not hasattr(blobs, "__len__"):
-        raise ValueError("blobs must be a list of JPEG files (bytes or 1-D uint8 arrays)")
+        raise ValueError("blobs must be a list of %s files (bytes or 1-D uint8 arrays)" % kind)
     parts = []
     for b in blobs:
         if isinstance(b, (bytes, bytearray, memoryview)):
@@ -73,7 +73,7 @@ def pack_jpegs(blobs):
         else:
             a = np.asarray(b)
             if a.ndim != 1 or a.dtype != np.uint8:
-                raise ValueError("a JPEG file must be bytes or a 1-D uint8 array, got %s %r" % (a.dtype, a.shape))
+                raise ValueError("a %s file must be bytes or a 1-D uint8 array, got %s %r" % (kind, a.dtype, a.shape))
         parts.append(a)
     flat = np.ascontiguousarray(np.concatenate(parts) if parts else np.zeros(0, np.uint8))
     off = np.concatenate([[0], np.cumsum([p.size for p in parts])]).astype(np.int64)
@@ -126,3 +126,43 @@ def jpeg_stats(ctx=None):
     out = np.zeros(4, np.int64)
     _lib.check(ctx.lib.vpk_jpeg_stats(ctx.h, _lib.ptr(out)), "vpk_jpeg_stats")
     return {"subsequences": int(out[0]), "redecoded": int(out[1]), "max_rounds": int(out[2]), "global_rounds": int(out[3])}
+
+
+def png_info(blobs):
+    """Walks each file's chunks (headers, IHDR and PLTE; never the image data); needs no GPU.  Returns a list of
+    (width, height, colour type, support) with support 0 for a file the decoder takes, else the reason it is refused
+    (vpk.h VPK_PNG_*, named in _lib.PNG_REASONS)."""
+    flat, off = pack_jpegs(blobs, "PNG")
+    B = len(off) - 1
+    if B == 0:
+        return []
+    w, h, t, s = (np.zeros(B, np.int32) for _ in range(4))
+    _lib.check(_lib.load().vpk_png_info(_lib.ptr(flat), _lib.ptr(off), B, _lib.ptr(w), _lib.ptr(h), _lib.ptr(t), _lib.ptr(s)),
+               "vpk_png_info")
+    return [(int(a), int(b), int(c), int(d)) for a, b, c, d in zip(w, h, t, s)]
+
+
+def decode_pngs(blobs, ctx=None):
+    """Decodes 8-bit and lower PNG files on the device, bit for bit with libpng (alpha dropped, no colour management).
+    Returns (arrays, status): (H, W, 3) uint8 RGB arrays for colour types 2, 3 and 6, (H, W) gray for types 0 and 4,
+    and an int32 status per file (0, or _lib.PNG_CORRUPT for a damaged stream, whose pixels are unspecified).  A
+    refused file raises VpkError naming its index and reason."""
+    flat, off = pack_jpegs(blobs, "PNG")
+    B = len(off) - 1
+    if B == 0:
+        return [], np.zeros(0, np.int32)
+    info = png_info(blobs)
+    for k, (w, h, t, s) in enumerate(info):
+        if s != 0:
+            raise _lib.VpkError("decode_pngs: file %d is not supported: %s" % (k, _lib.PNG_REASONS[s]))
+    ctx = ctx or _lib.default_context()
+    nc = [1 if t in (0, 4) else 3 for _, _, t, _ in info]
+    out = np.empty(max(sum(w * h * c for (w, h, _, _), c in zip(info, nc)), 1), np.uint8)
+    status = np.empty(B, np.int32)
+    _lib.check(ctx.lib.vpk_decode_pngs(ctx.h, _lib.ptr(flat), _lib.ptr(off), B, _lib.ptr(out), _lib.ptr(status)), "vpk_decode_pngs")
+    res, pos = [], 0
+    for (w, h, _, _), c in zip(info, nc):
+        n = w * h * c
+        res.append(out[pos:pos + n].reshape((h, w, 3) if c == 3 else (h, w)))
+        pos += n
+    return res, status

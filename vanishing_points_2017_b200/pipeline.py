@@ -130,6 +130,29 @@ class Pipeline:
         self._off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
         return counts, [(int(a), int(b)) for a, b in zip(oh, ow)], status
 
+    def upload_pngs(self, blobs, target_size=None, **lsd_kwargs):
+        """upload_photos() from PNG files (a list of bytes or 1-D uint8 arrays of the file contents): the files are
+        decoded on the device (images.decode_pngs) where the preparation kernel reads them, so only the files cross
+        PCIe.  Returns (counts, shapes, status): as upload_photos, plus an int32 status per file (0, or
+        _lib.PNG_CORRUPT: a damaged stream, whose rows come from unspecified pixels).  A refused or gray (colour type 0
+        or 4) file raises VpkError naming its index and reason."""
+        from .images import pack_jpegs, _target
+        flat, off = pack_jpegs(blobs, "PNG")
+        B = len(off) - 1
+        if B == 0:
+            raise ValueError("upload_pngs needs at least one file")
+        cfg = _lib.lsd_config(**lsd_kwargs)
+        counts = np.empty(B, np.int32)
+        ow = np.empty(B, np.int32)
+        oh = np.empty(B, np.int32)
+        status = np.empty(B, np.int32)
+        _lib.check(self.ctx.lib.vpk_pipeline_upload_pngs(self.ctx.h, _lib.ptr(flat), _lib.ptr(off), B, _target(target_size),
+                                                         C.byref(cfg), _lib.ptr(counts), _lib.ptr(ow), _lib.ptr(oh),
+                                                         _lib.ptr(status)), "vpk_pipeline_upload_pngs")
+        self._B = B
+        self._off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
+        return counts, [(int(a), int(b)) for a, b in zip(oh, ow)], status
+
     def run(self):
         _lib.check(self.ctx.lib.vpk_pipeline_run(self.ctx.h, self.size, self.mode, self.alpha, C.byref(self.cfg)),
                    "vpk_pipeline_run")
