@@ -394,6 +394,53 @@ VPK_API int vpk_pipeline_upload_pngs(vpk_ctx* ctx, const uint8_t* data, const in
                                      int32_t target_size, const vpk_lsd_config* cfg, int32_t* counts_out,
                                      int32_t* out_widths, int32_t* out_heights, int32_t* status_out);
 
+/* ---- N8: mixed batches of files in front of photo preparation -------------------- */
+/* The dataset listing of the reference's evaluation.get_data_list (*.jpg, *.png and *.pgm in one dataset) in one
+ * call; DESIGN.md section 4.10.  Each file's format comes from its leading bytes: JPEG (FF D8 FF), PNG (the PNG
+ * signature) or netpbm ("P1" .. "P7"), of which binary PGM (P5) with maxval 255 is taken; its payload is the photo.
+ * JPEG and PNG files are decoded as vpk_decode_jpegs / vpk_decode_pngs do.  A file is gray when its decoded photo has
+ * one channel (a 1-component JPEG, PNG colour type 0 or 4, a PGM), else RGB.  Gray photos are prepared as the
+ * reference prepares them: skimage 0.12's rgb2gray returns a 2-D input unchanged, so datum['image'] is the resized
+ * uint8 plane, and detect_lsd_lines multiplies it by 255 only if its maximum is at most 1.
+ * Files: host array `data`, file b the byte_offsets[b] .. byte_offsets[b+1] bytes (B+1 non-decreasing entries). */
+enum { VPK_FILE_UNKNOWN = 0, VPK_FILE_JPEG = 1, VPK_FILE_PNG = 2, VPK_FILE_PGM = 3 };
+enum {
+    VPK_PGM_OK = 0,
+    VPK_PGM_ASCII = 1,          /* ASCII PGM (P2) */
+    VPK_PGM_BITMAP = 2,         /* PBM bitmaps (P1, P4) */
+    VPK_PGM_PAM = 3,            /* PAM (P7) */
+    VPK_PGM_PPM = 4,            /* colour netpbm (P3, P6): not a format the reference lists */
+    VPK_PGM_MAXVAL = 5,         /* maxval below 255 (the reference's rescale by ImageMagick is not pinned) */
+    VPK_PGM_DEPTH = 6,          /* maxval above 255: 16-bit samples */
+    VPK_PGM_MALFORMED = 7       /* a header that is not magic, width, height, maxval separated by whitespace and '#'
+                                 * comments with exactly one whitespace byte before the payload, or a truncated
+                                 * payload (bytes after the payload are allowed) */
+};
+/* Sniffs and parses every file (headers only); host only, needs no device or context.  formats (B) VPK_FILE_*;
+ * widths / heights (B) the photo's size (0 where the header does not give it); channels (B) 3 for RGB, 1 for gray, 0
+ * where unknown; support (B) the format's own reason code (VPK_JPEG_*, VPK_PNG_*, VPK_PGM_*; 0: taken), 1 for a file
+ * of unknown format.  Each may be NULL. */
+VPK_API int vpk_file_info(const uint8_t* data, const int64_t* byte_offsets, int32_t n, int32_t* formats, int32_t* widths,
+                          int32_t* heights, int32_t* channels, int32_t* support);
+/* Decodes every file on the device, each format's files by its decoder.  pixels_out: photo after photo, row-major
+ * height x width x channels bytes (RGB or gray); status_out (B): the format's own OK / CORRUPT code (VPK_JPEG_*,
+ * VPK_PNG_*; a PGM is always VPK_PGM_OK).  A refused or unknown file fails the call with VPK_ERR_ARG before any device
+ * work, naming its index, its format and the reason. */
+VPK_API int vpk_decode_files(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t n, uint8_t* pixels_out,
+                             int32_t* status_out);
+/* The reference's datum['image'] of every file as float64, photo after photo, each a row-major out_heights[b] x
+ * out_widths[b] plane (see vpk_prepared_size): rgb2gray in [0, 1] for RGB photos (vpk_prepare_images), the resized
+ * uint8 values for gray ones.  Refused files as vpk_decode_files. */
+VPK_API int vpk_prepare_files(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t n, int32_t target_size,
+                              int32_t* out_widths, int32_t* out_heights, double* planes_out);
+/* vpk_prepare_files followed by vpk_pipeline_upload_images on detect_lsd_lines' input (the plane times 255 when its
+ * maximum is at most 1, decided on the device), in input order: only the files cross PCIe, each once.  counts_out /
+ * out_widths / out_heights as vpk_pipeline_upload_photos, status_out (B) as vpk_decode_files (each may be NULL).
+ * Refused files as vpk_decode_files. */
+VPK_API int vpk_pipeline_upload_files(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t n,
+                                      int32_t target_size, const vpk_lsd_config* cfg, int32_t* counts_out,
+                                      int32_t* out_widths, int32_t* out_heights, int32_t* status_out);
+
 /* ---- N1: horizon line and orthogonal VP triplet --------------------------- */
 /* calc_horizon.calculate_horizon_and_ortho_vp(em_result, maxbest=10, theta_vmin=pi/10, theta_z=pi/4)
  * (reference calc_horizon.py:19-225; callers example.py:65, benchmark.py:233) for a batch of EM

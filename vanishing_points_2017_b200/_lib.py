@@ -26,6 +26,7 @@ SYMBOLS = [
     "vpk_prepared_size", "vpk_prepare_images", "vpk_pipeline_upload_photos",
     "vpk_jpeg_info", "vpk_decode_jpegs", "vpk_pipeline_upload_jpegs", "vpk_jpeg_stats",
     "vpk_png_info", "vpk_decode_pngs", "vpk_pipeline_upload_pngs",
+    "vpk_file_info", "vpk_decode_files", "vpk_prepare_files", "vpk_pipeline_upload_files",
 ]
 PIX_U8, PIX_F64 = 0, 1
 # vpk.h VPK_JPEG_*: support codes of vpk_jpeg_info and the decode status
@@ -34,6 +35,11 @@ JPEG_OK, JPEG_CORRUPT = 0, 8
 # vpk.h VPK_PNG_*: support codes of vpk_png_info and the decode status
 PNG_REASONS = ["ok", "not png", "depth", "malformed", "corrupt"]
 PNG_OK, PNG_CORRUPT = 0, 4
+# vpk.h VPK_FILE_*: formats of vpk_file_info; VPK_PGM_*: support codes of a PGM file
+FILE_UNKNOWN, FILE_JPEG, FILE_PNG, FILE_PGM = 0, 1, 2, 3
+FILE_FORMATS = ["unknown", "jpeg", "png", "pgm"]
+PGM_REASONS = ["ok", "ascii", "bitmap", "pam", "ppm", "maxval", "depth", "malformed"]
+PGM_OK = 0
 
 
 class VpkError(RuntimeError):
@@ -139,6 +145,12 @@ def load():
         lib.vpk_decode_pngs.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
         lib.vpk_pipeline_upload_pngs.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(LsdConfig),
                                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.vpk_file_info.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.vpk_decode_files.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
+        lib.vpk_prepare_files.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                          C.c_void_p]
+        lib.vpk_pipeline_upload_files.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(LsdConfig),
+                                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.vpk_abi_version.argtypes = []
         lib.vpk_last_error.argtypes = []
         _lib = lib

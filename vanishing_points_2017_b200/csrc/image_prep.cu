@@ -12,6 +12,9 @@
 //                             half up for 2 x 2 (OpenCV's vectorised path), half to even otherwise
 //                  generic    computeResizeAreaTab's partial / full / partial taps in float64, rint, clamp
 //
+// Gray photos (one channel: row N8, section 4.10) take the same paths on one channel and write the uint8 values
+// themselves (skimage 0.12's rgb2gray returns a 2-D input unchanged); for LSD's input, prep_gray_scale then applies
+// detect_lsd_lines' "* 255 if max <= 1" per gray image from a flag the tiles set.
 // Tile extents adapt to the largest factor of the batch so the source rectangle fits in shared memory.  Every
 // floating-point operation is a single correctly rounded __d*_rn operation (no FMA contraction, no libm), every sum
 // runs in increasing source index.  A VPK_DEFINES=VPK_PREP_CHECKS build asserts every shared- and global-memory index.
@@ -35,12 +38,12 @@ static constexpr size_t kPrepSmemBudget = 64 * 1024;     // preferred shared mem
 enum { PREP_IDENTITY = 0, PREP_AREA = 1, PREP_INTEGER = 2 };
 
 struct PrepState {
-    DBuf rgb, meta, out;
+    DBuf rgb, meta, out, big;
 };
 
 void prep_free(vpk_ctx* ctx) {
     if (!ctx->prep) return;
-    ctx->prep->rgb.release(); ctx->prep->meta.release(); ctx->prep->out.release();
+    ctx->prep->rgb.release(); ctx->prep->meta.release(); ctx->prep->out.release(); ctx->prep->big.release();
     delete ctx->prep;
     ctx->prep = nullptr;
 }
@@ -52,6 +55,7 @@ struct PrepImage {
     int32_t w, h, W, H;
     int32_t mode, kx, ky;   // PREP_*; block size of the integer path
     int32_t tiles_x;
+    int32_t ch;             // channels of the photo: 3 (RGB) or 1 (gray)
 };
 
 // the taps of one output column (row): lead partial tap, nfull full taps, trail partial tap, consecutive source
@@ -122,10 +126,85 @@ __device__ __forceinline__ int to_u8(double s, const PrepImage& g) {
     return (int)(q + (2 * r > area || (2 * r == area && (half_up || (q & 1)))));
 }
 
+// One tile of one image with C channels (3: RGB, 1: gray).  RGB: rgb2gray of the uint8 result, times out_scale.  Gray:
+// the uint8 values themselves; if `big` is set, big[b] becomes 1 when some value of image b exceeds 1.
+template <int C>
+__device__ __forceinline__ void prep_tile(const PrepImage& g, int b, int x0, int y0, int TW, int TH, int nx_max, int ny_max,
+                                          double out_scale, const uint8_t* __restrict__ src, double* __restrict__ dst,
+                                          int32_t* __restrict__ big, unsigned char* smem, int64_t n_src, int64_t n_out) {
+    const int nc = min(TW, g.W - x0), nr = min(TH, g.H - y0);
+    PREP_CHECK(nc > 0 && nr > 0);
+    bool over = false;                              // gray: some value of this tile exceeds 1
+    if (g.mode == PREP_IDENTITY) {
+        for (int i = threadIdx.x; i < nc * nr; i += blockDim.x) {
+            const int x = x0 + i % nc, y = y0 + i / nc;
+            const int64_t p = ((int64_t)y * g.w + x) * C;
+            PREP_CHECK(g.src + p + C - 1 < n_src && g.dst + (int64_t)y * g.W + x < n_out);
+            if (C == 3) {
+                dst[(int64_t)y * g.W + x] = gray(src[p], src[p + 1], src[p + 2], out_scale);
+            } else {
+                dst[(int64_t)y * g.W + x] = (double)src[p];
+                over |= src[p] > 1;
+            }
+        }
+    } else {
+        Taps* tx = reinterpret_cast<Taps*>(smem);
+        Taps* ty = tx + TW;
+        double* T = reinterpret_cast<double*>(ty + TH);                               // ny_max x TW x C
+        uint8_t* S = reinterpret_cast<uint8_t*>(T + (size_t)ny_max * TW * C);         // ny_max x nx_max x C
+        if (threadIdx.x < nc) tx[threadIdx.x] = make_taps(x0 + threadIdx.x, g.w, g.sx, g.mode, g.kx);
+        else if (threadIdx.x >= TW && threadIdx.x < TW + nr) ty[threadIdx.x - TW] = make_taps(y0 + threadIdx.x - TW, g.h, g.sy, g.mode, g.ky);
+        __syncthreads();
+        const int xa = tx[0].first, ya = ty[0].first;
+        const int nx = last_tap(tx[nc - 1]) - xa + 1, ny = last_tap(ty[nr - 1]) - ya + 1;
+        PREP_CHECK(xa >= 0 && ya >= 0 && xa + nx <= g.w && ya + ny <= g.h && nx <= nx_max && ny <= ny_max);
+        // stage the source rectangle (row by row, contiguous bytes)
+        const int rowb = nx * C;
+        for (int i = threadIdx.x; i < ny * rowb; i += blockDim.x) {
+            const int r = i / rowb, c = i - r * rowb;
+            const int64_t p = ((int64_t)(ya + r) * g.w + xa) * C + c;
+            PREP_CHECK(g.src + p < n_src && i < ny_max * nx_max * C);
+            S[i] = src[p];
+        }
+        __syncthreads();
+        // x pass: T[r][j][c] for every staged row r and output column j
+        for (int i = threadIdx.x; i < ny * nc * C; i += blockDim.x) {
+            const int c = i % C, j = (i / C) % nc, r = i / (C * nc);
+            const Taps& q = tx[j];
+            PREP_CHECK(q.first >= xa && last_tap(q) < xa + nx && (r * TW + j) * C + c < ny_max * TW * C);
+            T[(r * TW + j) * C + c] = tap_sum(q, S + r * rowb + (q.first - xa) * C + c, C);
+        }
+        __syncthreads();
+        // y pass, uint8, then gray (RGB) or the value itself (gray)
+        for (int i = threadIdx.x; i < nr * nc; i += blockDim.x) {
+            const int j = i % nc, r = i / nc;
+            const Taps& q = ty[r];
+            PREP_CHECK(q.first >= ya && last_tap(q) < ya + ny);
+            const double* col = T + ((q.first - ya) * TW + j) * C;
+            const int64_t o = (int64_t)(y0 + r) * g.W + x0 + j;
+            if (C == 3) {
+                const int v0 = to_u8(tap_sum(q, col, TW * 3), g);
+                const int v1 = to_u8(tap_sum(q, col + 1, TW * 3), g);
+                const int v2 = to_u8(tap_sum(q, col + 2, TW * 3), g);
+                PREP_CHECK(g.dst + o < n_out && v0 >= 0 && v0 <= 255 && v1 >= 0 && v1 <= 255 && v2 >= 0 && v2 <= 255);
+                dst[o] = gray(v0, v1, v2, out_scale);
+            } else {
+                const int v = to_u8(tap_sum(q, col, TW), g);
+                PREP_CHECK(g.dst + o < n_out && v >= 0 && v <= 255);
+                dst[o] = (double)v;
+                over |= v > 1;
+            }
+        }
+    }
+    if (C == 1 && big) {                            // uniform per CTA: every thread reaches the barrier
+        if (__syncthreads_or(over) && threadIdx.x == 0) big[b] = 1;
+    }
+}
+
 __global__ void __launch_bounds__(kPrepThreads) image_prep(const uint8_t* __restrict__ rgb, const PrepImage* __restrict__ im,
                                                            const int32_t* __restrict__ tile_off, int B, int TW, int TH, int nx_max,
-                                                           int ny_max, double out_scale, double* __restrict__ out, int64_t n_src,
-                                                           int64_t n_out) {
+                                                           int ny_max, double out_scale, double* __restrict__ out,
+                                                           int32_t* __restrict__ big, int64_t n_src, int64_t n_out) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int t = blockIdx.x;
     int lo = 0, hi = B - 1;
@@ -136,59 +215,26 @@ __global__ void __launch_bounds__(kPrepThreads) image_prep(const uint8_t* __rest
     const PrepImage g = im[lo];
     const int tl = t - tile_off[lo];
     const int x0 = (tl % g.tiles_x) * TW, y0 = (tl / g.tiles_x) * TH;
-    const int nc = min(TW, g.W - x0), nr = min(TH, g.H - y0);
-    PREP_CHECK(nc > 0 && nr > 0);
-    const uint8_t* src = rgb + g.src;
-    double* dst = out + g.dst;
-    if (g.mode == PREP_IDENTITY) {
-        for (int i = threadIdx.x; i < nc * nr; i += blockDim.x) {
-            const int x = x0 + i % nc, y = y0 + i / nc;
-            const int64_t p = ((int64_t)y * g.w + x) * 3;
-            PREP_CHECK(g.src + p + 2 < n_src && g.dst + (int64_t)y * g.W + x < n_out);
-            dst[(int64_t)y * g.W + x] = gray(src[p], src[p + 1], src[p + 2], out_scale);
+    if (g.ch == 3) prep_tile<3>(g, lo, x0, y0, TW, TH, nx_max, ny_max, out_scale, rgb + g.src, out + g.dst, big, smem, n_src, n_out);
+    else prep_tile<1>(g, lo, x0, y0, TW, TH, nx_max, ny_max, out_scale, rgb + g.src, out + g.dst, big, smem, n_src, n_out);
+}
+
+// detect_lsd_lines' "* 255 if max <= 1" for the gray images: the plane of gray image gray_idx[k] is multiplied by
+// `scale` unless the preparation kernel flagged a value above 1 in it
+__global__ void __launch_bounds__(kPrepThreads) prep_gray_scale(const PrepImage* __restrict__ im, const int32_t* __restrict__ gray_idx,
+                                                                int n_gray, const int32_t* __restrict__ big, double scale,
+                                                                double* __restrict__ out, int64_t n_out) {
+    for (int k = blockIdx.y; k < n_gray; k += gridDim.y) {
+        const int b = gray_idx[k];
+        if (big[b]) continue;
+        const PrepImage& g = im[b];
+        const int64_t n = (int64_t)g.W * g.H;
+        for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+            PREP_CHECK(g.ch == 1 && g.dst + i < n_out);
+            out[g.dst + i] = mul(out[g.dst + i], scale);
         }
-        return;
     }
-    Taps* tx = reinterpret_cast<Taps*>(smem);
-    Taps* ty = tx + TW;
-    double* T = reinterpret_cast<double*>(ty + TH);                               // ny_max x TW x 3
-    uint8_t* S = reinterpret_cast<uint8_t*>(T + (size_t)ny_max * TW * 3);         // ny_max x nx_max x 3
-    if (threadIdx.x < nc) tx[threadIdx.x] = make_taps(x0 + threadIdx.x, g.w, g.sx, g.mode, g.kx);
-    else if (threadIdx.x >= TW && threadIdx.x < TW + nr) ty[threadIdx.x - TW] = make_taps(y0 + threadIdx.x - TW, g.h, g.sy, g.mode, g.ky);
-    __syncthreads();
-    const int xa = tx[0].first, ya = ty[0].first;
-    const int nx = last_tap(tx[nc - 1]) - xa + 1, ny = last_tap(ty[nr - 1]) - ya + 1;
-    PREP_CHECK(xa >= 0 && ya >= 0 && xa + nx <= g.w && ya + ny <= g.h && nx <= nx_max && ny <= ny_max);
-    // stage the source rectangle (row by row, contiguous bytes)
-    const int rowb = nx * 3;
-    for (int i = threadIdx.x; i < ny * rowb; i += blockDim.x) {
-        const int r = i / rowb, c = i - r * rowb;
-        const int64_t p = ((int64_t)(ya + r) * g.w + xa) * 3 + c;
-        PREP_CHECK(g.src + p < n_src && i < ny_max * nx_max * 3);
-        S[i] = src[p];
-    }
-    __syncthreads();
-    // x pass: T[r][j][c] for every staged row r and output column j
-    for (int i = threadIdx.x; i < ny * nc * 3; i += blockDim.x) {
-        const int c = i % 3, j = (i / 3) % nc, r = i / (3 * nc);
-        const Taps& q = tx[j];
-        PREP_CHECK(q.first >= xa && last_tap(q) < xa + nx && (r * TW + j) * 3 + c < ny_max * TW * 3);
-        T[(r * TW + j) * 3 + c] = tap_sum(q, S + r * rowb + (q.first - xa) * 3 + c, 3);
-    }
-    __syncthreads();
-    // y pass, uint8, gray
-    for (int i = threadIdx.x; i < nr * nc; i += blockDim.x) {
-        const int j = i % nc, r = i / nc;
-        const Taps& q = ty[r];
-        PREP_CHECK(q.first >= ya && last_tap(q) < ya + ny);
-        const double* col = T + ((q.first - ya) * TW + j) * 3;
-        const int v0 = to_u8(tap_sum(q, col, TW * 3), g);
-        const int v1 = to_u8(tap_sum(q, col + 1, TW * 3), g);
-        const int v2 = to_u8(tap_sum(q, col + 2, TW * 3), g);
-        const int64_t o = (int64_t)(y0 + r) * g.W + x0 + j;
-        PREP_CHECK(g.dst + o < n_out && v0 >= 0 && v0 <= 255 && v1 >= 0 && v1 <= 255 && v2 >= 0 && v2 <= 255);
-        dst[o] = gray(v0, v1, v2, out_scale);
-    }
+    (void)n_out;
 }
 
 static void prepared_size(int w, int h, int target, int* W, int* H) {
@@ -200,19 +246,22 @@ static void prepared_size(int w, int h, int target, int* W, int* H) {
     *H = std::max(1, (int)nearbyint(h * s));
 }
 
-int prep_plan(const int64_t* byte_offsets, const int32_t* widths, const int32_t* heights, int32_t B,
+int prep_plan(const int64_t* byte_offsets, const int32_t* widths, const int32_t* heights, const int32_t* channels, int32_t B,
               int32_t target_size, const char* who, PrepPlan& p) {
     if (!byte_offsets || !widths || !heights || B <= 0) { set_error("%s: bad argument", who); return VPK_ERR_ARG; }
     if (byte_offsets[0] != 0) { set_error("%s: byte_offsets[0] must be 0", who); return VPK_ERR_ARG; }
     p.B = B;
     p.w.assign(widths, widths + B); p.h.assign(heights, heights + B);
+    if (channels) p.c.assign(channels, channels + B); else p.c.assign(B, 3);
     p.W.resize(B); p.H.resize(B);
     p.src_off.assign(byte_offsets, byte_offsets + B + 1);
     p.pix_off.assign(B + 1, 0);
     for (int b = 0; b < B; ++b) {
-        const int w = widths[b], h = heights[b];
-        if (w <= 0 || h <= 0 || byte_offsets[b + 1] - byte_offsets[b] != 3 * (int64_t)w * h) {
-            set_error("%s: photo %d: byte_offsets[b+1] - byte_offsets[b] must be 3 * widths[b] * heights[b] > 0", who, b);
+        const int w = widths[b], h = heights[b], c = p.c[b];
+        if (c != 1 && c != 3) { set_error("%s: photo %d: %d channels (1 or 3)", who, b, c); return VPK_ERR_ARG; }
+        if (w <= 0 || h <= 0 || byte_offsets[b + 1] - byte_offsets[b] != c * (int64_t)w * h) {
+            if (channels) set_error("%s: photo %d: byte_offsets[b+1] - byte_offsets[b] must be channels[b] * widths[b] * heights[b] > 0", who, b);
+            else set_error("%s: photo %d: byte_offsets[b+1] - byte_offsets[b] must be 3 * widths[b] * heights[b] > 0", who, b);
             return VPK_ERR_ARG;
         }
         prepared_size(w, h, target_size, &p.W[b], &p.H[b]);
@@ -229,11 +278,19 @@ int prep_input(vpk_ctx* ctx, const PrepPlan& p, uint8_t** d_rgb) {
     return VPK_OK;
 }
 
+int prep_output(vpk_ctx* ctx, int64_t n_out, double** d_out) {
+    VPK_CUDA(cudaSetDevice(ctx->device));
+    if (!ctx->prep) ctx->prep = new PrepState();
+    VPK_TRY(ctx->prep->out.ensure((size_t)std::max<int64_t>(n_out, 1) * sizeof(double)));
+    *d_out = ctx->prep->out.as<double>();
+    return VPK_OK;
+}
+
 // shared memory of a TW x TH tile whose source rectangle spans at most fx, fy source pixels per output pixel
-static size_t tile_smem(int TW, int TH, double fx, double fy, int* nx, int* ny) {
+static size_t tile_smem(int TW, int TH, double fx, double fy, int C, int* nx, int* ny) {
     *nx = (int)ceil(TW * fx) + 3;
     *ny = (int)ceil(TH * fy) + 3;
-    return (size_t)(TW + TH) * sizeof(Taps) + (size_t)*ny * TW * 3 * sizeof(double) + (((size_t)*nx * *ny * 3 + 15) & ~(size_t)15);
+    return (size_t)(TW + TH) * sizeof(Taps) + (size_t)*ny * TW * C * sizeof(double) + (((size_t)*nx * *ny * C + 15) & ~(size_t)15);
 }
 
 int prep_run(vpk_ctx* ctx, const PrepPlan& p, double out_scale, double* d_out) {
@@ -243,23 +300,27 @@ int prep_run(vpk_ctx* ctx, const PrepPlan& p, double out_scale, double* d_out) {
     PrepState* s = ctx->prep;
     cudaStream_t st = ctx->stream;
     std::vector<PrepImage> im(B);
+    std::vector<int32_t> gray_idx;
     double fx = 1.0, fy = 1.0;
+    int C = 1;                                      // the most channels of a resized photo: sizes the staging
     for (int b = 0; b < B; ++b) {
         PrepImage& g = im[b];
         g.src = p.src_off[b]; g.dst = p.pix_off[b];
         g.w = p.w[b]; g.h = p.h[b]; g.W = p.W[b]; g.H = p.H[b];
+        g.ch = p.c[b];
         g.sx = 1.0 / ((double)g.W / g.w);
         g.sy = 1.0 / ((double)g.H / g.h);
         g.kx = g.w / g.W; g.ky = g.h / g.H;
         g.mode = g.W == g.w && g.H == g.h ? PREP_IDENTITY : g.w % g.W == 0 && g.h % g.H == 0 ? PREP_INTEGER : PREP_AREA;
-        if (g.mode != PREP_IDENTITY) { fx = std::max(fx, g.sx); fy = std::max(fy, g.sy); }
+        if (g.mode != PREP_IDENTITY) { fx = std::max(fx, g.sx); fy = std::max(fy, g.sy); C = std::max(C, g.ch); }
+        if (g.ch == 1) gray_idx.push_back(b);
     }
     // the largest tile whose source rectangle fits the budget: halve the height first, then the width
     int TW = kTileW, TH = kTileH, nx = 0, ny = 0;
-    size_t smem = tile_smem(TW, TH, fx, fy, &nx, &ny);
+    size_t smem = tile_smem(TW, TH, fx, fy, C, &nx, &ny);
     while (smem > kPrepSmemBudget && (TH > 1 || TW > 1)) {
         if (TH > 1) TH >>= 1; else TW >>= 1;
-        smem = tile_smem(TW, TH, fx, fy, &nx, &ny);
+        smem = tile_smem(TW, TH, fx, fy, C, &nx, &ny);
     }
     int smem_max = 0;
     VPK_CUDA(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
@@ -276,16 +337,39 @@ int prep_run(vpk_ctx* ctx, const PrepPlan& p, double out_scale, double* d_out) {
         tile_off[b + 1] = tile_off[b] + (int32_t)n;
     }
     const int64_t n_src = p.src_off[B], n_out = p.pix_off[B];
-    const size_t im_bytes = (size_t)B * sizeof(PrepImage);
-    VPK_TRY(s->meta.ensure(im_bytes + (size_t)(B + 1) * sizeof(int32_t)));
+    const int n_gray = (int)gray_idx.size();
+    // gray planes of LSD's input (out_scale != 1) follow detect_lsd_lines' rule: each image's "some value > 1" flag
+    const bool rule = n_gray > 0 && out_scale != 1.0;
+    const size_t im_bytes = (size_t)B * sizeof(PrepImage), tile_bytes = (size_t)(B + 1) * sizeof(int32_t);
+    VPK_TRY(s->meta.ensure(im_bytes + tile_bytes + (size_t)n_gray * sizeof(int32_t)));
     VPK_CUDA(cudaMemcpyAsync(s->meta.p, im.data(), im_bytes, cudaMemcpyHostToDevice, st));
-    VPK_CUDA(cudaMemcpyAsync(s->meta.as<char>() + im_bytes, tile_off.data(), (size_t)(B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    VPK_CUDA(cudaMemcpyAsync(s->meta.as<char>() + im_bytes, tile_off.data(), tile_bytes, cudaMemcpyHostToDevice, st));
+    int32_t* d_big = nullptr;
+    const int32_t* d_gray = reinterpret_cast<const int32_t*>(s->meta.as<char>() + im_bytes + tile_bytes);
+    if (rule) {
+        VPK_CUDA(cudaMemcpyAsync(s->meta.as<char>() + im_bytes + tile_bytes, gray_idx.data(), (size_t)n_gray * sizeof(int32_t),
+                                 cudaMemcpyHostToDevice, st));
+        VPK_TRY(s->big.ensure((size_t)B * sizeof(int32_t)));
+        d_big = s->big.as<int32_t>();
+        VPK_CUDA(cudaMemsetAsync(d_big, 0, (size_t)B * sizeof(int32_t), st));
+    }
     if (smem > 48 * 1024) VPK_CUDA(cudaFuncSetAttribute(image_prep, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    KernelScope ks(ctx, "image_prep");
-    image_prep<<<tile_off[B], kPrepThreads, smem, st>>>(s->rgb.as<uint8_t>(), s->meta.as<PrepImage>(),
-                                                        reinterpret_cast<const int32_t*>(s->meta.as<char>() + im_bytes), B, TW, TH,
-                                                        nx, ny, out_scale, d_out, n_src, n_out);
-    return check_launch("image_prep");
+    {
+        KernelScope ks(ctx, "image_prep");
+        image_prep<<<tile_off[B], kPrepThreads, smem, st>>>(s->rgb.as<uint8_t>(), s->meta.as<PrepImage>(),
+                                                            reinterpret_cast<const int32_t*>(s->meta.as<char>() + im_bytes), B, TW, TH,
+                                                            nx, ny, out_scale, d_out, d_big, n_src, n_out);
+        VPK_TRY(check_launch("image_prep"));
+    }
+    if (rule) {
+        int64_t most = 1;
+        for (int b : gray_idx) most = std::max<int64_t>(most, (int64_t)p.W[b] * p.H[b]);
+        const dim3 grid((unsigned)std::min<int64_t>((most + kPrepThreads - 1) / kPrepThreads, 64), (unsigned)std::min(n_gray, 65535));
+        KernelScope ks(ctx, "prep_gray_scale");
+        prep_gray_scale<<<grid, kPrepThreads, 0, st>>>(s->meta.as<PrepImage>(), d_gray, n_gray, d_big, out_scale, d_out, n_out);
+        VPK_TRY(check_launch("prep_gray_scale"));
+    }
+    return VPK_OK;
 }
 
 }  // namespace vpk
@@ -306,7 +390,7 @@ int vpk_prepare_images(vpk_ctx* ctx, const uint8_t* rgb, const int64_t* byte_off
                        int32_t n_images, int32_t target_size, int32_t* out_widths, int32_t* out_heights, double* gray_out) {
     if (!ctx || !out_widths || !out_heights) { set_error("vpk_prepare_images: bad argument"); return VPK_ERR_ARG; }
     PrepPlan p;
-    VPK_TRY(prep_plan(byte_offsets, widths, heights, n_images, target_size, "vpk_prepare_images", p));
+    VPK_TRY(prep_plan(byte_offsets, widths, heights, nullptr, n_images, target_size, "vpk_prepare_images", p));
     if (!rgb) { set_error("vpk_prepare_images: rgb is NULL"); return VPK_ERR_ARG; }
     if (!gray_out) { set_error("vpk_prepare_images: gray_out is NULL"); return VPK_ERR_ARG; }
     VPK_CUDA(cudaSetDevice(ctx->device));

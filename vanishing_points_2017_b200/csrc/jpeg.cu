@@ -370,7 +370,7 @@ int jpeg_parse(const uint8_t* data, const int64_t* byte_offsets, int32_t B, cons
     return VPK_OK;
 }
 
-static const char* reason_name(int r) {
+const char* jpeg_reason_name(int r) {
     switch (r) {
         case VPK_JPEG_PROGRESSIVE: return "progressive";
         case VPK_JPEG_ARITHMETIC: return "arithmetic coding";
@@ -386,7 +386,7 @@ static const char* reason_name(int r) {
 int jpeg_require(const std::vector<jpeg::Header>& hs, bool rgb_only, const char* who) {
     for (size_t b = 0; b < hs.size(); ++b) {
         if (hs[b].support != jpeg::OK) {
-            set_error("%s: photo %zu is not supported: reason %d (%s)", who, b, hs[b].support, reason_name(hs[b].support));
+            set_error("%s: photo %zu is not supported: reason %d (%s)", who, b, hs[b].support, jpeg_reason_name(hs[b].support));
             return VPK_ERR_ARG;
         }
         if (rgb_only && hs[b].nc != 3) {

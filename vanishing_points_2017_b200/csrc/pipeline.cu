@@ -62,17 +62,17 @@ static int upload_detected(vpk_ctx* ctx, const double* d_rows, const std::vector
     return VPK_OK;
 }
 
-// Decoded files into the resident batch: `decode(rgb_off, d_rgb, status)` writes photo b's h x w x 3 RGB bytes at
-// d_rgb + rgb_off[b], where the preparation kernel reads them; then preparation, LSD and the normalisation, as
-// vpk_pipeline_upload_photos.  Only the files cross PCIe.
+// Decoded files into the resident batch: `decode(rgb_off, d_rgb, status)` writes photo b's h x w x c bytes (c[b]: 3
+// for RGB, 1 for gray) at d_rgb + rgb_off[b], where the preparation kernel reads them; then preparation, LSD and the
+// normalisation, as vpk_pipeline_upload_photos.  Only the files cross PCIe.
 template <typename Decode>
-static int upload_decoded(vpk_ctx* ctx, const std::vector<int32_t>& w, const std::vector<int32_t>& h, int32_t B, int32_t target_size,
-                          const vpk_lsd_config* cfg, const char* who, Decode decode, int32_t* counts_out, int32_t* out_widths,
-                          int32_t* out_heights, int32_t* status_out) {
+static int upload_decoded(vpk_ctx* ctx, const std::vector<int32_t>& w, const std::vector<int32_t>& h, const std::vector<int32_t>& c,
+                          int32_t B, int32_t target_size, const vpk_lsd_config* cfg, const char* who, Decode decode,
+                          int32_t* counts_out, int32_t* out_widths, int32_t* out_heights, int32_t* status_out) {
     std::vector<int64_t> rgb_off(B + 1, 0);
-    for (int b = 0; b < B; ++b) rgb_off[b + 1] = rgb_off[b] + 3 * (int64_t)w[b] * h[b];
+    for (int b = 0; b < B; ++b) rgb_off[b + 1] = rgb_off[b] + (int64_t)c[b] * w[b] * h[b];
     PrepPlan pp;
-    VPK_TRY(prep_plan(rgb_off.data(), w.data(), h.data(), B, target_size, who, pp));
+    VPK_TRY(prep_plan(rgb_off.data(), w.data(), h.data(), c.data(), B, target_size, who, pp));
     std::vector<int32_t> counts(B), row_off, status(B);
     LsdPlan lp;
     VPK_TRY(lsd_plan(pp.pix_off.data(), pp.W.data(), pp.H.data(), B, VPK_PIX_F64, cfg, counts.data(), lp));
@@ -169,7 +169,7 @@ int vpk_pipeline_upload_photos(vpk_ctx* ctx, const uint8_t* rgb, const int64_t* 
                                int32_t* counts_out, int32_t* out_widths, int32_t* out_heights) {
     if (!ctx) { set_error("vpk_pipeline_upload_photos: bad argument"); return VPK_ERR_ARG; }
     PrepPlan pp;
-    VPK_TRY(prep_plan(byte_offsets, widths, heights, B, target_size, "vpk_pipeline_upload_photos", pp));
+    VPK_TRY(prep_plan(byte_offsets, widths, heights, nullptr, B, target_size, "vpk_pipeline_upload_photos", pp));
     if (!rgb) { set_error("vpk_pipeline_upload_photos: rgb is NULL"); return VPK_ERR_ARG; }
     // the detector reads the prepared planes (float64, x 255) where the preparation kernel writes them
     std::vector<int32_t> counts(B), row_off;
@@ -196,7 +196,7 @@ int vpk_pipeline_upload_jpegs(vpk_ctx* ctx, const uint8_t* data, const int64_t* 
     if (!ctx) { set_error("vpk_pipeline_upload_jpegs: bad argument"); return VPK_ERR_ARG; }
     std::vector<int32_t> w, h, nc;
     VPK_TRY(jpeg_plan(ctx, data, byte_offsets, B, true, "vpk_pipeline_upload_jpegs", w, h, nc));
-    return upload_decoded(ctx, w, h, B, target_size, cfg, "vpk_pipeline_upload_jpegs",
+    return upload_decoded(ctx, w, h, nc, B, target_size, cfg, "vpk_pipeline_upload_jpegs",
                           [&](const int64_t* rgb_off, uint8_t* d_rgb, int32_t* status) {
                               return jpeg_decode(ctx, data, byte_offsets, rgb_off, d_rgb, status);
                           },
@@ -209,10 +209,21 @@ int vpk_pipeline_upload_pngs(vpk_ctx* ctx, const uint8_t* data, const int64_t* b
     if (!ctx) { set_error("vpk_pipeline_upload_pngs: bad argument"); return VPK_ERR_ARG; }
     std::vector<int32_t> w, h, nc;
     VPK_TRY(png_plan(ctx, data, byte_offsets, B, true, "vpk_pipeline_upload_pngs", w, h, nc));
-    return upload_decoded(ctx, w, h, B, target_size, cfg, "vpk_pipeline_upload_pngs",
+    return upload_decoded(ctx, w, h, nc, B, target_size, cfg, "vpk_pipeline_upload_pngs",
                           [&](const int64_t* rgb_off, uint8_t* d_rgb, int32_t* status) {
                               return png_decode(ctx, data, byte_offsets, rgb_off, d_rgb, status);
                           },
+                          counts_out, out_widths, out_heights, status_out);
+}
+
+int vpk_pipeline_upload_files(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t B, int32_t target_size,
+                              const vpk_lsd_config* cfg, int32_t* counts_out, int32_t* out_widths, int32_t* out_heights,
+                              int32_t* status_out) {
+    if (!ctx) { set_error("vpk_pipeline_upload_files: bad argument"); return VPK_ERR_ARG; }
+    FilesPlan fp;
+    VPK_TRY(files_plan(ctx, data, byte_offsets, B, "vpk_pipeline_upload_files", fp));
+    return upload_decoded(ctx, fp.w, fp.h, fp.c, B, target_size, cfg, "vpk_pipeline_upload_files",
+                          [&](const int64_t*, uint8_t* d_rgb, int32_t* status) { return files_decode(ctx, fp, d_rgb, status); },
                           counts_out, out_widths, out_heights, status_out);
 }
 

@@ -282,7 +282,7 @@ int png_parse(const uint8_t* data, const int64_t* byte_offsets, int32_t B, const
     return VPK_OK;
 }
 
-static const char* reason_name(int r) {
+const char* png_reason_name(int r) {
     switch (r) {
         case VPK_PNG_NOT_PNG: return "not a PNG file";
         case VPK_PNG_DEPTH: return "16-bit samples";
@@ -298,7 +298,7 @@ int png_plan(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int
     VPK_TRY(png_parse(data, byte_offsets, B, who, hs));
     for (int b = 0; b < B; ++b) {
         if (hs[b].support != png::OK) {
-            set_error("%s: photo %d is not supported: reason %d (%s)", who, b, hs[b].support, reason_name(hs[b].support));
+            set_error("%s: photo %d is not supported: reason %d (%s)", who, b, hs[b].support, png_reason_name(hs[b].support));
             return VPK_ERR_ARG;
         }
         if (rgb_only && png::out_channels(hs[b].ctype) != 3) {

@@ -226,19 +226,22 @@ int lsd_plan(const int64_t* pixel_offsets, const int32_t* widths, const int32_t*
 int lsd_input(vpk_ctx* ctx, const LsdPlan& plan, void** d_in);
 int lsd_detect(vpk_ctx* ctx, const LsdPlan& plan, int32_t* counts_out, const double** d_rows, std::vector<int32_t>& row_offsets);
 
-// image_prep.cu: resize (INTER_AREA) + rgb2gray of a ragged batch of uint8 RGB photos.  prep_plan validates the
-// call and computes the prepared sizes (host only); prep_input sizes the device buffer of the photos and returns it
-// (photo b's bytes at plan.src_off[b]); prep_run writes the float64 gray planes of what was written there, multiplied
-// by out_scale, to d_out (image b's W'*H' plane at plan.pix_off[b]).
+// image_prep.cu: resize (INTER_AREA) + rgb2gray of a ragged batch of uint8 RGB or gray photos.  prep_plan validates
+// the call and computes the prepared sizes (host only; channels NULL: every photo RGB); prep_input sizes the device
+// buffer of the photos and returns it (photo b's h x w x c bytes at plan.src_off[b]); prep_run writes the float64
+// planes of what was written there to d_out (image b's W'*H' plane at plan.pix_off[b]): rgb2gray times out_scale for
+// RGB photos, the uint8 values for gray ones, and with out_scale != 1 (LSD's input) a gray plane whose values are all
+// at most 1 times out_scale (detect_lsd_lines' "* 255 if max <= 1", decided on the device).
 struct PrepPlan {
     int32_t B = 0;
-    std::vector<int32_t> w, h, W, H;
+    std::vector<int32_t> w, h, c, W, H;
     std::vector<int64_t> src_off;   // B+1 byte offsets of the photos
     std::vector<int64_t> pix_off;   // B+1 pixel offsets of the prepared planes
 };
-int prep_plan(const int64_t* byte_offsets, const int32_t* widths, const int32_t* heights, int32_t B,
+int prep_plan(const int64_t* byte_offsets, const int32_t* widths, const int32_t* heights, const int32_t* channels, int32_t B,
               int32_t target_size, const char* who, PrepPlan& plan);
 int prep_input(vpk_ctx* ctx, const PrepPlan& plan, uint8_t** d_rgb);
+int prep_output(vpk_ctx* ctx, int64_t n_out, double** d_out);     // the context's buffer of n_out prepared pixels
 int prep_run(vpk_ctx* ctx, const PrepPlan& plan, double out_scale, double* d_out);
 
 // jpeg.cu: jpeg_plan parses the files' markers (host only) and keeps the headers in the context; it fails with
@@ -258,6 +261,30 @@ int png_plan(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int
              std::vector<int32_t>& widths, std::vector<int32_t>& heights, std::vector<int32_t>& components);
 int png_decode(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, const int64_t* pix_off, uint8_t* d_out,
                int32_t* status_out);
+
+const char* jpeg_reason_name(int r);
+const char* png_reason_name(int r);
+
+// files.cu: mixed batches of JPEG, PNG and PGM files.  files_plan sniffs and parses every file (host only), fails with
+// VPK_ERR_ARG naming the first refused or unknown file with its format and reason, plans the JPEG and PNG subsets in
+// their decoders' states and lays out one photo buffer (file b's h x w x c bytes at pix_off[b]).  files_decode writes
+// every photo there, one decoder after the other on the context's stream (the PGM payloads by plain copies); each file
+// crosses PCIe once.  status_out (B) receives each format's own OK / CORRUPT code.
+struct FilesPlan {
+    int32_t B = 0;
+    const uint8_t* data = nullptr;
+    const int64_t* byte_offsets = nullptr;
+    std::vector<int32_t> fmt, w, h, c;
+    std::vector<int64_t> pix_off;               // B+1
+    std::vector<int32_t> sub[2];                // indices of the JPEG and PNG files
+    std::vector<uint8_t> pack[2];               // their bytes, when they are not one contiguous range of `data`
+    const uint8_t* sub_data[2] = {nullptr, nullptr};
+    std::vector<int64_t> sub_off[2];            // file offsets in sub_data
+    std::vector<int32_t> pgm;                   // indices of the PGM files
+    std::vector<int64_t> pgm_payload;           // byte offset of each one's payload in `data`
+};
+int files_plan(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t B, const char* who, FilesPlan& plan);
+int files_decode(vpk_ctx* ctx, const FilesPlan& plan, uint8_t* d_out, int32_t* status_out);
 
 void cnn_free(vpk_ctx* ctx);
 void em_free(vpk_ctx* ctx);

@@ -1,8 +1,8 @@
-"""PNG decoding (`vpk_decode_pngs`, row N7), JPEG decoding (`vpk_decode_jpegs`, row N6) and photo preparation in front of LSD on the device (`vpk_prepare_images`, row N5): the head of the reference's
+"""Mixed batches of JPEG, PNG and PGM files, colour or gray (`vpk_decode_files` / `vpk_prepare_files`, row N8), PNG decoding (`vpk_decode_pngs`, row N7), JPEG decoding (`vpk_decode_jpegs`, row N6) and photo preparation in front of LSD on the device (`vpk_prepare_images`, row N5): the head of the reference's
 evaluation.create_data_pickles (evaluation.py:139-154), i.e. `convert ... -resize TxT` (example.py:37: 640;
 benchmark.py:59-60: 800 for ECD / HLW; OpenCV 4.13's INTER_AREA rule stands in for ImageMagick), the 8-bit RGB read
 back, and skimage.color.rgb2gray.  Photos go over PCIe as uint8 RGB; the float64 gray planes are built on the device.
-DESIGN.md sections 4.7, 4.8 and 4.9.  No CPU fallback."""
+DESIGN.md sections 4.7 to 4.10.  No CPU fallback."""
 import ctypes as C
 
 import numpy as np
@@ -166,3 +166,67 @@ def decode_pngs(blobs, ctx=None):
         res.append(out[pos:pos + n].reshape((h, w, 3) if c == 3 else (h, w)))
         pos += n
     return res, status
+
+
+def file_info(blobs):
+    """Sniffs each file (JPEG, PNG or netpbm by its leading bytes) and reads its header; needs no GPU.  Returns a list
+    of (format, width, height, channels, support): format a _lib.FILE_* code (named in _lib.FILE_FORMATS), channels 3
+    for RGB and 1 for gray, support 0 for a file decode_files takes, else the format's own reason code
+    (_lib.JPEG_REASONS, _lib.PNG_REASONS, _lib.PGM_REASONS; 1 for an unknown format)."""
+    flat, off = pack_jpegs(blobs, "image")
+    B = len(off) - 1
+    if B == 0:
+        return []
+    f, w, h, c, s = (np.zeros(B, np.int32) for _ in range(5))
+    _lib.check(_lib.load().vpk_file_info(_lib.ptr(flat), _lib.ptr(off), B, _lib.ptr(f), _lib.ptr(w), _lib.ptr(h), _lib.ptr(c),
+                                         _lib.ptr(s)), "vpk_file_info")
+    return [(int(a), int(b), int(d), int(e), int(g)) for a, b, d, e, g in zip(f, w, h, c, s)]
+
+
+def _split(buf, shapes):
+    res, pos = [], 0
+    for shape in shapes:
+        n = int(np.prod(shape))
+        res.append(buf[pos:pos + n].reshape(shape))
+        pos += n
+    return res
+
+
+def decode_files(blobs, ctx=None):
+    """Decodes a mixed batch of JPEG, PNG and binary PGM files on the device, each format by its decoder, in one call.
+    Returns (arrays, status): (H, W, 3) uint8 RGB arrays, (H, W) for gray files, and an int32 status per file (the
+    format's own code: 0, _lib.JPEG_CORRUPT or _lib.PNG_CORRUPT).  A refused or unknown file raises VpkError naming its
+    index, format and reason (file_info tells them beforehand)."""
+    flat, off = pack_jpegs(blobs, "image")
+    B = len(off) - 1
+    if B == 0:
+        return [], np.zeros(0, np.int32)
+    ctx = ctx or _lib.default_context()
+    info = file_info(blobs)
+    shapes = [(h, w, 3) if c == 3 else (h, w) for _, w, h, c, _ in info]
+    out = np.empty(max(sum(int(np.prod(s)) for s in shapes), 1), np.uint8)
+    status = np.empty(B, np.int32)
+    _lib.check(ctx.lib.vpk_decode_files(ctx.h, _lib.ptr(flat), _lib.ptr(off), B, _lib.ptr(out), _lib.ptr(status)), "vpk_decode_files")
+    return _split(out, shapes), status
+
+
+def prepare_files(blobs, target_size=None, ctx=None):
+    """The reference's datum['image'] of each file of a mixed batch (decode_files, then the preparation of
+    prepare_images), in one device call: float64 (H', W') planes in [0, 1] for colour files (rgb2gray), uint8 (H', W')
+    planes for gray files (skimage 0.12's rgb2gray returns a 2-D input unchanged), which is what
+    evaluation.reference_data(images=...) stores.  Refused files as decode_files."""
+    flat, off = pack_jpegs(blobs, "image")
+    B = len(off) - 1
+    if B == 0:
+        return []
+    ctx = ctx or _lib.default_context()
+    t = _target(target_size)
+    info = file_info(blobs)
+    n = sum(int(np.prod(prepared_size(w, h, t))) if s == 0 and w > 0 and h > 0 else 0 for _, w, h, _, s in info)
+    out = np.empty(max(n, 1), np.float64)
+    ow = np.empty(B, np.int32)
+    oh = np.empty(B, np.int32)
+    _lib.check(ctx.lib.vpk_prepare_files(ctx.h, _lib.ptr(flat), _lib.ptr(off), B, t, _lib.ptr(ow), _lib.ptr(oh), _lib.ptr(out)),
+               "vpk_prepare_files")
+    planes = _split(out, [(int(H), int(W)) for W, H in zip(ow, oh)])
+    return [p if c == 3 else p.astype(np.uint8) for p, (_, _, _, c, _) in zip(planes, info)]

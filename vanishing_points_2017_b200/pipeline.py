@@ -153,6 +153,31 @@ class Pipeline:
         self._off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
         return counts, [(int(a), int(b)) for a, b in zip(oh, ow)], status
 
+    def upload_files(self, blobs, target_size=None, **lsd_kwargs):
+        """upload_photos() from a mixed batch of files (a list of bytes or 1-D uint8 arrays): JPEG, PNG and binary PGM,
+        colour or gray, as evaluation.get_data_list lists them.  Each format's files are decoded on the device by its
+        decoder; colour files are prepared as upload_photos does, gray ones as the reference does (the resized uint8
+        plane, times 255 only if its maximum is at most 1), and LSD and the normalisation follow for the whole batch in
+        input order.  Only the files cross PCIe.  Returns (counts, shapes, status) as upload_jpegs, status being each
+        format's own code (0, _lib.JPEG_CORRUPT or _lib.PNG_CORRUPT).  A refused or unknown file raises VpkError
+        naming its index, format and reason (images.file_info tells them beforehand)."""
+        from .images import pack_jpegs, _target
+        flat, off = pack_jpegs(blobs, "image")
+        B = len(off) - 1
+        if B == 0:
+            raise ValueError("upload_files needs at least one file")
+        cfg = _lib.lsd_config(**lsd_kwargs)
+        counts = np.empty(B, np.int32)
+        ow = np.empty(B, np.int32)
+        oh = np.empty(B, np.int32)
+        status = np.empty(B, np.int32)
+        _lib.check(self.ctx.lib.vpk_pipeline_upload_files(self.ctx.h, _lib.ptr(flat), _lib.ptr(off), B, _target(target_size),
+                                                          C.byref(cfg), _lib.ptr(counts), _lib.ptr(ow), _lib.ptr(oh),
+                                                          _lib.ptr(status)), "vpk_pipeline_upload_files")
+        self._B = B
+        self._off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
+        return counts, [(int(a), int(b)) for a, b in zip(oh, ow)], status
+
     def run(self):
         _lib.check(self.ctx.lib.vpk_pipeline_run(self.ctx.h, self.size, self.mode, self.alpha, C.byref(self.cfg)),
                    "vpk_pipeline_run")
