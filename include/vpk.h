@@ -462,6 +462,50 @@ VPK_API int vpk_pipeline_horizon(vpk_ctx* ctx, int32_t maxbest, double theta_vmi
                                  const double* true_horizons, const double* scales, const double* heights, double* points,
                                  int32_t* best_combo, double* errors);
 
+/* ---- N9: pipeline input and output in CUDA memory ------------------------------- */
+/* The entry points above in a form for data that is already on the device (photos decoded by another GPU decoder,
+ * gray planes, segments from a model) and for results consumed there; DESIGN.md section 4.11.  The data pointers
+ * below are caller-owned DEVICE (or managed) memory of the context's device; every other pointer is host memory.
+ * Interop: the library links the CUDA runtime statically and runs on the device's primary context (cudaSetDevice),
+ * the one PyTorch and the CUDA runtime of other libraries use, so their device pointers and stream handles are valid
+ * here.  Strides are in ELEMENTS, non-negative (0 repeats an element), so views (crops, column slices, a CHW tensor
+ * permuted to HWC) need no copy; no element outside ptr + sum (extent - 1) * stride is read.
+ * Ordering: `stream` is the caller's stream (a cudaStream_t; 0: the legacy default stream).  Each call's device work
+ * runs after the work queued on `stream` before the call (an event recorded there, waited for on the context's
+ * stream), and device outputs are ordered before the work queued on `stream` after the call (the reverse event).
+ * The upload calls still synchronise the host with the context's stream before they return (they return the
+ * per-image counts and plan the ragged batch on the host), so their inputs may be reused once they return;
+ * vpk_pipeline_fetch_device and vpk_pipeline_horizon_device never block the host.
+ * Validation happens before any device work: a pointer that is host memory, memory of another device or not a CUDA
+ * pointer, a negative stride, a zero size or a channel count other than 1 or 3 fails with VPK_ERR_ARG, naming the
+ * image. */
+/* vpk_pipeline_upload from device segments: (sum N, 4) float64, element (n, k) at segments[n * row_stride + k * col_stride];
+ * offsets (B+1) are host memory. */
+VPK_API int vpk_pipeline_upload_device(vpk_ctx* ctx, const double* segments, int64_t row_stride, int64_t col_stride,
+                                       const int32_t* offsets, int32_t n_images, void* stream);
+/* vpk_pipeline_upload_images from device gray images of one dtype (VPK_PIX_U8 or VPK_PIX_F64): images (B) device
+ * pointers, image b's pixel (y, x) at images[b][y * strides[2b] + x * strides[2b+1]], widths[b] x heights[b]. */
+VPK_API int vpk_pipeline_upload_images_device(vpk_ctx* ctx, const void* const* images, const int64_t* strides,
+                                              const int32_t* widths, const int32_t* heights, int32_t n_images, int32_t dtype,
+                                              const vpk_lsd_config* cfg, void* stream, int32_t* counts_out);
+/* vpk_pipeline_upload_photos from device uint8 photos: photo b's sample (y, x, c) at photos[b][y * strides[3b] +
+ * x * strides[3b+1] + c * strides[3b+2]], widths[b] x heights[b] x channels[b].  A 3-channel photo is prepared as by
+ * vpk_pipeline_upload_photos, a 1-channel photo as a gray file by vpk_pipeline_upload_files (the resized uint8 plane,
+ * times 255 only if its maximum is at most 1).  counts_out / out_widths / out_heights as vpk_pipeline_upload_photos. */
+VPK_API int vpk_pipeline_upload_photos_device(vpk_ctx* ctx, const uint8_t* const* photos, const int64_t* strides,
+                                              const int32_t* widths, const int32_t* heights, const int32_t* channels,
+                                              int32_t n_images, int32_t target_size, const vpk_lsd_config* cfg, void* stream,
+                                              int32_t* counts_out, int32_t* out_widths, int32_t* out_heights);
+/* vpk_pipeline_fetch into device buffers of exactly its layout: the vpk_em_result fields (decision_metric ignored),
+ * sigout (B,20,20) float32 and sphere_images (B,S,S) uint8 are device pointers; out, sigout and sphere_images may be
+ * NULL.  Asynchronous. */
+VPK_API int vpk_pipeline_fetch_device(vpk_ctx* ctx, vpk_em_result* out, float* sigout, uint8_t* sphere_images, void* stream);
+/* vpk_pipeline_horizon into device arrays points (B,5,3), best_combo (B,3), errors (B) or NULL; with errors, the
+ * contiguous true_horizons (B,3), scales (B) and heights (B) are device arrays too.  Asynchronous. */
+VPK_API int vpk_pipeline_horizon_device(vpk_ctx* ctx, int32_t maxbest, double theta_vmin, double theta_z,
+                                        const double* true_horizons, const double* scales, const double* heights,
+                                        double* points, int32_t* best_combo, double* errors, void* stream);
+
 /* device time of the last vpk_pipeline_run per stage: [lines+sphere, cnn, em, total] ms */
 VPK_API int vpk_pipeline_stage_ms(vpk_ctx* ctx, float ms[4]);
 

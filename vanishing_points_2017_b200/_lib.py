@@ -1,7 +1,9 @@
 """ctypes binding of libvpk.so (include/vpk.h).  No CPU fallback: if the
 library or a CUDA device is missing, calls fail loudly."""
+import collections
 import ctypes as C
 import os
+import sys
 import threading
 
 import numpy as np
@@ -27,6 +29,8 @@ SYMBOLS = [
     "vpk_jpeg_info", "vpk_decode_jpegs", "vpk_pipeline_upload_jpegs", "vpk_jpeg_stats",
     "vpk_png_info", "vpk_decode_pngs", "vpk_pipeline_upload_pngs",
     "vpk_file_info", "vpk_decode_files", "vpk_prepare_files", "vpk_pipeline_upload_files",
+    "vpk_pipeline_upload_device", "vpk_pipeline_upload_images_device", "vpk_pipeline_upload_photos_device",
+    "vpk_pipeline_fetch_device", "vpk_pipeline_horizon_device",
 ]
 PIX_U8, PIX_F64 = 0, 1
 # vpk.h VPK_JPEG_*: support codes of vpk_jpeg_info and the decode status
@@ -151,6 +155,15 @@ def load():
                                           C.c_void_p]
         lib.vpk_pipeline_upload_files.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.POINTER(LsdConfig),
                                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.vpk_pipeline_upload_device.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p]
+        lib.vpk_pipeline_upload_images_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                                          C.c_int32, C.POINTER(LsdConfig), C.c_void_p, C.c_void_p]
+        lib.vpk_pipeline_upload_photos_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                          C.c_int32, C.c_int32, C.POINTER(LsdConfig), C.c_void_p, C.c_void_p,
+                                                          C.c_void_p, C.c_void_p]
+        lib.vpk_pipeline_fetch_device.argtypes = [C.c_void_p, C.POINTER(EmResult), C.c_void_p, C.c_void_p, C.c_void_p]
+        lib.vpk_pipeline_horizon_device.argtypes = [C.c_void_p, C.c_int32, C.c_double, C.c_double, C.c_void_p, C.c_void_p,
+                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.vpk_abi_version.argtypes = []
         lib.vpk_last_error.argtypes = []
         _lib = lib
@@ -277,3 +290,89 @@ def as_offsets(offsets):
     if o.ndim != 1 or o.size < 1 or o[0] != 0 or np.any(np.diff(o) < 0):
         raise ValueError("offsets must be a non-decreasing int array starting at 0")
     return o
+
+
+# ---- arrays in CUDA memory (__cuda_array_interface__), row N9 ----
+U8, F64, I32, I64 = "|u1", "<f8", "<i4", "<i8"
+_TYPESTR_ALIASES = {"<u1": U8, "=u1": U8, ">u1": U8, "=f8": F64, "=i4": I32, "=i8": I64}
+
+CudaArray = collections.namedtuple("CudaArray", "ptr shape strides typestr stream")
+CudaArray.__doc__ = """An array in CUDA memory: data pointer, shape, strides in BYTES (always given), typestr (U8, F64, I32 or
+I64 for their aliases) and the stream its producer exported (__cuda_array_interface__ v3; None: none to order after)."""
+
+
+def is_cuda_array(obj):
+    return hasattr(obj, "__cuda_array_interface__")
+
+
+def cuda_array(obj, typestrs=(U8, F64), ndims=(2, 3), channels=(1, 3)):
+    """The __cuda_array_interface__ (v2 or v3) of `obj` as a CudaArray; strides None (C-contiguous) are filled in.
+    ValueError for a typestr not in `typestrs`, a rank not in `ndims`, a 3-D array whose last extent is not in
+    `channels`, a mask, a negative stride or a stride that is not a whole number of elements.  Imports nothing."""
+    cai = obj.__cuda_array_interface__
+    version = int(cai.get("version", 0))
+    if version < 2:
+        raise ValueError("__cuda_array_interface__ version %d; 2 or later is read" % version)
+    if cai.get("mask") is not None:
+        raise ValueError("masked CUDA arrays are not taken")
+    typestr = _TYPESTR_ALIASES.get(cai["typestr"], cai["typestr"])
+    if typestr not in typestrs:
+        raise ValueError("CUDA array of type %r; expected %s" % (cai["typestr"], " or ".join(typestrs)))
+    shape = tuple(int(s) for s in cai["shape"])
+    if len(shape) not in ndims:
+        raise ValueError("CUDA array of shape %r; expected %s dimensions" % (shape, " or ".join(str(n) for n in ndims)))
+    if len(shape) == 3 and channels is not None and shape[2] not in channels:
+        raise ValueError("CUDA array of shape %r: %d channels, expected %s" % (shape, shape[2], " or ".join(str(c) for c in channels)))
+    itemsize = int(typestr[2:])
+    strides = cai.get("strides")
+    if strides is None:
+        strides, step = [], itemsize
+        for s in reversed(shape):
+            strides.insert(0, step)
+            step *= s
+    strides = tuple(int(s) for s in strides)
+    if len(strides) != len(shape):
+        raise ValueError("CUDA array: %d strides for %d dimensions" % (len(strides), len(shape)))
+    if any(s < 0 for s in strides):
+        raise ValueError("CUDA array with negative strides %r; make it contiguous first" % (strides,))
+    if any(s % itemsize for s in strides):
+        raise ValueError("CUDA array strides %r are not whole elements of %d bytes" % (strides, itemsize))
+    stream = cai.get("stream") if version >= 3 else None
+    return CudaArray(int(cai["data"][0] or 0), shape, strides, typestr, None if stream is None else int(stream))
+
+
+def _handle(stream):
+    """cudaStream_t of a stream object (torch .cuda_stream, cupy .ptr) or an int handle."""
+    for attr in ("cuda_stream", "ptr"):
+        if hasattr(stream, attr):
+            return int(getattr(stream, attr))
+    return int(stream)
+
+
+def torch_stream(handle, device):
+    import torch
+    if handle in (0, 1):
+        return torch.cuda.default_stream(device)
+    return torch.cuda.ExternalStream(handle, device=device)
+
+
+def call_stream(stream, device, arrays=()):
+    """The cudaStream_t a device call is ordered on: `stream` (a stream object or handle; 0 the legacy default stream), or
+    if None PyTorch's current stream of `device` when torch is imported, else 0.  Work queued on a CAI v3 stream that
+    an input exports and that differs from it is ordered before it with an event."""
+    if stream is not None:
+        h = _handle(stream)
+    elif "torch" in sys.modules:
+        h = int(sys.modules["torch"].cuda.current_stream(device).cuda_stream)
+    else:
+        h = 0
+    legacy = lambda s: 0 if s in (0, 1) else s      # noqa: E731  (CAI v3 writes the legacy default stream as 1)
+    others = {legacy(a.stream) for a in arrays if a.stream is not None} - {legacy(h)}
+    if others:
+        import torch
+        target = torch_stream(h, device)
+        for s in sorted(others):
+            ev = torch.cuda.Event()
+            ev.record(torch_stream(s, device))
+            target.wait_event(ev)
+    return h

@@ -85,6 +85,8 @@ int vpk_destroy(vpk_ctx* ctx) {
     ctx->d_hist.release(); ctx->d_img.release(); ctx->d_weights.release(); ctx->d_misc.release(); ctx->d_curves_tab.release();
     ctx->h_stage.release();
     for (auto& e : ctx->marks) if (e) cudaEventDestroy(e);
+    ctx->d_pack.release();
+    for (auto& e : ctx->io_ev) if (e) cudaEventDestroy(e);
     cudaStreamDestroy(ctx->stream);
     delete ctx;
     return VPK_OK;

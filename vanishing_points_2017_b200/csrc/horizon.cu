@@ -229,6 +229,26 @@ void horizon_unpack(const void* h_rec, int32_t B, double* points, int32_t* best_
     }
 }
 
+// the same on the device, one thread per image, into the caller's device arrays
+__global__ void horizon_unpack_kernel(const HorizonOut* __restrict__ r, int32_t B, double* __restrict__ points,
+                                      int32_t* __restrict__ best_combo, double* __restrict__ errors) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    const double* src[5] = {r[b].hP1, r[b].hP2, r[b].zVP, r[b].hVP1, r[b].hVP2};
+    for (int q = 0; q < 5; ++q)
+        for (int k = 0; k < 3; ++k) points[((size_t)b * 5 + q) * 3 + k] = src[q][k];
+    for (int k = 0; k < 3; ++k) best_combo[(size_t)b * 3 + k] = r[b].combo[k];
+    if (errors) errors[b] = r[b].err;
+}
+
+int horizon_unpack_dev(vpk_ctx* ctx, const void* d_rec, int32_t B, double* d_points, int32_t* d_best_combo, double* d_errors) {
+    if (B <= 0) return VPK_OK;
+    KernelScope ks(ctx, "horizon_unpack");
+    horizon_unpack_kernel<<<(B + 127) / 128, 128, 0, ctx->stream>>>(static_cast<const HorizonOut*>(d_rec), B, d_points, d_best_combo,
+                                                                      d_errors);
+    return check_launch("horizon_unpack");
+}
+
 }  // namespace vpk
 
 using namespace vpk;

@@ -98,24 +98,71 @@ using namespace vpk;
 
 extern "C" {
 
-int vpk_pipeline_upload(vpk_ctx* ctx, const double* segments, const int32_t* offsets, int32_t B) {
-    if (!ctx || !offsets || B <= 0 || offsets[0] != 0) { set_error("vpk_pipeline_upload: bad argument"); return VPK_ERR_ARG; }
-    for (int b = 0; b < B; ++b) if (offsets[b + 1] < offsets[b]) { set_error("vpk_pipeline_upload: offsets must be non-decreasing"); return VPK_ERR_ARG; }
-    const int64_t sumN = offsets[B];
-    if (sumN > 0 && !segments) { set_error("vpk_pipeline_upload: segments is NULL"); return VPK_ERR_ARG; }
+// the resident batch's buffers for the segment offsets `offsets` (B+1, checked by the caller)
+static int begin_batch(vpk_ctx* ctx, const int32_t* offsets, int32_t B, PipeState** out) {
     VPK_CUDA(cudaSetDevice(ctx->device));
     if (!ctx->pipe) {
         ctx->pipe = new PipeState();
         for (auto& e : ctx->pipe->ev) VPK_CUDA(cudaEventCreate(&e));
     }
     PipeState* p = ctx->pipe;
+    const int64_t sumN = offsets[B];
     p->B = B; p->sumN = sumN; p->have_result = false;
     p->h_offsets.assign(offsets, offsets + B + 1);
     VPK_TRY(p->seg.ensure((sumN + 1) * 4 * sizeof(double)));
     VPK_TRY(p->lines.ensure((sumN + 1) * 3 * sizeof(double)));
     VPK_TRY(p->offsets.ensure((B + 1) * sizeof(int32_t)));
-    if (sumN) VPK_CUDA(cudaMemcpyAsync(p->seg.p, segments, sumN * 4 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
     VPK_CUDA(cudaMemcpyAsync(p->offsets.p, offsets, (B + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+    *out = p;
+    return VPK_OK;
+}
+
+static int check_offsets(const int32_t* offsets, int32_t B, const char* who) {
+    if (!offsets || B <= 0 || offsets[0] != 0) { set_error("%s: bad argument", who); return VPK_ERR_ARG; }
+    for (int b = 0; b < B; ++b) if (offsets[b + 1] < offsets[b]) { set_error("%s: offsets must be non-decreasing", who); return VPK_ERR_ARG; }
+    return VPK_OK;
+}
+
+// element strides of caller arrays: non-negative, and small enough that no byte offset overflows
+static int check_stride(int64_t s, const char* who, const char* what, int b) {
+    if (s < 0) { set_error("%s: %s %d: negative stride %lld", who, what, b, (long long)s); return VPK_ERR_ARG; }
+    if (s > ((int64_t)1 << 40)) { set_error("%s: %s %d: stride %lld too large", who, what, b, (long long)s); return VPK_ERR_ARG; }
+    return VPK_OK;
+}
+
+int vpk_pipeline_upload(vpk_ctx* ctx, const double* segments, const int32_t* offsets, int32_t B) {
+    if (!ctx) { set_error("vpk_pipeline_upload: bad argument"); return VPK_ERR_ARG; }
+    VPK_TRY(check_offsets(offsets, B, "vpk_pipeline_upload"));
+    const int64_t sumN = offsets[B];
+    if (sumN > 0 && !segments) { set_error("vpk_pipeline_upload: segments is NULL"); return VPK_ERR_ARG; }
+    PipeState* p = nullptr;
+    VPK_TRY(begin_batch(ctx, offsets, B, &p));
+    if (sumN) VPK_CUDA(cudaMemcpyAsync(p->seg.p, segments, sumN * 4 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    VPK_CUDA(cudaStreamSynchronize(ctx->stream));
+    return VPK_OK;
+}
+
+int vpk_pipeline_upload_device(vpk_ctx* ctx, const double* segments, int64_t row_stride, int64_t col_stride, const int32_t* offsets,
+                               int32_t B, void* stream) {
+    const char* who = "vpk_pipeline_upload_device";
+    if (!ctx) { set_error("%s: bad argument", who); return VPK_ERR_ARG; }
+    VPK_TRY(check_offsets(offsets, B, who));
+    const int64_t sumN = offsets[B];
+    if (sumN > 0) {
+        VPK_TRY(check_stride(row_stride, who, "segments", 0));
+        VPK_TRY(check_stride(col_stride, who, "segments", 0));
+        VPK_TRY(check_device_ptr(ctx, segments, who, "segments", "vpk_pipeline_upload"));
+        if (reinterpret_cast<uintptr_t>(segments) % sizeof(double)) { set_error("%s: segments is not 8-byte aligned", who); return VPK_ERR_ARG; }
+    }
+    VPK_CUDA(cudaSetDevice(ctx->device));
+    VPK_TRY(stream_enter(ctx, stream));
+    PipeState* p = nullptr;
+    VPK_TRY(begin_batch(ctx, offsets, B, &p));
+    if (sumN) {
+        std::vector<PackItem> it(1);
+        it[0] = PackItem{reinterpret_cast<const uint8_t*>(segments), row_stride * 8, col_stride * 8, 0, 0, (int32_t)sumN, 4, 1, 8, 0, 0};
+        VPK_TRY(pack_dev(ctx, it, p->seg.as<uint8_t>(), sumN * 4 * (int64_t)sizeof(double)));
+    }
     VPK_CUDA(cudaStreamSynchronize(ctx->stream));
     return VPK_OK;
 }
@@ -188,6 +235,69 @@ int vpk_pipeline_upload_photos(vpk_ctx* ctx, const uint8_t* rgb, const int64_t* 
     if (out_widths) memcpy(out_widths, pp.W.data(), (size_t)B * sizeof(int32_t));
     if (out_heights) memcpy(out_heights, pp.H.data(), (size_t)B * sizeof(int32_t));
     return VPK_OK;
+}
+
+int vpk_pipeline_upload_images_device(vpk_ctx* ctx, const void* const* images, const int64_t* strides, const int32_t* widths,
+                                      const int32_t* heights, int32_t B, int32_t dtype, const vpk_lsd_config* cfg, void* stream,
+                                      int32_t* counts_out) {
+    const char* who = "vpk_pipeline_upload_images_device";
+    if (!ctx || !images || !strides || !widths || !heights || B <= 0) { set_error("%s: bad argument", who); return VPK_ERR_ARG; }
+    if (dtype != VPK_PIX_U8 && dtype != VPK_PIX_F64) { set_error("%s: dtype must be VPK_PIX_U8 or VPK_PIX_F64", who); return VPK_ERR_ARG; }
+    const int esz = dtype == VPK_PIX_U8 ? 1 : 8;
+    std::vector<int64_t> pix_off(B + 1, 0);
+    char what[32];
+    for (int b = 0; b < B; ++b) {
+        if (widths[b] <= 0 || heights[b] <= 0) { set_error("%s: image %d: size %d x %d", who, b, widths[b], heights[b]); return VPK_ERR_ARG; }
+        VPK_TRY(check_stride(strides[2 * b], who, "image", b));
+        VPK_TRY(check_stride(strides[2 * b + 1], who, "image", b));
+        snprintf(what, sizeof(what), "image %d", b);
+        VPK_TRY(check_device_ptr(ctx, images[b], who, what, "vpk_pipeline_upload_images"));
+        if (reinterpret_cast<uintptr_t>(images[b]) % esz) { set_error("%s: image %d is not %d-byte aligned", who, b, esz); return VPK_ERR_ARG; }
+        pix_off[b + 1] = pix_off[b] + (int64_t)widths[b] * heights[b];
+    }
+    std::vector<int32_t> counts(B), row_off;
+    LsdPlan lp;
+    VPK_TRY(lsd_plan(pix_off.data(), widths, heights, B, dtype, cfg, counts.data(), lp));
+    void* d_in = nullptr;
+    VPK_TRY(lsd_input(ctx, lp, &d_in));
+    VPK_TRY(stream_enter(ctx, stream));
+    std::vector<PackItem> items(B);
+    for (int b = 0; b < B; ++b)
+        items[b] = PackItem{static_cast<const uint8_t*>(images[b]), strides[2 * b] * esz, strides[2 * b + 1] * esz, 0, pix_off[b] * esz,
+                            heights[b], widths[b], 1, esz, 0, 0};
+    VPK_TRY(pack_dev(ctx, items, static_cast<uint8_t*>(d_in), pix_off[B] * esz));
+    const double* d_rows = nullptr;
+    VPK_TRY(lsd_detect(ctx, lp, counts.data(), &d_rows, row_off));
+    VPK_TRY(upload_detected(ctx, d_rows, row_off, widths, heights, B));
+    if (counts_out) memcpy(counts_out, counts.data(), (size_t)B * sizeof(int32_t));
+    return VPK_OK;
+}
+
+int vpk_pipeline_upload_photos_device(vpk_ctx* ctx, const uint8_t* const* photos, const int64_t* strides, const int32_t* widths,
+                                      const int32_t* heights, const int32_t* channels, int32_t B, int32_t target_size,
+                                      const vpk_lsd_config* cfg, void* stream, int32_t* counts_out, int32_t* out_widths,
+                                      int32_t* out_heights) {
+    const char* who = "vpk_pipeline_upload_photos_device";
+    if (!ctx || !photos || !strides || !widths || !heights || !channels || B <= 0) { set_error("%s: bad argument", who); return VPK_ERR_ARG; }
+    char what[32];
+    for (int b = 0; b < B; ++b) {
+        if (widths[b] <= 0 || heights[b] <= 0) { set_error("%s: photo %d: size %d x %d", who, b, widths[b], heights[b]); return VPK_ERR_ARG; }
+        if (channels[b] != 1 && channels[b] != 3) { set_error("%s: photo %d: %d channels (1 or 3)", who, b, channels[b]); return VPK_ERR_ARG; }
+        for (int k = 0; k < 3; ++k) VPK_TRY(check_stride(strides[3 * b + k], who, "photo", b));
+        snprintf(what, sizeof(what), "photo %d", b);
+        VPK_TRY(check_device_ptr(ctx, photos[b], who, what, "vpk_pipeline_upload_photos"));
+    }
+    std::vector<int32_t> w(widths, widths + B), h(heights, heights + B), c(channels, channels + B);
+    return upload_decoded(ctx, w, h, c, B, target_size, cfg, who,
+                          [&](const int64_t* rgb_off, uint8_t* d_rgb, int32_t*) {
+                              VPK_TRY(stream_enter(ctx, stream));
+                              std::vector<PackItem> items(B);
+                              for (int b = 0; b < B; ++b)
+                                  items[b] = PackItem{photos[b], strides[3 * b], strides[3 * b + 1], strides[3 * b + 2], rgb_off[b],
+                                                      h[b], w[b], c[b], 1, 0, 0};
+                              return pack_dev(ctx, items, d_rgb, rgb_off[B]);
+                          },
+                          counts_out, out_widths, out_heights, nullptr);
 }
 
 int vpk_pipeline_upload_jpegs(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t B, int32_t target_size,
@@ -326,6 +436,76 @@ int vpk_pipeline_fetch(vpk_ctx* ctx, vpk_em_result* out, float* sigout, uint8_t*
         if (p->sumN) memcpy(out->vp_assoc, p->h_assoc.p, p->sumN * sizeof(int32_t));
     }
     return VPK_OK;
+}
+
+int vpk_pipeline_fetch_device(vpk_ctx* ctx, vpk_em_result* out, float* sigout, uint8_t* sphere_images, void* stream) {
+    const char* who = "vpk_pipeline_fetch_device";
+    if (!ctx || !ctx->pipe || !ctx->pipe->have_result) { set_error("%s: nothing to fetch", who); return VPK_ERR_STATE; }
+    PipeState* p = ctx->pipe;
+    const size_t B = p->B;
+    if (out) {
+        const void* f[8] = {out->status, out->n_vp, out->iterations, out->vp, out->sigma, out->counts, out->counts_weighted, out->vp_assoc};
+        const char* names[8] = {"status", "n_vp", "iterations", "vp", "sigma", "counts", "counts_weighted", "vp_assoc"};
+        for (int k = 0; k < 8; ++k)
+            if (k < 7 || p->sumN) VPK_TRY(check_device_ptr(ctx, f[k], who, names[k], "vpk_pipeline_fetch"));
+    }
+    if (sigout) VPK_TRY(check_device_ptr(ctx, sigout, who, "sigout", "vpk_pipeline_fetch"));
+    if (sphere_images) VPK_TRY(check_device_ptr(ctx, sphere_images, who, "sphere_images", "vpk_pipeline_fetch"));
+    VPK_CUDA(cudaSetDevice(ctx->device));
+    VPK_TRY(stream_enter(ctx, stream));
+    auto D2D = [&](void* dst, const void* src, size_t bytes) {
+        return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, ctx->stream);
+    };
+    if (out) {
+        // the packed block of vpk_pipeline_run: vp | sigma | counts_weighted | status | n_vp | iterations | counts
+        const double* f = p->out_small.as<double>();
+        VPK_CUDA(D2D(out->vp, f, B * VPK_MAX_VP * 3 * sizeof(double))); f += B * VPK_MAX_VP * 3;
+        VPK_CUDA(D2D(out->sigma, f, B * VPK_MAX_VP * sizeof(double))); f += B * VPK_MAX_VP;
+        VPK_CUDA(D2D(out->counts_weighted, f, B * VPK_MAX_VP * sizeof(double))); f += B * VPK_MAX_VP;
+        const int32_t* ip = reinterpret_cast<const int32_t*>(f);
+        VPK_CUDA(D2D(out->status, ip, B * sizeof(int32_t))); ip += B;
+        VPK_CUDA(D2D(out->n_vp, ip, B * sizeof(int32_t))); ip += B;
+        VPK_CUDA(D2D(out->iterations, ip, B * sizeof(int32_t))); ip += B;
+        VPK_CUDA(D2D(out->counts, ip, B * VPK_MAX_VP * sizeof(int32_t)));
+        if (p->sumN) VPK_CUDA(D2D(out->vp_assoc, p->out.vp_assoc, p->sumN * sizeof(int32_t)));
+    }
+    if (sigout) VPK_CUDA(D2D(sigout, p->sigout.p, B * kCells * sizeof(float)));
+    if (sphere_images) VPK_CUDA(D2D(sphere_images, p->images.p, B * (size_t)p->S * p->S));
+    return stream_leave(ctx, stream);
+}
+
+int vpk_pipeline_horizon_device(vpk_ctx* ctx, int32_t maxbest, double theta_vmin, double theta_z, const double* true_horizons,
+                                const double* scales, const double* heights, double* points, int32_t* best_combo, double* errors,
+                                void* stream) {
+    const char* who = "vpk_pipeline_horizon_device";
+    if (!ctx || !ctx->pipe || !ctx->pipe->have_result) { set_error("%s: no completed run", who); return VPK_ERR_STATE; }
+    if (maxbest < 0 || (errors && !(true_horizons && scales && heights))) { set_error("%s: bad argument", who); return VPK_ERR_ARG; }
+    VPK_TRY(check_device_ptr(ctx, points, who, "points", "vpk_pipeline_horizon"));
+    VPK_TRY(check_device_ptr(ctx, best_combo, who, "best_combo", "vpk_pipeline_horizon"));
+    if (errors) {
+        VPK_TRY(check_device_ptr(ctx, errors, who, "errors", "vpk_pipeline_horizon"));
+        VPK_TRY(check_device_ptr(ctx, true_horizons, who, "true_horizons", "vpk_pipeline_horizon"));
+        VPK_TRY(check_device_ptr(ctx, scales, who, "scales", "vpk_pipeline_horizon"));
+        VPK_TRY(check_device_ptr(ctx, heights, who, "heights", "vpk_pipeline_horizon"));
+    }
+    VPK_CUDA(cudaSetDevice(ctx->device));
+    PipeState* p = ctx->pipe;
+    const size_t B = p->B;
+    VPK_TRY(p->horizon.ensure(horizon_out_bytes(p->B)));
+    VPK_TRY(stream_enter(ctx, stream));
+    const double* d_truth = nullptr;
+    if (errors) {
+        // (B,3) true horizons | (B) scales | (B) heights, the block horizon_dev reads
+        VPK_TRY(p->truth.ensure(5 * B * sizeof(double)));
+        double* d = p->truth.as<double>();
+        VPK_CUDA(cudaMemcpyAsync(d, true_horizons, 3 * B * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+        VPK_CUDA(cudaMemcpyAsync(d + 3 * B, scales, B * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+        VPK_CUDA(cudaMemcpyAsync(d + 4 * B, heights, B * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+        d_truth = d;
+    }
+    VPK_TRY(horizon_dev(ctx, p->out.vp, p->out.counts, p->out.n_vp, p->B, maxbest, theta_vmin, theta_z, d_truth, p->horizon.p));
+    VPK_TRY(horizon_unpack_dev(ctx, p->horizon.p, p->B, points, best_combo, errors));
+    return stream_leave(ctx, stream);
 }
 
 int vpk_pipeline_horizon(vpk_ctx* ctx, int32_t maxbest, double theta_vmin, double theta_z, const double* true_horizons,

@@ -113,6 +113,8 @@ struct vpk_ctx {
     vpk::HBuf h_stage;
 
     cudaEvent_t marks[4] = {nullptr, nullptr, nullptr, nullptr};   // vpk_mark: device timestamps on this context's stream
+    vpk::DBuf d_pack;                                               // device_pack's descriptors
+    cudaEvent_t io_ev[2] = {nullptr, nullptr};                      // caller stream -> context stream, and back
 
     vpk::CnnState* cnn = nullptr;
     vpk::EmState* em = nullptr;
@@ -285,6 +287,25 @@ struct FilesPlan {
 };
 int files_plan(vpk_ctx* ctx, const uint8_t* data, const int64_t* byte_offsets, int32_t B, const char* who, FilesPlan& plan);
 int files_decode(vpk_ctx* ctx, const FilesPlan& plan, uint8_t* d_out, int32_t* status_out);
+
+// device_io.cu: input in caller-owned CUDA memory.  pack_dev gathers the items (each a (rows, cols, ch) array of
+// esz-byte elements at src with byte strides s0, s1, s2) row-major into d_dst + items[b].dst on the context's stream;
+// it fills rows_per_tile and dense itself.  check_device_ptr refuses anything but device or managed memory of the
+// context's device (host_entry: the entry point that takes host memory).  stream_enter orders the context's stream
+// after the work queued on `stream` (0: the legacy default stream), stream_leave orders `stream` after the context's.
+struct PackItem {
+    const uint8_t* src;
+    int64_t s0, s1, s2;
+    int64_t dst;
+    int32_t rows, cols, ch, esz;
+    int32_t rows_per_tile, dense;
+};
+int pack_dev(vpk_ctx* ctx, std::vector<PackItem>& items, uint8_t* d_dst, int64_t dst_bytes);
+int check_device_ptr(vpk_ctx* ctx, const void* p, const char* who, const char* what, const char* host_entry);
+int stream_enter(vpk_ctx* ctx, void* stream);
+int stream_leave(vpk_ctx* ctx, void* stream);
+// horizon.cu: horizon_unpack on the device, into caller device arrays (errors may be NULL)
+int horizon_unpack_dev(vpk_ctx* ctx, const void* d_rec, int32_t B, double* d_points, int32_t* d_best_combo, double* d_errors);
 
 void cnn_free(vpk_ctx* ctx);
 void em_free(vpk_ctx* ctx);

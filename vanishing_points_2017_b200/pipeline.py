@@ -46,7 +46,13 @@ class Pipeline:
         self._off = None
 
     # -- the three steps of include/vpk.h, so callers can time them separately
-    def upload(self, segments, offsets):
+    def upload(self, segments, offsets, stream=None):
+        """segments (sum N, 4) float64 with image b's rows offsets[b] .. offsets[b+1]-1.  Segments in CUDA memory
+        (anything exposing __cuda_array_interface__, e.g. a torch CUDA tensor or a column slice of a wider one) are
+        gathered on the device, ordered after the work queued on `stream` (see _lib.call_stream); offsets may then be
+        host or device memory, the latter costing one device-to-host copy on that stream."""
+        if _lib.is_cuda_array(segments):
+            return self._upload_device(segments, offsets, stream)
         seg = _lib.as_f64(segments, 4)
         off = _lib.as_offsets(offsets)
         if off[-1] != seg.shape[0]:
@@ -54,6 +60,25 @@ class Pipeline:
         self._B, self._off = off.size - 1, off
         _lib.check(self.ctx.lib.vpk_pipeline_upload(self.ctx.h, _lib.ptr(seg), _lib.ptr(off), self._B),
                    "vpk_pipeline_upload")
+
+    def _upload_device(self, segments, offsets, stream):
+        a = _lib.cuda_array(segments, (_lib.F64,), (2,))
+        if a.shape[1] != 4:
+            raise ValueError("expected a (N,4) array, got %r" % (a.shape,))
+        dev = self.ctx.device
+        if _lib.is_cuda_array(offsets):
+            st = _lib.call_stream(stream, dev, [a, _lib.cuda_array(offsets, (_lib.I32, _lib.I64), (1,))])
+            import torch
+            with torch.cuda.stream(_lib.torch_stream(st, dev)):
+                offsets = torch.as_tensor(offsets, device=torch.device("cuda", dev)).to("cpu").numpy()
+        else:
+            st = _lib.call_stream(stream, dev, [a])
+        off = _lib.as_offsets(offsets)
+        if off[-1] != a.shape[0]:
+            raise ValueError("offsets[-1] must equal the number of segments")
+        self._B, self._off = off.size - 1, off
+        _lib.check(self.ctx.lib.vpk_pipeline_upload_device(self.ctx.h, a.ptr, a.strides[0] // 8, a.strides[1] // 8, _lib.ptr(off),
+                                                           self._B, st), "vpk_pipeline_upload_device")
 
     def upload_lsd(self, lsd_rows, offsets, widths, heights):
         """upload() for raw LSD rows (flat (sum N, ncols) array, pixels): normalised on the device
@@ -68,30 +93,52 @@ class Pipeline:
         _lib.check(self.ctx.lib.vpk_pipeline_upload_lsd(self.ctx.h, _lib.ptr(lsd), lsd.shape[1], _lib.ptr(off), _lib.ptr(w),
                                                         _lib.ptr(h), self._B), "vpk_pipeline_upload_lsd")
 
-    def upload_images(self, images, **lsd_kwargs):
+    def upload_images(self, images, stream=None, **lsd_kwargs):
         """upload() from grayscale images (a list of 2-D arrays of any sizes, uint8 or float64 gray values): the
         LSD detector (lsd.detect_line_segments with `lsd_kwargs`, lsd.pyx's defaults otherwise) and the
         normalisation of evaluation.py:240-249 run on the device into the resident batch; only the per-image
-        segment counts come back.  Returns them."""
+        segment counts come back.  Returns them.  Images in CUDA memory (__cuda_array_interface__: torch CUDA tensors,
+        strided views included; all uint8 or all float64) are gathered on the device, ordered after the work queued
+        on `stream` (see _lib.call_stream)."""
         from .lsd import pack_images
         if len(images) == 0:
             raise ValueError("upload_images needs at least one image")
-        flat, dt, off, w, h = pack_images(images)
         cfg = _lib.lsd_config(**lsd_kwargs)
         counts = np.empty(len(images), np.int32)
-        _lib.check(self.ctx.lib.vpk_pipeline_upload_images(self.ctx.h, _lib.ptr(flat), dt, _lib.ptr(off), _lib.ptr(w), _lib.ptr(h),
-                                                           len(images), C.byref(cfg), _lib.ptr(counts)), "vpk_pipeline_upload_images")
+        dev = _device_arrays(images, "images", (_lib.U8, _lib.F64), (2,))
+        if dev is not None:
+            if len({a.typestr for a in dev}) != 1:
+                raise ValueError("images in CUDA memory must be all uint8 or all float64")
+            ptrs = (C.c_void_p * len(dev))(*[a.ptr for a in dev])
+            es = 1 if dev[0].typestr == _lib.U8 else 8
+            strides = np.array([[a.strides[0] // es, a.strides[1] // es] for a in dev], np.int64)
+            h, w = (np.array([a.shape[k] for a in dev], np.int32) for k in (0, 1))
+            st = _lib.call_stream(stream, self.ctx.device, dev)
+            _lib.check(self.ctx.lib.vpk_pipeline_upload_images_device(
+                self.ctx.h, ptrs, _lib.ptr(strides), _lib.ptr(w), _lib.ptr(h), len(dev), _lib.PIX_U8 if es == 1 else _lib.PIX_F64,
+                C.byref(cfg), st, _lib.ptr(counts)), "vpk_pipeline_upload_images_device")
+        else:
+            flat, dt, off, w, h = pack_images(images)
+            _lib.check(self.ctx.lib.vpk_pipeline_upload_images(self.ctx.h, _lib.ptr(flat), dt, _lib.ptr(off), _lib.ptr(w), _lib.ptr(h),
+                                                               len(images), C.byref(cfg), _lib.ptr(counts)), "vpk_pipeline_upload_images")
         self._B = len(images)
         self._off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
         return counts
 
-    def upload_photos(self, photos, target_size=None, **lsd_kwargs):
+    def upload_photos(self, photos, target_size=None, stream=None, **lsd_kwargs):
         """upload_images() from RGB photos (a list of (H, W, 3) uint8 arrays of any sizes): the preparation of
         evaluation.py:139-154 (images.prepare_images: resize to `target_size`, rgb2gray), LSD on the gray planes
         times 255 and the normalisation run on the device; the photos cross PCIe as uint8 RGB and nothing but the
         per-image counts and sizes comes back.  Returns (counts, shapes): shapes are the prepared (H', W') pairs,
-        the frames the segments are normalised in (horizons(image_heights=...), evaluation.reference_data)."""
+        the frames the segments are normalised in (horizons(image_heights=...), evaluation.reference_data).
+        Photos in CUDA memory (__cuda_array_interface__, e.g. torchvision.io.decode_jpeg(..., device="cuda") output)
+        are gathered on the device, ordered after the work queued on `stream` (see _lib.call_stream): (H, W, 3) uint8
+        views of any strides (a CHW tensor passed as t.permute(1, 2, 0), crops), or (H, W) uint8 gray photos, which
+        are prepared as upload_files prepares gray files."""
         from .images import pack_photos, _target
+        dev = _device_arrays(photos, "photos", (_lib.U8,), (2, 3))
+        if dev is not None:
+            return self._upload_photos_device(dev, _target(target_size), stream, lsd_kwargs)
         flat, off, w, h = pack_photos(photos)
         if len(w) == 0:
             raise ValueError("upload_photos needs at least one photo")
@@ -103,6 +150,22 @@ class Pipeline:
         _lib.check(self.ctx.lib.vpk_pipeline_upload_photos(self.ctx.h, _lib.ptr(flat), _lib.ptr(off), _lib.ptr(w), _lib.ptr(h), B,
                                                            _target(target_size), C.byref(cfg), _lib.ptr(counts), _lib.ptr(ow),
                                                            _lib.ptr(oh)), "vpk_pipeline_upload_photos")
+        self._B = B
+        self._off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
+        return counts, [(int(a), int(b)) for a, b in zip(oh, ow)]
+
+    def _upload_photos_device(self, dev, target, stream, lsd_kwargs):
+        cfg = _lib.lsd_config(**lsd_kwargs)
+        B = len(dev)
+        ptrs = (C.c_void_p * B)(*[a.ptr for a in dev])
+        strides = np.array([list(a.strides) + [0] * (3 - len(a.shape)) for a in dev], np.int64)
+        h, w = (np.array([a.shape[k] for a in dev], np.int32) for k in (0, 1))
+        ch = np.array([a.shape[2] if len(a.shape) == 3 else 1 for a in dev], np.int32)
+        counts, ow, oh = (np.empty(B, np.int32) for _ in range(3))
+        st = _lib.call_stream(stream, self.ctx.device, dev)
+        _lib.check(self.ctx.lib.vpk_pipeline_upload_photos_device(self.ctx.h, ptrs, _lib.ptr(strides), _lib.ptr(w), _lib.ptr(h),
+                                                                  _lib.ptr(ch), B, target, C.byref(cfg), st, _lib.ptr(counts),
+                                                                  _lib.ptr(ow), _lib.ptr(oh)), "vpk_pipeline_upload_photos_device")
         self._B = B
         self._off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
         return counts, [(int(a), int(b)) for a, b in zip(oh, ow)]
@@ -182,7 +245,14 @@ class Pipeline:
         _lib.check(self.ctx.lib.vpk_pipeline_run(self.ctx.h, self.size, self.mode, self.alpha, C.byref(self.cfg)),
                    "vpk_pipeline_run")
 
-    def fetch(self, want_response=False, want_sphere=False, raw=False):
+    def fetch(self, want_response=False, want_sphere=False, raw=False, device=False, stream=None):
+        """The EM results of the last run(): per-image dicts (raw=False) or the flat arrays (raw=True), plus the CNN
+        responses and sphere images when asked for -> (results, sig, sphere).  device=True returns torch CUDA tensors
+        of the flat arrays instead (a dict with the keys of pipeline.RAW_PER_IMAGE and "vp_assoc"; sig (B, 20, 20)
+        float32, sphere (B, S, S) uint8), written on the device without blocking the host and ordered before the work
+        queued on `stream` after the call (see _lib.call_stream)."""
+        if device:
+            return self._fetch_device(want_response, want_sphere, stream)
         arrs, res = _alloc_result(self._B, int(self._off[-1]), False)
         sig = np.empty((self._B, 20, 20), np.float32) if want_response else None
         sph = np.empty((self._B, self.size, self.size), np.uint8) if want_sphere else None
@@ -191,11 +261,34 @@ class Pipeline:
         out = arrs if raw else unpack_results(arrs, self._off)
         return (out, sig, sph) if (want_response or want_sphere) else out
 
+    def _fetch_device(self, want_response, want_sphere, stream):
+        import torch
+        dev = torch.device("cuda", self.ctx.device)
+        st = _lib.call_stream(stream, self.ctx.device)
+        B, n = self._B, int(self._off[-1])
+        tdt = {np.int32: torch.int32, np.float64: torch.float64}
+        with torch.cuda.stream(_lib.torch_stream(st, self.ctx.device)):       # the tensors belong to that stream
+            out = {k: torch.empty((B,) + _RAW_TAIL[k], dtype=tdt[_RAW_DTYPES[k]], device=dev) for k in RAW_PER_IMAGE}
+            out["vp_assoc"] = torch.empty(n, dtype=torch.int32, device=dev)
+            sig = torch.empty((B, 20, 20), dtype=torch.float32, device=dev) if want_response else None
+            sph = torch.empty((B, self.size, self.size), dtype=torch.uint8, device=dev) if want_sphere else None
+        res = _lib.EmResult(*[out[k].data_ptr() for k in ("status", "n_vp", "iterations", "vp", "sigma", "counts", "counts_weighted",
+                                                          "vp_assoc")], None)
+        _lib.check(self.ctx.lib.vpk_pipeline_fetch_device(self.ctx.h, C.byref(res), None if sig is None else sig.data_ptr(),
+                                                          None if sph is None else sph.data_ptr(), st), "vpk_pipeline_fetch_device")
+        return (out, sig, sph) if (want_response or want_sphere) else out
+
     def horizons(self, maxbest=10, theta_vmin=np.pi / 10., theta_z=np.pi / 4., true_horizons=None, scales=None,
-                 image_heights=None):
+                 image_heights=None, device=False, stream=None):
         """calc_horizon.calculate_horizon_and_ortho_vp (calc_horizon.py:19-225) on the device-resident EM
         result of the last run(): one (hP1, hP2, zVP, hVP1, hVP2, best_combo) tuple per image; with ground-truth
-        horizons also the horizon errors of benchmark.py:247-253 -> (tuples, errors)."""
+        horizons also the horizon errors of benchmark.py:247-253 -> (tuples, errors).  device=True returns torch
+        CUDA tensors (points (B, 5, 3) float64 = hP1, hP2, zVP, hVP1, hVP2; best_combo (B, 3) int32, -1 where fewer
+        than three VPs take part; errors (B) float64 or None), written without blocking the host and ordered before
+        the work queued on `stream` after the call (see _lib.call_stream); the ground truth may then be host or
+        device arrays."""
+        if device:
+            return self._horizons_device(maxbest, theta_vmin, theta_z, true_horizons, scales, image_heights, stream)
         from . import calc_horizon
         points = np.empty((self._B, 5, 3), np.float64)
         combo = np.empty((self._B, 3), np.int32)
@@ -206,6 +299,27 @@ class Pipeline:
         n_vp = np.array([3 if c[2] >= 0 else 0 for c in combo])
         out = calc_horizon._unpack(points, combo, n_vp, 3)
         return out if err is None else (out, err)
+
+    def _horizons_device(self, maxbest, theta_vmin, theta_z, true_horizons, scales, image_heights, stream):
+        import torch
+        dev = torch.device("cuda", self.ctx.device)
+        B = self._B
+        arrays = [_lib.cuda_array(a, (_lib.F64, _lib.I32, _lib.I64), (1, 2)) for a in (true_horizons, scales, image_heights) if _lib.is_cuda_array(a)]
+        st = _lib.call_stream(stream, self.ctx.device, arrays)
+        with torch.cuda.stream(_lib.torch_stream(st, self.ctx.device)):
+            points = torch.empty((B, 5, 3), dtype=torch.float64, device=dev)
+            combo = torch.empty((B, 3), dtype=torch.int32, device=dev)
+            truth, err = [None] * 3, None
+            if true_horizons is not None:
+                f64 = lambda a: torch.as_tensor(a, dtype=torch.float64, device=dev)   # noqa: E731
+                truth = [f64(true_horizons).reshape(B, 3).contiguous(), f64(scales).expand(B).contiguous(),
+                         f64(image_heights).expand(B).contiguous()]
+                err = torch.empty(B, dtype=torch.float64, device=dev)
+        ptr = lambda t: None if t is None else t.data_ptr()   # noqa: E731
+        _lib.check(self.ctx.lib.vpk_pipeline_horizon_device(self.ctx.h, int(maxbest), float(theta_vmin), float(theta_z),
+                                                            *[ptr(t) for t in truth], ptr(points), ptr(combo), ptr(err), st),
+                   "vpk_pipeline_horizon_device")
+        return points, combo, err
 
     def stage_ms(self):
         ms = (C.c_float * 4)()
@@ -342,6 +456,18 @@ _RAW_DTYPES = {"status": np.int32, "n_vp": np.int32, "iterations": np.int32, "vp
 _RAW_TAIL = {"status": (), "n_vp": (), "iterations": (), "vp": (_lib.VPK_MAX_VP, 3), "sigma": (_lib.VPK_MAX_VP,),
              "counts": (_lib.VPK_MAX_VP,), "counts_weighted": (_lib.VPK_MAX_VP,)}
 _gather_cache = {}
+
+
+def _device_arrays(items, what, typestrs, ndims):
+    """CudaArrays of a list whose members expose __cuda_array_interface__, None if none does (the host route)."""
+    if isinstance(items, np.ndarray) or not hasattr(items, "__len__"):
+        return None
+    flags = [_lib.is_cuda_array(x) for x in items]
+    if not any(flags):
+        return None
+    if not all(flags):
+        raise ValueError("%s must be all in CUDA memory or all host arrays" % what)
+    return [_lib.cuda_array(x, typestrs, ndims) for x in items]
 
 
 def _blob_layout(n_img, n_seg):
